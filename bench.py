@@ -2,7 +2,7 @@
 """Benchmark of the Pix2Pix G+D training iteration (BASELINE.json metric: "Pix2Pix G+D train
 images/sec at 256^2").
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 ours:       one process per GPU (torchrun for N > 1), batch 64 per GPU, 256x256 synthetic RGB pairs,
             bf16 tensor-core kernels from libgap_b200.so; prints ONE JSON line on rank 0.
@@ -420,8 +420,32 @@ def _max_over_ranks(dist, world, dev, *vals):
     return list(vals)
 
 
+DUMP_PARAM_SAMPLE = 1 << 19     # state_dict / gradient entries per network that --dump-outputs keeps
+
+
+def dump_outputs(out_dir: str, tr, losses: torch.Tensor) -> None:
+    """--dump-outputs: what one training step `tr` just ran hands its caller, as .npy files in `out_dir` (58 MB in
+    all): the step's [loss_d, loss_g] (fp64), the generator's output images of the step (fp32 NCHW, the whole batch)
+    and, for each network, one fixed seeded sample of its state_dict after the step's Adam update (floating-point
+    entries flattened in key order, fp32) and of the step's parameter gradients (parameters in key order, fp32: a first
+    Adam step moves every weight by about lr * sign(gradient), so the weights alone hardly show gradient magnitudes).
+    Two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    np.save(out / "losses.npy", losses.detach().cpu().double().numpy())
+    np.save(out / "fake_B.npy", tr.G.output_nchw().cpu().numpy())
+    for name, net in (("G", tr.G), ("D", tr.D)):
+        flat = torch.cat([v.detach().reshape(-1).float() for v in net.state_dict().values() if v.is_floating_point()])
+        idx = torch.randint(flat.numel(), (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(0)).sort().values
+        np.save(out / f"{name}_state_sample.npy", flat[idx.to(flat.device)].cpu().numpy())
+        flat = torch.cat([net.grad(k).reshape(-1) for k in net.key_order if k in net.views])
+        idx = torch.randint(flat.numel(), (DUMP_PARAM_SAMPLE,), generator=torch.Generator().manual_seed(1)).sort().values
+        np.save(out / f"{name}_grad_sample.npy", flat[idx.to(flat.device)].cpu().numpy())
+
+
 def run_ours(args) -> None:
-    from gan_aug_pfa_b200 import _lib, ops, parallel
+    from gan_aug_pfa_b200 import _lib, checkpoint, ops, parallel
     from gan_aug_pfa_b200.io import PairPrefetcher
     from gan_aug_pfa_b200.pix2pix import Pix2PixTrainer
 
@@ -430,6 +454,7 @@ def run_ours(args) -> None:
     torch.manual_seed(0)
     tr = Pix2PixTrainer(dev, world=world)     # world > 1: bucketed NCCL all-reduce overlapped with the backward pass;
     #                                           replicas are broadcast from rank 0 at construction
+    start = checkpoint.trainer_state(tr) if args.dump_outputs else None     # the seeded initial state
     N = BATCH_PER_GPU
     gen = torch.Generator().manual_seed(1234 + rank)
     n_batches = 2
@@ -494,6 +519,16 @@ def run_ours(args) -> None:
     (ms,) = _max_over_ranks(dist, world, dev, e0.elapsed_time(e1))
     value = world * N * args.steps / (ms * 1e-3)
     loss_host = losses.cpu().tolist()
+    if args.dump_outputs:
+        # The timed steps train from the weights the warm-up and calibration steps left, and the step's fp32 atomic
+        # reductions do not add up in the same order on every run, so those weights (and what is computed from them)
+        # drift apart from run to run.  The step that is written out is therefore the timed step function once more,
+        # on the last timed step's batch, from the seeded initial state: restored in place (captured graphs stay
+        # valid), these inputs are the same on every run.
+        checkpoint.load_trainer_state(tr, start, restore_rng=False)
+        out = step_fn(*devb[(args.steps - 1) % n_batches])
+        if rank == 0:
+            dump_outputs(args.dump_outputs, tr, out)
 
     # ---- end to end through the public API: pinned host batches -> PairPrefetcher (H2D on a copy stream into two
     # staging buffers while the previous iteration computes) -> train_step -> the step's losses copied back to pinned
@@ -799,7 +834,16 @@ def main() -> None:
                     help="skip the quick generator-inference / Siamese legs appended to the pix2pix_train line")
     ap.add_argument("--no-baselines", dest="baselines", action="store_false",
                     help="skip the drop-in, cuDNN library and CPU baseline legs (single GPU only)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="pix2pix_train: after the timed steps, run the timed step once more from the seeded initial "
+                         "weights on the last timed batch and write what it computed (losses, generated images, a "
+                         "seeded sample of the updated weights and of the step's gradients) as .npy files into DIR; the "
+                         "legs after the timed window then continue from that restored-and-stepped state")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "pix2pix_train"):
+        ap.error("--dump-outputs needs --impl ours --workload pix2pix_train")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

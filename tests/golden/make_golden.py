@@ -5,8 +5,9 @@ Run in the build container (the reference tree is not available on the GPU box):
 
 Fixtures (all small; tensors are stored only for the reduced-size configurations):
   gan_small.pt      UNetGenerator(3,3,num_downs=5,ngf=8) / NLayerDiscriminator(6,ndf=8) at 32x32, batch 2:
-                    seeded state_dicts, inputs, train-mode forward outputs, BatchNorm buffers after the
-                    forward, parameter gradients of the reference D loss and G loss.
+                    sha256 of the seeded state_dicts, inputs, train-mode forward outputs, BatchNorm buffers
+                    after the forward, parameter gradients of the reference D loss and G loss (the larger
+                    generator gradients as a fixed seeded sample, see gan_small_fixture).
   gan_full.json     default-size models (ngf=64, 256x256, batch 1): sha256 of the seeded state_dicts,
                     output checksums, and the (loss_d, loss_g) sequence of three iterations of the
                     reference's own train_gan_one_epoch.
@@ -48,6 +49,25 @@ def sd_hash(sd):
     return h.hexdigest()
 
 
+GRAD_SAMPLE = 8192      # gan_small.pt keeps this many entries of each larger gradient tensor
+
+
+def gan_small_fixture(full: dict) -> dict:
+    """What gan_small.pt stores of `full`, kept under 1 MB: the seeded initial state_dicts as sha256 (spec.py reproduces
+    them bit for bit), and of each generator gradient with more than GRAD_SAMPLE entries a fixed seeded sample of its
+    flattened entries ("grads_g_sample": name -> {"idx": int32, "val": fp32}) instead of the whole tensor."""
+    out = {k: v for k, v in full.items() if k not in ("sd_g", "sd_d", "grads_g")}
+    out["sd_g_sha256"], out["sd_d_sha256"] = sd_hash(full["sd_g"]), sd_hash(full["sd_d"])
+    out["grads_g"], out["grads_g_sample"] = {}, {}
+    for n, g in full["grads_g"].items():
+        if g.numel() <= GRAD_SAMPLE:
+            out["grads_g"][n] = g
+        else:
+            idx = torch.randperm(g.numel(), generator=torch.Generator().manual_seed(0))[:GRAD_SAMPLE].sort().values
+            out["grads_g_sample"][n] = {"idx": idx.to(torch.int32), "val": g.reshape(-1)[idx].clone()}
+    return out
+
+
 def main():
     sys.path.insert(0, str(REF))
     real_makedirs = os.makedirs
@@ -78,14 +98,14 @@ def main():
     pred_g = D(torch.cat((A, fake), 1))
     loss_g = bce(pred_g, torch.ones_like(pred_g)) + torch.nn.L1Loss()(fake, B) * 100.0
     gg = torch.autograd.grad(loss_g, list(G.parameters()))
-    torch.save({
+    torch.save(gan_small_fixture({
         "sd_g": sd_g0, "sd_d": sd_d0, "A": A, "B": B, "fake": fake.detach(), "pred_real": pred_real.detach(),
         "pred_fake": pred_fake.detach(), "loss_d": float(loss_d), "loss_g": float(loss_g),
         "buffers_g": {k: v.clone() for k, v in G.state_dict().items() if "running" in k or "num_batches" in k},
         "buffers_d": {k: v.clone() for k, v in D.state_dict().items() if "running" in k or "num_batches" in k},
         "grads_d": {n: g for (n, _), g in zip(D.named_parameters(), gd)},
         "grads_g": {n: g for (n, _), g in zip(G.named_parameters(), gg)},
-    }, OUT / "gan_small.pt")
+    }), OUT / "gan_small.pt")
 
     # ---------------- gan_full: the reference's own loop, default sizes
     torch.manual_seed(0)
