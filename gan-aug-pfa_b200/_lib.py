@@ -132,6 +132,10 @@ _SIGNATURES = {
     "gap_bn_param_grads": (C.c_int, [_P, _I, _P, _P, _P]),
     "gap_bn_bwd_finalize": (C.c_int, [_P, _P, _P, _I, _P, _P, _P, _P]),
     "gap_colsum_bf16": (C.c_int, [_P, _L, _L, _I, _P, _P]),
+    "gap_in_stats": (C.c_int, [_P, _L, _I, _L, _I, _P, _P]),
+    "gap_in_act": (C.c_int, [_P, _L, _I, _L, _I, _P, _P, _P, _L, _I, _P, _L, _I, _P]),
+    "gap_in_bwd_reduce": (C.c_int, [_P, _L, _P, _L, _P, _L, _F, _P, _P, _I, _L, _I, _P, _P]),
+    "gap_in_bwd_apply": (C.c_int, [_P, _L, _P, _L, _P, _L, _F, _P, _P, _I, _L, _I, _P, _P, _L, _P, _P]),
     "gap_adam_flat": (C.c_int, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _I, _F, _P]),
     "gap_adam_flat_devstep": (C.c_int, [_P, _P, _P, _P, _L, _F, _F, _F, _F, _F, _I, _P, _F, _P]),
     "gap_gan_losses": (C.c_int, [_P, _D, _D, _D, _P, _P]),

@@ -57,7 +57,7 @@ def _set_rng_state(d: dict, device) -> None:
 def trainer_state(trainer, extra: Optional[dict] = None) -> dict:
     """Everything needed to continue a Pix2PixTrainer run as if it had never stopped."""
     torch.cuda.synchronize(trainer.dev)
-    return {"format": FORMAT, "kind": "pix2pix", "G": _net_state(trainer.G), "D": _net_state(trainer.D),
+    return {"format": FORMAT, "kind": "pix2pix", "norm": trainer.norm, "G": _net_state(trainer.G), "D": _net_state(trainer.D),
             "hyper": {"lr_g": trainer.lr_g, "lr_d": trainer.lr_d, "betas": list(trainer.betas)},
             "dropout": {"seed": trainer.G.dropout_seed, "calls": trainer.G.dropout_calls},
             "rng": _rng_state(trainer.dev), "extra": extra or {}}
@@ -66,6 +66,9 @@ def trainer_state(trainer, extra: Optional[dict] = None) -> dict:
 def load_trainer_state(trainer, state: dict, restore_rng: bool = True) -> dict:
     if state.get("format") != FORMAT or state.get("kind") != "pix2pix":
         raise ValueError("not a gap_b200 pix2pix checkpoint")
+    norm = state.get("norm", "batch")       # checkpoints written before InstanceNorm support are BatchNorm runs
+    if norm != trainer.norm:
+        raise ValueError(f"checkpoint was written by a norm={norm!r} trainer; this trainer uses norm={trainer.norm!r}")
     _load_net(trainer.G, state["G"])
     _load_net(trainer.D, state["D"])
     trainer.lr_g, trainer.lr_d = state["hyper"]["lr_g"], state["hyper"]["lr_d"]

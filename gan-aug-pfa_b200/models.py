@@ -27,6 +27,29 @@ from .pix2pix import DiscriminatorEngine, GeneratorEngine
 # ------------------------------------------------------------------------------------------------
 # module skeletons: identical structure to the reference so that keys and RNG consumption match
 # ------------------------------------------------------------------------------------------------
+# the keyword defaults of the two normalisations the reference handles (models.py:173-176); a norm_layer is accepted only
+# in these configurations, given as the class or as functools.partial(class, <some of these keywords>)
+_NORM_DEFAULTS = {
+    nn.BatchNorm2d: ("batch", dict(eps=1e-5, momentum=0.1, affine=True, track_running_stats=True)),
+    nn.InstanceNorm2d: ("instance", dict(eps=1e-5, momentum=0.1, affine=False, track_running_stats=False)),
+}
+_SUPPORTED_NORMS = ("nn.BatchNorm2d, functools.partial(nn.BatchNorm2d, affine=True, track_running_stats=True), "
+                    "nn.InstanceNorm2d or functools.partial(nn.InstanceNorm2d, affine=False, track_running_stats=False)")
+
+
+def norm_kind(norm_layer, use_dropout: bool = False) -> str:
+    """"batch" or "instance" for a norm_layer argument the native engines implement; NotImplementedError otherwise."""
+    func, args, kw = norm_layer, (), {}
+    if isinstance(norm_layer, functools.partial):
+        func, args, kw = norm_layer.func, norm_layer.args, norm_layer.keywords
+    kind, defaults = _NORM_DEFAULTS.get(func, (None, {}))
+    if kind is None or args or any(k not in defaults or v != defaults[k] for k, v in kw.items()):
+        raise NotImplementedError(f"norm_layer={norm_layer!r} is not implemented natively; supported: {_SUPPORTED_NORMS}")
+    if kind == "instance" and use_dropout:
+        raise NotImplementedError("norm_layer=nn.InstanceNorm2d together with use_dropout=True is not implemented natively")
+    return kind
+
+
 def _is_dense_permutation(t: torch.Tensor) -> bool:
     """True when the tensor's elements tile a contiguous block of memory exactly once in SOME dimension order (what
     torch calls non-overlapping and dense): foreach optimizers keep their fast path for such parameters."""
@@ -170,6 +193,7 @@ class UnetSkipConnectionBlock(_NativeModule):
                                             bool(outermost), bool(innermost)))
         object.__setattr__(self, "_has_dropout", bool(use_dropout) or
                            (submodule is not None and getattr(submodule, "_has_dropout", False)))
+        object.__setattr__(self, "_norm", norm_kind(norm_layer, use_dropout))
         if type(norm_layer) == functools.partial:
             use_bias = norm_layer.func == nn.InstanceNorm2d
         else:
@@ -200,6 +224,8 @@ class UnetSkipConnectionBlock(_NativeModule):
         while blk is not None:
             if not isinstance(blk, UnetSkipConnectionBlock):
                 raise NotImplementedError("the native path needs UnetSkipConnectionBlock sub-modules")
+            if blk._norm != self._norm:
+                raise NotImplementedError("nested blocks must all use the same norm_layer")
             out.append(blk._shape)
             blk = blk._sub
         return out
@@ -209,7 +235,7 @@ class UnetSkipConnectionBlock(_NativeModule):
         if self._has_dropout:
             raise NotImplementedError("stand-alone blocks with use_dropout=True are not implemented natively "
                                       "(UNetGenerator(use_dropout=True) is)")
-        return GeneratorEngine(device, init=False, spec=GeneratorSpec.for_block_chain(self._chain()))
+        return GeneratorEngine(device, init=False, spec=GeneratorSpec.for_block_chain(self._chain(), norm=self._norm))
 
     def forward(self, x):
         """models.py:204-208: `self.model(x)` for the outermost block, else `torch.cat([x, self.model(x)], 1)` — where x
@@ -255,8 +281,7 @@ class UNetGenerator(_NativeModule):
 
     def __init__(self, input_nc, output_nc, num_downs=7, ngf=64, norm_layer=nn.BatchNorm2d, use_dropout=False):
         super().__init__()
-        if norm_layer is not nn.BatchNorm2d:
-            raise NotImplementedError("only norm_layer=nn.BatchNorm2d (the reference default) is implemented natively")
+        self._norm = norm_kind(norm_layer, use_dropout)
         self._cfg = (input_nc, output_nc, num_downs, ngf)
         self._use_dropout = bool(use_dropout)
         blk = UnetSkipConnectionBlock(ngf * 8, ngf * 8, input_nc=None, submodule=None, norm_layer=norm_layer,
@@ -272,7 +297,7 @@ class UNetGenerator(_NativeModule):
 
     def _make_engine(self, device):
         i, o, n, f = self._cfg
-        return GeneratorEngine(device, i, o, n, f, init=False, use_dropout=self._use_dropout)
+        return GeneratorEngine(device, i, o, n, f, init=False, use_dropout=self._use_dropout, norm=self._norm)
 
     def forward(self, input):
         return _GeneratorFn.apply(self, input, torch.is_grad_enabled(), *self.parameters())
@@ -325,8 +350,7 @@ class NLayerDiscriminator(_NativeModule):
 
     def __init__(self, input_nc, ndf=64, n_layers=3, norm_layer=nn.BatchNorm2d):
         super().__init__()
-        if norm_layer is not nn.BatchNorm2d:
-            raise NotImplementedError("only norm_layer=nn.BatchNorm2d (the reference default) is implemented natively")
+        self._norm = norm_kind(norm_layer)
         self._cfg = (input_nc, ndf, n_layers)
         use_bias = False
         kw, padw = 4, 1
@@ -344,7 +368,7 @@ class NLayerDiscriminator(_NativeModule):
 
     def _make_engine(self, device):
         i, d, n = self._cfg
-        return DiscriminatorEngine(device, i, d, n, init=False)
+        return DiscriminatorEngine(device, i, d, n, init=False, norm=self._norm)
 
     def forward(self, input):
         return _DiscriminatorFn.apply(self, input, torch.is_grad_enabled(), *self.parameters())

@@ -517,6 +517,70 @@ def colsum_bf16(x: torch.Tensor, c: int, out: torch.Tensor) -> None:
     _lib.check(_lib.lib().gap_colsum_bf16(_ptr(x), x.stride(-2), pixels, c, _ptr(out), _stream()), "gap_colsum_bf16")
 
 
+def _in_view(y: torch.Tensor) -> tuple[int, int, int, int]:
+    """(n, h*w, c, pixel stride) of an InstanceNorm input; a 1x1 map has no spatial statistics (torch raises too)."""
+    n, h, w, c, ld = _nhwc_view(y)
+    if h * w < 2:
+        raise ValueError(f"InstanceNorm2d needs more than one spatial element per channel, got input size {tuple(y.shape)}")
+    return n, h * w, c, ld
+
+
+def _in_same(y: torch.Tensor, *others: Optional[torch.Tensor]) -> None:
+    for t in others:
+        if t is not None and (t.dtype != torch.bfloat16 or tuple(t.shape) != tuple(y.shape)):
+            raise ValueError(f"expected a bf16 tensor of shape {tuple(y.shape)}, got {t.dtype} {tuple(t.shape)}")
+
+
+def _in_vecs(n: int, c: int, *vecs: torch.Tensor) -> None:
+    for v in vecs:
+        if v.dtype != torch.float32 or v.numel() != n * c:
+            raise ValueError(f"per-(image, channel) vectors must be fp32 [{n}][{c}]")
+
+
+def in_stats(y: torch.Tensor, sums: torch.Tensor) -> None:
+    """sums [2][N*C] fp64 += per-(image, channel) [sum y, sum y^2] of the NHWC bf16 tensor y."""
+    n, hw, c, ld = _in_view(y)
+    if sums.dtype != torch.float64 or sums.numel() != 2 * n * c:
+        raise ValueError(f"sums must be fp64 [2 * {n} * {c}]")
+    _lib.check(_lib.lib().gap_in_stats(_ptr(y), ld, n, hw, c, _ptr(sums), _stream()), "gap_in_stats")
+
+
+def in_act(y: torch.Tensor, scale, shift, out1: torch.Tensor, act1: int, out2: Optional[torch.Tensor] = None,
+           act2: int = ACT_NONE) -> None:
+    """out1 = act1(y*scale + shift), out2 = act2(same) with per-(image, channel) scale / shift [N][C]."""
+    n, hw, c, ld = _in_view(y)
+    _in_same(y, out1, out2)
+    _in_vecs(n, c, scale, shift)
+    _lib.check(_lib.lib().gap_in_act(_ptr(y), ld, n, hw, c, _ptr(scale), _ptr(shift), _ptr(out1), out1.stride(-2), act1,
+                                     _ptr(out2), 0 if out2 is None else out2.stride(-2), act2, _stream()), "gap_in_act")
+
+
+def in_bwd_reduce(y, g1, g2, slope, scale, shift, sums) -> None:
+    n, hw, c, ld = _in_view(y)
+    _in_same(y, g1, g2)
+    _in_vecs(n, c, scale, shift)
+    if sums.dtype != torch.float64 or sums.numel() != 2 * n * c:
+        raise ValueError(f"sums must be fp64 [2 * {n} * {c}]")
+    _lib.check(_lib.lib().gap_in_bwd_reduce(_ptr(y), ld, _ptr(g1), g1.stride(-2), _ptr(g2),
+                                            0 if g2 is None else g2.stride(-2), slope, _ptr(scale), _ptr(shift), n, hw, c,
+                                            _ptr(sums), _stream()), "gap_in_bwd_reduce")
+
+
+def in_bwd_apply(y, g1, g2, slope, scale, shift, sums, dy, dbias: Optional[torch.Tensor] = None) -> None:
+    """dy = InstanceNorm backward of the activated gradient; dbias (fp32 [C], optional) += its per-channel sum."""
+    n, hw, c, ld = _in_view(y)
+    _in_same(y, g1, g2, dy)
+    _in_vecs(n, c, scale, shift)
+    if sums.dtype != torch.float64 or sums.numel() != 2 * n * c:
+        raise ValueError(f"sums must be fp64 [2 * {n} * {c}]")
+    if dbias is not None and (dbias.dtype != torch.float32 or dbias.numel() != c):
+        raise ValueError(f"dbias must be fp32 [{c}]")
+    _lib.check(_lib.lib().gap_in_bwd_apply(_ptr(y), ld, _ptr(g1), g1.stride(-2), _ptr(g2),
+                                           0 if g2 is None else g2.stride(-2), slope, _ptr(scale), _ptr(shift), n, hw, c,
+                                           _ptr(sums), _ptr(dy), dy.stride(-2), _ptr(dbias), _stream()),
+               "gap_in_bwd_apply")
+
+
 def adam_flat(p, g, m, v, lr, beta1, beta2, eps, weight_decay, decoupled, step, grad_scale=1.0) -> None:
     _lib.check(_lib.lib().gap_adam_flat(_ptr(p), _ptr(g), _ptr(m), _ptr(v), p.numel(), lr, beta1, beta2, eps,
                                         weight_decay, 1 if decoupled else 0, step, grad_scale, _stream()),

@@ -32,6 +32,7 @@ from .spec import DiscriminatorSpec, GeneratorSpec
 
 BN_EPS = 1e-5
 BN_MOMENTUM = 0.1
+IN_EPS = 1e-5           # nn.InstanceNorm2d default
 LAMBDA_L1 = 100.0  # train_gan.py:33
 
 
@@ -111,13 +112,34 @@ class _BN:
         self.invstd = torch.empty(self.c, device=dev)
 
 
-class _Net:
-    """Shared plumbing: parameter store, BatchNorm bookkeeping, state_dict import/export."""
+@dataclass
+class _IN:
+    """InstanceNorm2d(affine=False) state for one layer: no parameters, no buffers; per-(image, channel) statistics of
+    the current activation set, sized by the batch in _alloc."""
+    name: str
+    c: int
+    sums: torch.Tensor = None       # fp64 [2][N*C]: forward [sum y, sum y^2], then backward [sum d, sum d*xhat]; zero at rest
+    scale: torch.Tensor = None      # fp32 [N][C] = invstd
+    shift: torch.Tensor = None      # fp32 [N][C] = -mean * invstd
+    mean: torch.Tensor = None
+    invstd: torch.Tensor = None
 
-    def __init__(self, device: torch.device) -> None:
+    def allocate(self, n: int, dev: torch.device) -> None:
+        self.sums = torch.zeros(2 * n * self.c, device=dev, dtype=torch.float64)
+        self.scale, self.shift, self.mean, self.invstd = (torch.empty(n, self.c, device=dev) for _ in range(4))
+
+
+class _Net:
+    """Shared plumbing: parameter store, BatchNorm / InstanceNorm bookkeeping, state_dict import/export."""
+
+    def __init__(self, device: torch.device, norm: str = "batch") -> None:
+        if norm not in ("batch", "instance"):
+            raise ValueError(f"norm must be 'batch' or 'instance', got {norm!r}")
         self.dev = device
+        self.norm = norm
         self.store = ParamStore()
         self.bns: Dict[str, _BN] = {}
+        self.ins: Dict[str, _IN] = {}
         # state_dict key -> (segment name, shape, strides) for weights / biases / BN affine
         self.views: Dict[str, Tuple[str, Tuple[int, ...], Tuple[int, ...]]] = {}
         self.key_order: List[str] = []
@@ -178,6 +200,11 @@ class _Net:
 
     def _reg_vec(self, key: str, n: int) -> None:
         self._reg(key, n, (n,), (1,))
+
+    def _reg_in(self, prefix: str, c: int) -> _IN:
+        m = _IN(prefix, c)
+        self.ins[prefix] = m
+        return m
 
     def _reg_bn(self, prefix: str, c: int) -> _BN:
         self._reg_vec(prefix + ".weight", c)
@@ -247,6 +274,8 @@ class _Net:
         snap = {a: getattr(self, a) for a in self._BUFFER_ATTRS if hasattr(self, a)}
         snap["_bn"] = {k: (b.scale.clone(), b.shift.clone(), b.mean.clone(), b.invstd.clone())
                        for k, b in self.bns.items()}
+        # the InstanceNorm tensors belong to the activation set: the next forward's _alloc replaces them
+        snap["_in"] = {k: (m.sums, m.scale, m.shift, m.mean, m.invstd) for k, m in self.ins.items()}
         snap["_n"] = self._n
         self._n = None
         return snap
@@ -257,6 +286,10 @@ class _Net:
                 for k, (sc, sh, mu, iv) in v.items():
                     b = self.bns[k]
                     b.scale, b.shift, b.mean, b.invstd = sc, sh, mu, iv
+            elif a == "_in":
+                for k, t in v.items():
+                    m = self.ins[k]
+                    m.sums, m.scale, m.shift, m.mean, m.invstd = t
             else:
                 setattr(self, a, v)
 
@@ -322,6 +355,21 @@ class _Net:
         ops.bn_eval_scale_shift(self.param(bn.name + ".weight"), self.param(bn.name + ".bias"), bn.running_mean,
                                 bn.running_var, BN_EPS, bn.scale, bn.shift)
 
+    # -- InstanceNorm helpers -------------------------------------------------------------------
+    def _in_forward(self, m: _IN, y: torch.Tensor, out1, act1, out2=None, act2=ACT_NONE) -> None:
+        """act(InstanceNorm(y)) into out1 (and out2): the same in train and eval mode (no running statistics)."""
+        ops.in_stats(y, m.sums)
+        ops.bn_finalize(m.sums, y.shape[1] * y.shape[2], None, None, IN_EPS, 0.0, 1, None, None, None, m.scale, m.shift,
+                        m.mean, m.invstd)
+        ops.in_act(y, m.scale, m.shift, out1, act1, out2, act2)
+
+    def _in_backward(self, m: _IN, y, g1, g2, slope: float, dy, dbias: Optional[torch.Tensor] = None) -> None:
+        """dy = InstanceNorm backward of d = act'(xhat)*g1 (+ relu'(xhat)*g2); dbias += its per-channel sum (the bias of
+        the conv in front, analytically zero)."""
+        ops.in_bwd_reduce(y, g1, g2, slope, m.scale, m.shift, m.sums)
+        ops.in_bwd_apply(y, g1, g2, slope, m.scale, m.shift, m.sums, dy, dbias)
+        ops.bn_param_grads(m.sums, None, None)      # re-zeroes the sums
+
     def _bn_backward(self, bn: _BN, y, g1, g2, slope: float, dy, param_grads: bool = True) -> None:
         count = y.numel() // y.shape[-1]
         ops.bn_bwd_reduce(y, g1, g2, slope, bn.scale, bn.shift, bn.mean, bn.invstd, bn.sums)
@@ -337,18 +385,22 @@ class _Net:
 # Generator
 # ================================================================================================
 class GeneratorEngine(_Net):
-    """UNetGenerator(input_nc=3, output_nc=3, num_downs, ngf, BatchNorm2d, use_dropout=False)."""
+    """UNetGenerator(input_nc=3, output_nc=3, num_downs, ngf, BatchNorm2d or InstanceNorm2d, use_dropout)."""
 
     _BUFFER_ATTRS = ("S", "x_nhwc", "A", "R", "Rin", "yd", "yu", "fake_bf", "fake_f32", "dpre", "gR", "gRin", "gA",
                      "dyu", "dyd", "xin", "out_cat")
 
     def __init__(self, device, input_nc: int = 3, output_nc: int = 3, num_downs: int = 7, ngf: int = 64,
                  init: bool = True, use_dropout: bool = False, dropout_seed: int = 0,
-                 spec: Optional[GeneratorSpec] = None) -> None:
+                 spec: Optional[GeneratorSpec] = None, norm: str = "batch") -> None:
         """`spec` (GeneratorSpec.for_block_chain) builds the engine of a stand-alone UnetSkipConnectionBlock instead of a
         whole UNetGenerator.  With spec.virtual0 the chain starts at an inner block: level 0 has no layers, the input
-        is the block's C[0]-channel feature map and the output is torch.cat([x, model(x)], 1) (models.py:208)."""
-        super().__init__(device)
+        is the block's C[0]-channel feature map and the output is torch.cat([x, model(x)], 1) (models.py:208).
+        norm="instance": nn.InstanceNorm2d layers (no state) and conv biases everywhere; a given spec carries its norm."""
+        super().__init__(device, spec.norm if spec is not None else norm)
+        inst = self.norm == "instance"
+        if inst and use_dropout:
+            raise NotImplementedError("InstanceNorm2d together with use_dropout=True is not implemented natively")
         # nn.Dropout(0.5) after the up-norm of the num_downs-5 blocks at ngf*8 (models.py:156-157,197-198); their up
         # outputs are yu[j] for j = L-2 ... L-1-(num_downs-5)
         self.use_dropout = use_dropout
@@ -360,7 +412,7 @@ class GeneratorEngine(_Net):
                 raise NotImplementedError("the native generator supports input_nc = output_nc = 3")
             if ngf % 64 != 0 or num_downs < 5:
                 raise NotImplementedError("ngf must be a multiple of 64 and num_downs >= 5")
-            spec = GeneratorSpec(input_nc, output_nc, num_downs, ngf)
+            spec = GeneratorSpec(input_nc, output_nc, num_downs, ngf, norm=norm)
         else:
             if use_dropout:
                 raise NotImplementedError("stand-alone blocks with dropout are not implemented natively")
@@ -375,18 +427,26 @@ class GeneratorEngine(_Net):
         if not v0:
             self._reg_small(self.k_up[0] + ".weight", 2 * C[0], 3, 64)
             self._reg_vec(self.k_up[0] + ".bias", 3)
+        # ubn / dbn: the norm layers (_BN or _IN); with InstanceNorm each conv's bias segment follows its weight
+        norm_reg = self._reg_in if inst else self._reg_bn
         self.ubn: List[Optional[_BN]] = [None] * L
         self.dbn: List[Optional[_BN]] = [None] * L
         for j in range(1, L):
             cin = C[j] if j == L - 1 else 2 * C[j]
             self._reg_convT(self.k_up[j] + ".weight", cin, C[j - 1])
-            self.ubn[j] = self._reg_bn(self.k_ubn[j], C[j - 1])
+            if inst:
+                self._reg_vec(self.k_up[j] + ".bias", C[j - 1])
+            self.ubn[j] = norm_reg(self.k_ubn[j], C[j - 1])
         for j in range(L - 1, 0, -1):
             self._reg_conv(self.k_down[j] + ".weight", C[j], C[j - 1])
+            if inst:
+                self._reg_vec(self.k_down[j] + ".bias", C[j])
             if self.k_dbn[j] is not None:
-                self.dbn[j] = self._reg_bn(self.k_dbn[j], C[j])
+                self.dbn[j] = norm_reg(self.k_dbn[j], C[j])
         if not v0:
             self._reg_small(self.k_down[0] + ".weight", C[0], 3, 64)
+            if inst:
+                self._reg_vec(self.k_down[0] + ".bias", C[0])
         self.store.allocate(device)
         for bn in self.bns.values():
             bn.allocate(device)
@@ -483,6 +543,8 @@ class GeneratorEngine(_Net):
         self.gA = [torch.empty(n, S[j][0], S[j][1], C[j], **bf) for j in range(L - 1)]
         self.dyu = [None] + [torch.empty_like(self.yu[j]) for j in range(1, L)]
         self.dyd = [torch.empty(n, S[j][0], S[j][1], C[j], **bf) for j in range(L)]
+        for m in self.ins.values():
+            m.allocate(n, self.dev)
         self._n = (n, h, w)
         self.alloc_gen += 1
 
@@ -526,10 +588,17 @@ class GeneratorEngine(_Net):
         g_s2 = ops.geom_conv_fwd(4, 2, 1)
         g_1x1 = ops.geom_conv_fwd(1, 1, 0)
         g_ph = ops.geom_phase_k4s2p1()
+        inst = self.norm == "instance"
+        bias = (lambda k: self.param(k + ".bias")) if inst else (lambda k: None)
         if not v0:
-            ops.thin_conv_fwd(self.x_nhwc, None, self.w_d_thin, None, self.A[0], ACT_LRELU, self.R[0][..., :C[0]], ACT_RELU)
+            ops.thin_conv_fwd(self.x_nhwc, None, self.w_d_thin, bias(self.k_down[0]), self.A[0], ACT_LRELU,
+                              self.R[0][..., :C[0]], ACT_RELU)
         for j in range(1, L - 1):
             bn = self.dbn[j]
+            if inst:        # per-image statistics: train and eval mode are the same
+                ops.conv_gemm([self.A[j - 1]], self.w_d_fwd[j], g_s2, self.yd[j], C[j], S[j], bias=bias(self.k_down[j]))
+                self._in_forward(bn, self.yd[j], self.A[j], ACT_LRELU, self.R[j][..., :C[j]], ACT_RELU)
+                continue
             if not self.training:      # eval: BatchNorm folds into the conv epilogue (scale, shift), no extra pass
                 self._bn_eval(bn)
                 ops.conv_gemm([self.A[j - 1]], self.w_d_fwd[j], g_s2, self.A[j], C[j], S[j], act=ACT_LRELU,
@@ -537,13 +606,18 @@ class GeneratorEngine(_Net):
                 continue
             ops.conv_gemm([self.A[j - 1]], self.w_d_fwd[j], g_s2, self.yd[j], C[j], S[j], stats=bn.stats)
             self._bn_forward(bn, self.yd[j], self.A[j], ACT_LRELU, self.R[j][..., :C[j]], ACT_RELU, bn_repeat)
-        ops.conv_gemm([self.A[L - 2]], self.w_d_fwd[L - 1], g_s2, self.Rin, C[L - 1], S[L - 1], act=ACT_RELU)
+        ops.conv_gemm([self.A[L - 2]], self.w_d_fwd[L - 1], g_s2, self.Rin, C[L - 1], S[L - 1], act=ACT_RELU,
+                      bias=bias(self.k_down[L - 1]))
         for j in range(L - 1, 0, -1):
             src = self.Rin if j == L - 1 else self.R[j]
             bn = self.ubn[j]
             # the parent's in-place ReLU (models.py:180) acts on the concatenated tensor; a stand-alone block returns
             # its up-norm output un-activated
             dst, act = (self.out_cat[..., C[0]:], ACT_NONE) if (v0 and j == 1) else (self.R[j - 1][..., C[j - 1]:], ACT_RELU)
+            if inst:
+                ops.conv_gemm([src], self.w_u_fwd[j], g_ph, self.yu[j], C[j - 1], S[j], bias=bias(self.k_up[j]))
+                self._in_forward(bn, self.yu[j], dst, act)
+                continue
             if not self.training:
                 self._bn_eval(bn)
                 ops.conv_gemm([src], self.w_u_fwd[j], g_ph, dst, C[j - 1], S[j], act=act, scale=bn.scale, bias=bn.shift)
@@ -600,16 +674,24 @@ class GeneratorEngine(_Net):
             ops.thin_conv_fwd(self.dpre, None, self.w_u_thin, None, self.gR[0])
         # up path, outer -> inner.  Every dgrad GEMM applies the activation backward of the layer below in its
         # epilogue and accumulates that layer's BatchNorm-backward sums (no separate reduce pass).
+        inst = self.norm == "instance"
         for j in range(1, L):
             bn = self.ubn[j]
             co = C[j - 1]
-            if self._dropout_layer(j):
-                ops.dropout_(self.gR[j - 1][..., co:], 0.5, self.dropout_seed, self._drop_off[j])   # same mask as forward
-            if j == 1 or self._dropout_layer(j):      # gR[0] comes from the thin-layer kernel: classic reduce + apply
-                # (slope 1: a stand-alone block's up-norm output is not followed by the parent's ReLU)
-                self._bn_backward(bn, self.yu[j], self.gR[j - 1][..., co:], None, 1.0 if (v0 and j == 1) else 0.0, self.dyu[j])
+            if inst:
+                # InstanceNorm: the dgrad below wrote the raw gradient of ReLU(IN(yu[j])); reduce + apply here
+                self._in_backward(bn, self.yu[j], self.gR[j - 1][..., co:], None, 1.0 if (v0 and j == 1) else 0.0,
+                                  self.dyu[j], self.grad(self.k_up[j] + ".bias"))
+                self._ready(self.k_up[j] + ".bias")
             else:
-                self._bn_backward_fused(bn, self.yu[j], self.gR[j - 1][..., co:], self.dyu[j])
+                if self._dropout_layer(j):
+                    ops.dropout_(self.gR[j - 1][..., co:], 0.5, self.dropout_seed, self._drop_off[j])   # same mask as forward
+                if j == 1 or self._dropout_layer(j):      # gR[0] comes from the thin-layer kernel: classic reduce + apply
+                    # (slope 1: a stand-alone block's up-norm output is not followed by the parent's ReLU)
+                    self._bn_backward(bn, self.yu[j], self.gR[j - 1][..., co:], None, 1.0 if (v0 and j == 1) else 0.0,
+                                      self.dyu[j])
+                else:
+                    self._bn_backward_fused(bn, self.yu[j], self.gR[j - 1][..., co:], self.dyu[j])
             src = self.Rin if j == L - 1 else self.R[j]
             ci = src.shape[-1]
             self._fork_wgrad(lambda src=src, j=j, co=co: ops.conv_wgrad(
@@ -619,8 +701,9 @@ class GeneratorEngine(_Net):
                 # innermost: Rin = ReLU(conv) has no BatchNorm -> the epilogue writes dyd[L-1] directly
                 ops.conv_gemm([self.dyu[j]], self.w_u_dg[j], g_s2, self.dyd[L - 1], ci, S[j],
                               bwd=self._bwd_epilogue(None, self.Rin, 0.0))
-            elif self._dropout_layer(j + 1):
-                # the dropout mask has to hit the gradient before the ReLU / BatchNorm backward: plain dgrad here
+            elif inst or self._dropout_layer(j + 1):
+                # the dropout mask has to hit the gradient before the ReLU / BatchNorm backward, and InstanceNorm's
+                # per-image sums do not fit the epilogue: plain dgrad here
                 ops.conv_gemm([self.dyu[j]], self.w_u_dg[j], g_s2, self.gR[j], ci, S[j])
             else:
                 nb = self.ubn[j + 1]     # second half of gR[j] = gradient at ReLU(BN(yu[j+1]))
@@ -630,9 +713,17 @@ class GeneratorEngine(_Net):
             self._fork_wgrad(lambda j=j: ops.conv_wgrad(
                 self.dyd[j], self.A[j - 1], gseg(self.k_down[j] + ".weight"), (4, 4), 2, (-1, -1), 16 * C[j - 1], C[j - 1]))
             self._ready(self.k_down[j] + ".weight", side=True)
+            if inst and j == L - 1:       # innermost down conv: ReLU without a norm, its bias gradient is a column sum
+                self._fork_wgrad(lambda: ops.colsum_bf16(self.dyd[L - 1], C[L - 1], self.grad(self.k_down[L - 1] + ".bias")))
+                self._ready(self.k_down[L - 1] + ".bias", side=True)
             jj = j - 1
             skip = self.gR[jj][..., :C[jj]]          # gradient through the ReLU'd skip copy (models.py:208)
-            if jj >= 1:
+            if jj >= 1 and inst:
+                ops.conv_gemm([self.dyd[j]], self.w_d_dg[j], g_ph, self.gA[jj], C[jj], S[j])
+                self._in_backward(self.dbn[jj], self.yd[jj], self.gA[jj], skip, 0.2, self.dyd[jj],
+                                  self.grad(self.k_down[jj] + ".bias"))
+                self._ready(self.k_down[jj] + ".bias")
+            elif jj >= 1:
                 bn = self.dbn[jj]
                 ops.conv_gemm([self.dyd[j]], self.w_d_dg[j], g_ph, self.gA[jj], C[jj], S[j], stats=bn.sums,
                               bwd=self._bwd_epilogue(bn, self.yd[jj], 0.2, g2=skip))
@@ -648,15 +739,17 @@ class GeneratorEngine(_Net):
                               bwd=self._bwd_epilogue(None, self.A[0], 0.2, g2=skip))
         if v0:
             return
-        self._fork_wgrad(lambda: ops.thin_conv_wgrad(self.dyd[0], self.x_nhwc, None, gseg(self.k_down[0] + ".weight"), 64))
-        self._ready(self.k_down[0] + ".weight", side=True)
+        dbias0 = self.grad(self.k_down[0] + ".bias") if inst else None
+        self._fork_wgrad(lambda: ops.thin_conv_wgrad(self.dyd[0], self.x_nhwc, None, gseg(self.k_down[0] + ".weight"), 64,
+                                                     dbias=dbias0))
+        self._ready(self.k_down[0] + ".weight", *((self.k_down[0] + ".bias",) if inst else ()), side=True)
 
 
 # ================================================================================================
 # Discriminator
 # ================================================================================================
 class DiscriminatorEngine(_Net):
-    """NLayerDiscriminator(input_nc=6, ndf, n_layers, BatchNorm2d)."""
+    """NLayerDiscriminator(input_nc=6, ndf, n_layers, BatchNorm2d or InstanceNorm2d)."""
 
     # BatchNorm + LeakyReLU of the last normalised layer (models.py:239-240) applied inside the Cout = 1 head's forward
     # and wgrad kernels instead of a separate pass that writes H (63 MB written + re-read per forward at batch 64)
@@ -664,13 +757,17 @@ class DiscriminatorEngine(_Net):
 
     _BUFFER_ATTRS = ("hs", "ws", "H", "y", "logits", "z_ws", "dlogits", "gH", "dy", "dfake", "_xa", "_xb")
 
-    def __init__(self, device, input_nc: int = 6, ndf: int = 64, n_layers: int = 3, init: bool = True) -> None:
-        super().__init__(device)
+    def __init__(self, device, input_nc: int = 6, ndf: int = 64, n_layers: int = 3, init: bool = True,
+                 norm: str = "batch") -> None:
+        super().__init__(device, norm)
+        if self.norm == "instance":
+            # the head's kernels take per-channel (scale, shift) only; InstanceNorm's are per image: H is materialised
+            self.fuse_head = False
         if input_nc != 6:
             raise NotImplementedError("the native discriminator supports input_nc = 6 (cat of two RGB images)")
         if ndf % 64 != 0 or n_layers < 1:
             raise NotImplementedError("ndf must be a multiple of 64")
-        self.spec = sp = DiscriminatorSpec(input_nc, ndf, n_layers)
+        self.spec = sp = DiscriminatorSpec(input_nc, ndf, n_layers, norm=self.norm)
         self.nl = n_layers
         self.C = C = sp.C
         self.k_conv, self.k_bn, self.n_conv = sp.k_conv, sp.k_bn, sp.n_conv
@@ -679,7 +776,7 @@ class DiscriminatorEngine(_Net):
         self.bn: List[Optional[_BN]] = [None] * self.n_conv
         for k in range(1, n_layers + 1):
             self._reg_conv(self.k_conv[k] + ".weight", C[k], C[k - 1])
-            self.bn[k] = self._reg_bn(self.k_bn[k], C[k])
+            self.bn[k] = (self._reg_in if self.norm == "instance" else self._reg_bn)(self.k_bn[k], C[k])
         self._reg_conv(self.k_conv[-1] + ".weight", 1, C[-1])
         self._reg_vec(self.k_conv[-1] + ".bias", 1)
         self.store.allocate(device)
@@ -765,6 +862,8 @@ class DiscriminatorEngine(_Net):
         self.gH = [torch.empty(n, hs[k], ws[k], C[k], **bf) for k in range(self.n_conv - 1)]
         self.dy = [torch.empty(n, hs[k], ws[k], C[k], **bf) for k in range(self.n_conv - 1)]
         self.dfake = torch.zeros(n, h, w, 4, device=self.dev)
+        for m in self.ins.values():
+            m.allocate(n, self.dev)
         self._n = (n, h, w, self.fuse_head)
         self.alloc_gen += 1
 
@@ -778,11 +877,14 @@ class DiscriminatorEngine(_Net):
         C = self.C
         self._xa, self._xb = xa, xb
         ops.thin_conv_fwd(xa, xb, self.w_thin, self.param(self.k_conv[0] + ".bias"), self.H[0], ACT_LRELU)
+        inst = self.norm == "instance"
         for k in range(1, self.n_conv - 1):
             bn = self.bn[k]
             ops.conv_gemm([self.H[k - 1]], self.w_fwd[k], ops.geom_conv_fwd(4, self.stride(k), 1), self.y[k], C[k],
-                          (self.hs[k], self.ws[k]), stats=bn.stats if self.training else None)
-            if self.H[k] is None:
+                          (self.hs[k], self.ws[k]), stats=bn.stats if (self.training and not inst) else None)
+            if inst:
+                self._in_forward(bn, self.y[k], self.H[k], ACT_LRELU)
+            elif self.H[k] is None:
                 self._bn_scale_shift(bn, self.y[k])          # applied by the head's kernels on the fly
             else:
                 self._bn_forward(bn, self.y[k], self.H[k], ACT_LRELU)
@@ -816,11 +918,18 @@ class DiscriminatorEngine(_Net):
                                                               pre=(lb.scale, lb.shift, 0.2)))
             else:
                 self._fork_wgrad(lambda: ops.cout1_conv_wgrad(self.dlogits, self.H[last - 1], wseg))
-        # the Cout = 1 dgrad kernel applies the LeakyReLU backward of the last BatchNorm layer and accumulates its sums
-        ops.cout1_conv_dgrad(self.dlogits, self.w_fwd[last].view(-1), self.gH[last - 1],
-                             bwd=dict(y=self.y[last - 1], scale=lb.scale, shift=lb.shift, slope=0.2, sums=lb.sums))
+        inst = self.norm == "instance"
+        if inst:        # plain input gradient of H; the InstanceNorm backward below applies the LeakyReLU backward
+            ops.cout1_conv_dgrad(self.dlogits, self.w_fwd[last].view(-1), self.gH[last - 1])
+        else:
+            # the Cout = 1 dgrad kernel applies the LeakyReLU backward of the last BatchNorm layer and accumulates its sums
+            ops.cout1_conv_dgrad(self.dlogits, self.w_fwd[last].view(-1), self.gH[last - 1],
+                                 bwd=dict(y=self.y[last - 1], scale=lb.scale, shift=lb.shift, slope=0.2, sums=lb.sums))
         for k in range(last - 1, 0, -1):
-            self._bn_backward_fused(self.bn[k], self.y[k], self.gH[k], self.dy[k], param_grads=wgrad)
+            if inst:
+                self._in_backward(self.bn[k], self.y[k], self.gH[k], None, 0.2, self.dy[k])
+            else:
+                self._bn_backward_fused(self.bn[k], self.y[k], self.gH[k], self.dy[k], param_grads=wgrad)
             s = self.stride(k)
             if wgrad:
                 self._fork_wgrad(lambda k=k, s=s: ops.conv_wgrad(
@@ -833,7 +942,9 @@ class DiscriminatorEngine(_Net):
             # algorithmic FLOPs of a dgrad = those of the layer's forward (the stride-1 dgrad runs its GEMM over the
             # 32x32 input grid with zero-padded borders: 6.6 % more MMA work than the 31x31 forward, not counted)
             fl = 2.0 * self.dy[k].shape[0] * self.hs[k] * self.ws[k] * C[k] * C[k - 1] * 16
-            if k - 1 >= 1:
+            if k - 1 >= 1 and inst:
+                ops.conv_gemm([self.dy[k]], self.w_dg[k], geom, self.gH[k - 1], C[k - 1], grid, flops=fl)
+            elif k - 1 >= 1:
                 nb = self.bn[k - 1]
                 ops.conv_gemm([self.dy[k]], self.w_dg[k], geom, self.gH[k - 1], C[k - 1], grid, stats=nb.sums,
                               bwd=self._bwd_epilogue(nb, self.y[k - 1], 0.2), flops=fl)
@@ -864,11 +975,14 @@ class Pix2PixTrainer:
 
     def __init__(self, device, lr_g: float = 1e-4, lr_d: float = 1e-4, beta1: float = 0.5, num_downs: int = 7,
                  ngf: int = 64, ndf: int = 64, n_layers: int = 3, allreduce=None, world: int = 1,
-                 bucket_elems: int = 8 << 20, use_dropout: bool = False) -> None:
+                 bucket_elems: int = 8 << 20, use_dropout: bool = False, norm: str = "batch") -> None:
+        """norm: "batch" (nn.BatchNorm2d, the reference default) or "instance" (nn.InstanceNorm2d, pix2pix's
+        `--norm instance`) in both networks."""
         self.dev = torch.device(device)
+        self.norm = norm
         # construction order G then D fixes the seeded weights (train_gan.py:138-139)
-        self.G = GeneratorEngine(self.dev, 3, 3, num_downs, ngf, use_dropout=use_dropout)
-        self.D = DiscriminatorEngine(self.dev, 6, ndf, n_layers)
+        self.G = GeneratorEngine(self.dev, 3, 3, num_downs, ngf, use_dropout=use_dropout, norm=norm)
+        self.D = DiscriminatorEngine(self.dev, 6, ndf, n_layers, norm=norm)
         self.lr_g, self.lr_d, self.betas = lr_g, lr_d, (beta1, 0.999)
         self.loss_acc = torch.zeros(4, device=self.dev, dtype=torch.float64)  # d_real, d_fake, g_gan, l1 (re-zeroed by
         self.loss_out = torch.zeros(2, device=self.dev, dtype=torch.float64)  # gap_gan_losses at the end of each step)

@@ -9,6 +9,13 @@ from typing import Dict, List, Optional
 import torch
 
 BN_LEAVES = ["weight", "bias", "running_mean", "running_var", "num_batches_tracked"]
+NORMS = ("batch", "instance")   # nn.BatchNorm2d | nn.InstanceNorm2d(affine=False, track_running_stats=False)
+
+
+def _check_norm(norm: str) -> str:
+    if norm not in NORMS:
+        raise ValueError(f"norm must be one of {NORMS}, got {norm!r}")
+    return norm
 
 
 def _kaiming_uniform_(t: torch.Tensor) -> None:
@@ -31,16 +38,20 @@ def _bn_entries(sd: Dict[str, torch.Tensor], prefix: str, c: int) -> None:
 
 
 class GeneratorSpec:
-    """UNetGenerator(input_nc, output_nc, num_downs, ngf) with BatchNorm2d, no dropout (models.py:149-208).
+    """UNetGenerator(input_nc, output_nc, num_downs, ngf) with BatchNorm2d or InstanceNorm2d, no dropout
+    (models.py:149-208).
 
     Block j (0 = outermost ... L-1 = innermost) owns down conv `k_down[j]` (C[j-1] -> C[j]) and up
     conv `k_up[j]` (2*C[j] or C[j] -> C[j-1]); down norm `k_dbn[j]` exists for 1 <= j <= L-2, up norm
-    `k_ubn[j]` for 1 <= j <= L-1."""
+    `k_ubn[j]` for 1 <= j <= L-1.  norm="instance": the norms hold no state, and every conv has a bias
+    (use_bias, models.py:173-176)."""
 
     def __init__(self, input_nc: int = 3, output_nc: int = 3, num_downs: int = 7, ngf: int = 64,
-                 C: Optional[List[int]] = None, root: str = "model.model", virtual0: bool = False) -> None:
+                 C: Optional[List[int]] = None, root: str = "model.model", virtual0: bool = False,
+                 norm: str = "batch") -> None:
         """`C`, `root`, `virtual0` describe a stand-alone UnetSkipConnectionBlock chain (see `for_block_chain`);
         by default the layout is UNetGenerator's."""
+        self.norm = _check_norm(norm)
         if C is None:
             if num_downs < 5:
                 raise ValueError("UNetGenerator needs num_downs >= 5 (models.py:155-161)")
@@ -69,7 +80,7 @@ class GeneratorSpec:
             raise ValueError("a U-Net needs at least one nested block")
 
     @classmethod
-    def for_block_chain(cls, chain) -> "GeneratorSpec":
+    def for_block_chain(cls, chain, norm: str = "batch") -> "GeneratorSpec":
         """Layout of a stand-alone UnetSkipConnectionBlock (models.py:167-208) and the blocks nested inside it.
         `chain` lists (outer_nc, inner_nc, input_nc, outermost, innermost) from the called block inwards."""
         outer0, inner0, in0, outermost0, _ = chain[0]
@@ -80,10 +91,10 @@ class GeneratorSpec:
             elif nxt[0] != i or nxt[2] != i or nxt[3]:
                 raise NotImplementedError("nested blocks must chain outer_nc == input_nc == the parent's inner_nc")
         if outermost0:
-            return cls(in0, outer0, C=[c[1] for c in chain], root="model")
+            return cls(in0, outer0, C=[c[1] for c in chain], root="model", norm=norm)
         if in0 != outer0:
             raise NotImplementedError("a stand-alone inner block needs input_nc == outer_nc (the reference's default)")
-        return cls(in0, outer0, C=[in0] + [c[1] for c in chain], root="model", virtual0=True)
+        return cls(in0, outer0, C=[in0] + [c[1] for c in chain], root="model", virtual0=True, norm=norm)
 
     def down_shape(self, j: int):
         return (self.C[j], self.input_nc if j == 0 else self.C[j - 1], 4, 4)
@@ -95,37 +106,46 @@ class GeneratorSpec:
     def key_order(self) -> List[str]:
         """state_dict() order of the reference module: depth-first through the nested Sequentials."""
         L = self.L
+        inst = self.norm == "instance"
+        conv = lambda k, bias: [k + ".weight"] + ([k + ".bias"] if bias else [])
+        norm = lambda k: [] if inst else [k + "." + l for l in BN_LEAVES]
 
         def block(j: int) -> List[str]:
             if j == 0:
                 if self.virtual0:
                     return block(1)
-                return [self.k_down[0] + ".weight"] + block(1) + [self.k_up[0] + ".weight", self.k_up[0] + ".bias"]
-            keys = [self.k_down[j] + ".weight"]
+                return conv(self.k_down[0], inst) + block(1) + conv(self.k_up[0], True)
+            keys = conv(self.k_down[j], inst)
             if j < L - 1:
-                keys += [self.k_dbn[j] + "." + l for l in BN_LEAVES]
+                keys += norm(self.k_dbn[j])
                 keys += block(j + 1)
-            keys.append(self.k_up[j] + ".weight")
-            keys += [self.k_ubn[j] + "." + l for l in BN_LEAVES]
+            keys += conv(self.k_up[j], inst)
+            keys += norm(self.k_ubn[j])
             return keys
 
         return block(0)
 
     def default_state_dict(self) -> Dict[str, torch.Tensor]:
         """Default torch init consuming the global CPU RNG exactly like UNetGenerator.__init__: blocks are
-        built innermost first (models.py:155-161); within a block downconv, then upconv (+bias)."""
+        built innermost first (models.py:155-161); within a block downconv (+bias with InstanceNorm), then upconv
+        (+bias).  InstanceNorm2d(affine=False) draws nothing and has no entries."""
         sd: Dict[str, torch.Tensor] = {}
-        for j in range(self.L - 1, 0 if self.virtual0 else -1, -1):
-            w = torch.empty(*self.down_shape(j))
+        inst = self.norm == "instance"
+
+        def conv(key: str, shape, bias: bool) -> None:
+            w = torch.empty(*shape)
             _kaiming_uniform_(w)
-            sd[self.k_down[j] + ".weight"] = w
-            u = torch.empty(*self.up_shape(j))
-            _kaiming_uniform_(u)
-            sd[self.k_up[j] + ".weight"] = u
-            if j == 0:
-                b = torch.empty(self.output_nc)
-                _bias_uniform_(b, u)
-                sd[self.k_up[0] + ".bias"] = b
+            sd[key + ".weight"] = w
+            if bias:
+                b = torch.empty(shape[1] if key in self.k_up else shape[0])
+                _bias_uniform_(b, w)
+                sd[key + ".bias"] = b
+
+        for j in range(self.L - 1, 0 if self.virtual0 else -1, -1):
+            conv(self.k_down[j], self.down_shape(j), inst)
+            conv(self.k_up[j], self.up_shape(j), inst or j == 0)
+            if inst:
+                continue
             if self.k_dbn[j] is not None:
                 _bn_entries(sd, self.k_dbn[j], self.C[j])
             if self.k_ubn[j] is not None:
@@ -134,10 +154,12 @@ class GeneratorSpec:
 
 
 class DiscriminatorSpec:
-    """NLayerDiscriminator(input_nc, ndf, n_layers) with BatchNorm2d (models.py:212-247)."""
+    """NLayerDiscriminator(input_nc, ndf, n_layers) with BatchNorm2d or InstanceNorm2d (models.py:212-247).  The middle
+    convs have no bias with either norm (use_bias = False, models.py:221)."""
 
-    def __init__(self, input_nc: int = 6, ndf: int = 64, n_layers: int = 3) -> None:
+    def __init__(self, input_nc: int = 6, ndf: int = 64, n_layers: int = 3, norm: str = "batch") -> None:
         self.input_nc, self.ndf, self.nl = input_nc, ndf, n_layers
+        self.norm = _check_norm(norm)
         self.C = [ndf * min(2 ** k, 8) for k in range(n_layers + 1)]
         idx = [0] + [2 + 3 * (k - 1) for k in range(1, n_layers + 2)]
         self.n_conv = n_layers + 2
@@ -161,7 +183,7 @@ class DiscriminatorSpec:
             keys.append(self.k_conv[k] + ".weight")
             if self.has_bias(k):
                 keys.append(self.k_conv[k] + ".bias")
-            else:
+            elif self.norm == "batch":
                 keys += [self.k_bn[k] + "." + l for l in BN_LEAVES]
         return keys
 
@@ -175,15 +197,15 @@ class DiscriminatorSpec:
                 b = torch.empty(w.size(0))
                 _bias_uniform_(b, w)
                 sd[self.k_conv[k] + ".bias"] = b
-            else:
+            elif self.norm == "batch":
                 _bn_entries(sd, self.k_bn[k], self.C[k])
         return {k: sd[k] for k in self.key_order()}
 
 
-def default_state_dicts(num_downs: int = 7, ngf: int = 64, ndf: int = 64, n_layers: int = 3):
+def default_state_dicts(num_downs: int = 7, ngf: int = 64, ndf: int = 64, n_layers: int = 3, norm: str = "batch"):
     """G then D, the construction order of train_gan.py:138-139 (defines the seeded weights)."""
-    g = GeneratorSpec(3, 3, num_downs, ngf).default_state_dict()
-    d = DiscriminatorSpec(6, ndf, n_layers).default_state_dict()
+    g = GeneratorSpec(3, 3, num_downs, ngf, norm=norm).default_state_dict()
+    d = DiscriminatorSpec(6, ndf, n_layers, norm=norm).default_state_dict()
     return g, d
 
 

@@ -346,6 +346,26 @@ int gap_bn_bwd_finalize(double* raw, const float* mean, const float* invstd, int
 /* bias gradient: out[c] += sum over pixels of x[pixel][c] */
 int gap_colsum_bf16(const void* x, int64_t ld, int64_t pixels, int c, float* out, void* stream);
 
+/* nn.InstanceNorm2d(affine=False, track_running_stats=False) (models.py:173-191 with norm_layer=nn.InstanceNorm2d):
+ * statistics per (image, channel) over hw = H*W >= 2 pixels, the same in train and eval mode (instance_norm.cu).
+ * y / g1 / g2 / outputs are NHWC bf16 [n][hw][>= c] with pixel strides that are multiples of 8, c % 8 == 0, c <= 2048.
+ * Per-(n,c) vectors are [N][C]; fp64 sums are [2][N*C], so gap_bn_finalize(sums, N*C, H*W, NULL, NULL, eps, 0, 1, NULL,
+ * NULL, NULL, scale, shift, mean, invstd) turns the forward sums into scale = invstd, shift = -mean*invstd (and re-zeroes
+ * them); gap_bn_param_grads(sums, N*C, NULL, NULL) re-zeroes the backward sums after gap_in_bwd_apply. */
+/* sums[0][n*C+c] += sum y, sums[1][n*C+c] += sum y^2 */
+int gap_in_stats(const void* y, int64_t ld, int n, int64_t hw, int c, double* sums, void* stream);
+/* out1 = act1(y*scale[n][c] + shift[n][c]), out2 = act2(same) (optional); act = NONE / LRELU / RELU */
+int gap_in_act(const void* y, int64_t ld, int n, int64_t hw, int c, const float* scale, const float* shift, void* out1,
+               int64_t ld1, int act1, void* out2, int64_t ld2, int act2, void* stream);
+/* xhat = y*scale + shift; d = xhat > 0 ? g1 + g2 : slope*g1 (g2 optional); sums[0] += sum d, sums[1] += sum d*xhat */
+int gap_in_bwd_reduce(const void* y, int64_t ld, const void* g1, int64_t ld_g1, const void* g2, int64_t ld_g2, float slope,
+                      const float* scale, const float* shift, int n, int64_t hw, int c, double* sums, void* stream);
+/* dy = scale * (d - sums[0]/hw - xhat*sums[1]/hw) (bf16); dbias (optional) += the per-channel sum of the fp32 dy over
+ * all images and pixels: the gradient of a conv bias in front of the norm */
+int gap_in_bwd_apply(const void* y, int64_t ld, const void* g1, int64_t ld_g1, const void* g2, int64_t ld_g2, float slope,
+                     const float* scale, const float* shift, int n, int64_t hw, int c, const double* sums, void* dy,
+                     int64_t ld_dy, float* dbias, void* stream);
+
 /* optim.Adam / optim.AdamW step on a flat fp32 buffer (train_gan.py:140-141,63,71; train.py:295,144).
  * grad_scale folds the 1/world_size of the data-parallel gradient all-reduce. */
 int gap_adam_flat(float* p, const float* g, float* m, float* v, int64_t n, float lr, float beta1, float beta2,
