@@ -102,11 +102,16 @@ _SIGNATURES = {
     "gap_cout1_conv_wgrad": (C.c_int, [_P, _I, _I, _I, _P, _L, _I, _I, _I, _I, _I, _P, _P, _P, _F, _P]),
     "gap_thin_conv_fwd": (C.c_int, [_P, _L, _P, _L, _I, _I, _I, _P, _P, _I, _P, _L, _I, _P, _L, _I, _P]),
     "gap_thin_conv_wgrad": (C.c_int, [_P, _L, _P, _L, _P, _L, _I, _I, _I, _I, _P, _L, _P, _P]),
+    "gap_thin_conv_wgrad_c": (C.c_int, [_P, _L, _P, _L, _I, _P, _L, _I, _I, _I, _I, _I, _P, _L, _P, _P]),
     "gap_thin_convT_fwd": (C.c_int, [_P, _L, _I, _I, _I, _I, _P, _P, _I, _P, _L, _P, _L, _P, _P]),
+    "gap_thin_convT_fwd_c": (C.c_int, [_P, _L, _I, _I, _I, _I, _I, _P, _P, _I, _P, _L, _P, _L, _P, _P]),
     "gap_u8_hwc_to_nhwc_bf16": (C.c_int, [_P, _P, _L, _L, _P]),
+    "gap_u8_hwc_to_nhwc_bf16_c": (C.c_int, [_P, _I, _P, _L, _L, _P]),
     "gap_resize_u8_to_nhwc_bf16": (C.c_int, [_P, _I, _I, _I, _I, _I, _P, _L, _P, _P]),
+    "gap_resize_u8_to_nhwc_bf16_c": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _P, _L, _P, _P]),
     "gap_resize_nearest_i64": (C.c_int, [_P, _I, _I, _I, _I, _I, _P, _P]),
     "gap_im2col_k3s1p1_c3": (C.c_int, [_P, _L, _P, _I, _I, _I, _P]),
+    "gap_im2col_k3s1p1_c": (C.c_int, [_P, _L, _I, _P, _I, _I, _I, _P]),
     "gap_maxpool2x2_fwd": (C.c_int, [_P, _L, _P, _L, _I, _I, _I, _I, _P]),
     "gap_maxpool2x2_bwd": (C.c_int, [_P, _L, _P, _L, _P, _L, _I, _I, _I, _I, _I, _P]),
     "gap_upsample_bilinear2x_fwd": (C.c_int, [_P, _L, _P, _L, _I, _I, _I, _I, _P]),

@@ -57,7 +57,9 @@ def _set_rng_state(d: dict, device) -> None:
 def trainer_state(trainer, extra: Optional[dict] = None) -> dict:
     """Everything needed to continue a Pix2PixTrainer run as if it had never stopped."""
     torch.cuda.synchronize(trainer.dev)
-    return {"format": FORMAT, "kind": "pix2pix", "norm": trainer.norm, "G": _net_state(trainer.G), "D": _net_state(trainer.D),
+    return {"format": FORMAT, "kind": "pix2pix", "norm": trainer.norm,
+            "channels": {"input_nc": trainer.input_nc, "output_nc": trainer.output_nc},
+            "G": _net_state(trainer.G), "D": _net_state(trainer.D),
             "hyper": {"lr_g": trainer.lr_g, "lr_d": trainer.lr_d, "betas": list(trainer.betas)},
             "dropout": {"seed": trainer.G.dropout_seed, "calls": trainer.G.dropout_calls},
             "rng": _rng_state(trainer.dev), "extra": extra or {}}
@@ -69,6 +71,12 @@ def load_trainer_state(trainer, state: dict, restore_rng: bool = True) -> dict:
     norm = state.get("norm", "batch")       # checkpoints written before InstanceNorm support are BatchNorm runs
     if norm != trainer.norm:
         raise ValueError(f"checkpoint was written by a norm={norm!r} trainer; this trainer uses norm={trainer.norm!r}")
+    # checkpoints written before channel counts were recorded are 3 -> 3 runs
+    ch = state.get("channels", {"input_nc": 3, "output_nc": 3})
+    mine = {"input_nc": trainer.input_nc, "output_nc": trainer.output_nc}
+    if ch != mine:
+        raise ValueError(f"checkpoint was written by a trainer with input_nc={ch['input_nc']}, output_nc={ch['output_nc']}; "
+                         f"this trainer has input_nc={mine['input_nc']}, output_nc={mine['output_nc']}")
     _load_net(trainer.G, state["G"])
     _load_net(trainer.D, state["D"])
     trainer.lr_g, trainer.lr_d = state["hyper"]["lr_g"], state["hyper"]["lr_d"]
@@ -83,13 +91,17 @@ def load_trainer_state(trainer, state: dict, restore_rng: bool = True) -> dict:
 
 def siamese_state(engine, extra: Optional[dict] = None) -> dict:
     torch.cuda.synchronize(engine.dev)
-    return {"format": FORMAT, "kind": "siamese", "net": _net_state(engine), "rng": _rng_state(engine.dev),
-            "extra": extra or {}}
+    return {"format": FORMAT, "kind": "siamese", "channels": {"n_channels": engine.n_channels}, "net": _net_state(engine),
+            "rng": _rng_state(engine.dev), "extra": extra or {}}
 
 
 def load_siamese_state(engine, state: dict, restore_rng: bool = True) -> dict:
     if state.get("format") != FORMAT or state.get("kind") != "siamese":
         raise ValueError("not a gap_b200 siamese checkpoint")
+    ch = state.get("channels", {"n_channels": 3}).get("n_channels", 3)
+    if ch != engine.n_channels:
+        raise ValueError(f"checkpoint was written by a Siamese U-Net with n_channels={ch}; this one has "
+                         f"n_channels={engine.n_channels}")
     _load_net(engine, state["net"])
     if restore_rng:
         _set_rng_state(state["rng"], engine.dev)

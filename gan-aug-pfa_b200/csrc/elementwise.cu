@@ -52,24 +52,28 @@ __global__ void nchw_f32_to_nhwc_bf16_kernel(const float* __restrict__ x, __nv_b
   }
 }
 
-// 3 channels into 4-slot pixels (the image inputs of both networks), 4 pixels per thread: three 16-byte plane loads and
-// one 32-byte store instead of 12 scalar loads and 12 two-byte stores (the scalar version ran at 2 TB/s).
-__global__ void nchw3_f32_to_nhwc4_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, long long hw4,
-                                               long long total4) {
+// 1..4 channels into 4-slot pixels (the image inputs of both networks), 4 pixels per thread: C 16-byte plane loads and
+// one 32-byte store instead of 4C scalar loads and 4C two-byte stores (the scalar version ran at 2 TB/s).  Slots >= C are
+// written as zero.
+template <int C>
+__global__ void nchw_f32_to_nhwc4_bf16_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ out, long long hw4,
+                                              long long total4) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total4;
        i += (long long)gridDim.x * blockDim.x) {
     const long long img = i / hw4, q = i - img * hw4;
-    const float4* base = reinterpret_cast<const float4*>(x) + img * 3 * hw4 + q;
-    const float4 r = __ldg(base), g = __ldg(base + hw4), b = __ldg(base + 2 * hw4);
+    const float4* base = reinterpret_cast<const float4*>(x) + img * C * hw4 + q;
+    float4 v[4];
+#pragma unroll
+    for (int ch = 0; ch < 4; ++ch) v[ch] = ch < C ? __ldg(base + ch * hw4) : make_float4(0.f, 0.f, 0.f, 0.f);
     uint4 lo, hi;
-    lo.x = pack_bf16x2(r.x, g.x);
-    lo.y = pack_bf16x2(b.x, 0.f);
-    lo.z = pack_bf16x2(r.y, g.y);
-    lo.w = pack_bf16x2(b.y, 0.f);
-    hi.x = pack_bf16x2(r.z, g.z);
-    hi.y = pack_bf16x2(b.z, 0.f);
-    hi.z = pack_bf16x2(r.w, g.w);
-    hi.w = pack_bf16x2(b.w, 0.f);
+    lo.x = pack_bf16x2(v[0].x, v[1].x);
+    lo.y = pack_bf16x2(v[2].x, v[3].x);
+    lo.z = pack_bf16x2(v[0].y, v[1].y);
+    lo.w = pack_bf16x2(v[2].y, v[3].y);
+    hi.x = pack_bf16x2(v[0].z, v[1].z);
+    hi.y = pack_bf16x2(v[2].z, v[3].z);
+    hi.z = pack_bf16x2(v[0].w, v[1].w);
+    hi.w = pack_bf16x2(v[2].w, v[3].w);
     uint4* o = reinterpret_cast<uint4*>(out + i * 16);
     o[0] = lo;
     o[1] = hi;
@@ -145,15 +149,15 @@ __global__ void gen_out_bwd_kernel(const float* __restrict__ fake, long long ld_
   }
 }
 
-// The same for the layout the trainer uses (3 channels in 4-slot NHWC tensors, hw % 4 == 0): four pixels per thread,
-// 128-bit loads of fake / dfake_d, the real image as three 32-bit words (uint8) or three float4 (fp32 planes), two 128-bit
-// stores (slot 3 is written as zero, which is what the slot holds), no per-pixel 64-bit division.  The per-pixel
-// scalar kernel above ran at 3.1 TB/s.
-template <bool REAL_U8>
-__global__ void __launch_bounds__(256) gen_out_bwd_c3_kernel(const float* __restrict__ fake, const void* __restrict__ real_v,
-                                                             long long hw, const float* __restrict__ dfake_d, float l1_scale,
-                                                             __nv_bfloat16* __restrict__ dpre, long long pixels,
-                                                             double* __restrict__ loss_acc) {
+// The same for the layout the trainer uses (C = 1..4 channels in 4-slot NHWC tensors, hw % 4 == 0): four pixels per
+// thread, 128-bit loads of fake / dfake_d, the real image as C 32-bit words (uint8) or C float4 (fp32 planes), two
+// 128-bit stores (slots >= C are written as zero, which is what they hold), no per-pixel 64-bit division.  The
+// per-pixel scalar kernel above ran at 3.1 TB/s.
+template <bool REAL_U8, int C>
+__global__ void __launch_bounds__(256) gen_out_bwd_vec_kernel(const float* __restrict__ fake, const void* __restrict__ real_v,
+                                                              long long hw, const float* __restrict__ dfake_d, float l1_scale,
+                                                              __nv_bfloat16* __restrict__ dpre, long long pixels,
+                                                              double* __restrict__ loss_acc) {
   float part = 0.f;
   const long long quads = pixels >> 2;
   for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < quads; q += (long long)gridDim.x * blockDim.x) {
@@ -165,18 +169,20 @@ __global__ void __launch_bounds__(256) gen_out_bwd_c3_kernel(const float* __rest
 #pragma unroll
       for (int k = 0; k < 4; ++k) dd[k] = __ldg(reinterpret_cast<const float4*>(dfake_d + (i + k) * 4));
     }
-    float r[4][3];
+    float r[4][C];
     if (REAL_U8) {
-      const uint32_t* rp = reinterpret_cast<const uint32_t*>(static_cast<const unsigned char*>(real_v) + i * 3);
-      const uint32_t w[3] = {__ldg(rp), __ldg(rp + 1), __ldg(rp + 2)};
+      const uint32_t* rp = reinterpret_cast<const uint32_t*>(static_cast<const unsigned char*>(real_v) + i * C);
+      uint32_t w[C];
 #pragma unroll
-      for (int b = 0; b < 12; ++b)
-        r[b / 3][b % 3] = (static_cast<float>((w[b >> 2] >> (8 * (b & 3))) & 0xffu) / 255.f) * 2.f - 1.f;
+      for (int k = 0; k < C; ++k) w[k] = __ldg(rp + k);
+#pragma unroll
+      for (int b = 0; b < 4 * C; ++b)
+        r[b / C][b % C] = (static_cast<float>((w[b >> 2] >> (8 * (b & 3))) & 0xffu) / 255.f) * 2.f - 1.f;
     } else {
       const long long img = i / hw, pix = i - img * hw;
-      const float* rp = static_cast<const float*>(real_v) + img * 3 * hw + pix;
+      const float* rp = static_cast<const float*>(real_v) + img * C * hw + pix;
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) {
+      for (int ch = 0; ch < C; ++ch) {
         const float4 v = __ldg(reinterpret_cast<const float4*>(rp + ch * hw));
         r[0][ch] = v.x; r[1][ch] = v.y; r[2][ch] = v.z; r[3][ch] = v.w;
       }
@@ -184,11 +190,11 @@ __global__ void __launch_bounds__(256) gen_out_bwd_c3_kernel(const float* __rest
     uint32_t pk[8];
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-      const float fv[3] = {f[k].x, f[k].y, f[k].z};
-      const float dv[3] = {dd[k].x, dd[k].y, dd[k].z};
-      float o[3];
+      const float fv[4] = {f[k].x, f[k].y, f[k].z, f[k].w};
+      const float dv[4] = {dd[k].x, dd[k].y, dd[k].z, dd[k].w};
+      float o[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
-      for (int ch = 0; ch < 3; ++ch) {
+      for (int ch = 0; ch < C; ++ch) {
         const float d = fv[ch] - r[k][ch];
         part += fabsf(d);
         float g = l1_scale * (d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f));
@@ -196,7 +202,7 @@ __global__ void __launch_bounds__(256) gen_out_bwd_c3_kernel(const float* __rest
         o[ch] = g * (1.f - fv[ch] * fv[ch]);
       }
       pk[2 * k] = pack_bf16x2(o[0], o[1]);
-      pk[2 * k + 1] = pack_bf16x2(o[2], 0.f);
+      pk[2 * k + 1] = pack_bf16x2(o[2], o[3]);
     }
     uint4* dst = reinterpret_cast<uint4*>(dpre + i * 4);
     dst[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
@@ -211,6 +217,19 @@ __global__ void __launch_bounds__(256) gen_out_bwd_c3_kernel(const float* __rest
     float v = lane < (blockDim.x >> 5) ? red[lane] : 0.f;
     v = warp_sum(v);
     if (lane == 0) atomicAdd(loss_acc, static_cast<double>(v));
+  }
+}
+
+template <bool REAL_U8>
+static void gen_out_bwd_vec_launch(const float* fake, const void* real, int64_t hw, const float* dfake_d, float l1_scale,
+                                   void* dpre, int64_t pixels, int c, double* loss_acc, cudaStream_t st) {
+  const int grid = grid_for(pixels / 4, 256, 148 * 8);
+  __nv_bfloat16* d = static_cast<__nv_bfloat16*>(dpre);
+  switch (c) {
+    case 1: gen_out_bwd_vec_kernel<REAL_U8, 1><<<grid, 256, 0, st>>>(fake, real, hw, dfake_d, l1_scale, d, pixels, loss_acc); break;
+    case 2: gen_out_bwd_vec_kernel<REAL_U8, 2><<<grid, 256, 0, st>>>(fake, real, hw, dfake_d, l1_scale, d, pixels, loss_acc); break;
+    case 3: gen_out_bwd_vec_kernel<REAL_U8, 3><<<grid, 256, 0, st>>>(fake, real, hw, dfake_d, l1_scale, d, pixels, loss_acc); break;
+    default: gen_out_bwd_vec_kernel<REAL_U8, 4><<<grid, 256, 0, st>>>(fake, real, hw, dfake_d, l1_scale, d, pixels, loss_acc); break;
   }
 }
 
@@ -864,12 +883,19 @@ int gap_nchw_f32_to_nhwc_bf16(const float* x, void* out, int n, int c, int h, in
                               void* stream) {
   GAP_CHECK_ARG(x && out && n > 0 && c > 0 && c <= out_ld, "gap_nchw_f32_to_nhwc_bf16: bad arguments");
   const long long hw = static_cast<long long>(h) * w;
-  if (c == 3 && out_ld == 4 && hw % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
+  if (c <= 4 && out_ld == 4 && hw % 4 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
       (reinterpret_cast<uintptr_t>(out) & 15) == 0) {
-    // (slot 3 is written as zero, which is what the 4-slot image layout holds there anyway)
+    // (slots >= c are written as zero, which is what the 4-slot image layout holds there anyway)
     const long long total4 = n * hw / 4;
-    nchw3_f32_to_nhwc4_bf16_kernel<<<grid_even(total4, 256, 148 * 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        x, static_cast<__nv_bfloat16*>(out), hw / 4, total4);
+    const int grid = grid_even(total4, 256, 148 * 8);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    __nv_bfloat16* o = static_cast<__nv_bfloat16*>(out);
+    switch (c) {
+      case 1: nchw_f32_to_nhwc4_bf16_kernel<1><<<grid, 256, 0, st>>>(x, o, hw / 4, total4); break;
+      case 2: nchw_f32_to_nhwc4_bf16_kernel<2><<<grid, 256, 0, st>>>(x, o, hw / 4, total4); break;
+      case 3: nchw_f32_to_nhwc4_bf16_kernel<3><<<grid, 256, 0, st>>>(x, o, hw / 4, total4); break;
+      default: nchw_f32_to_nhwc4_bf16_kernel<4><<<grid, 256, 0, st>>>(x, o, hw / 4, total4); break;
+    }
     GAP_LAUNCH_CHECK();
     return 0;
   }
@@ -905,12 +931,12 @@ int gap_tanh_bwd(const float* gout_nchw, const float* y_nhwc, int64_t ld_y, void
   return 0;
 }
 
-// the four-pixel kernel: 3 channels in dense 4-slot tensors, whole quads inside one image, 16-byte aligned pointers
-static bool gen_out_c3_ok(const void* fake, const void* real, const void* dfake_d, const void* dpre, int64_t ld_f,
-                          int64_t ld_d, int64_t ld_p, int64_t hw, int c) {
+// the four-pixel kernel: 1..4 channels in dense 4-slot tensors, whole quads inside one image, 16-byte aligned pointers
+static bool gen_out_vec_ok(const void* fake, const void* real, const void* dfake_d, const void* dpre, int64_t ld_f,
+                           int64_t ld_d, int64_t ld_p, int64_t hw, int c) {
   if (debug_get("gen_out_c3", 1) == 0) return false;
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-  return c == 3 && ld_f == 4 && ld_p == 4 && (!dfake_d || ld_d == 4) && hw % 4 == 0 && al16(fake) && al16(real) &&
+  return c <= 4 && ld_f == 4 && ld_p == 4 && (!dfake_d || ld_d == 4) && hw % 4 == 0 && al16(fake) && al16(real) &&
          al16(dfake_d) && al16(dpre);
 }
 
@@ -919,9 +945,9 @@ int gap_gen_out_bwd(const float* fake, int64_t ld_f, const float* real_nchw, int
                     double* loss_acc, void* stream) {
   GAP_CHECK_ARG(fake && real_nchw && dpre && loss_acc && pixels > 0 && c > 0 && hw > 0 && pixels % hw == 0,
                 "gap_gen_out_bwd: bad arguments");
-  if (gen_out_c3_ok(fake, real_nchw, dfake_d, dpre, ld_f, ld_d, ld_p, hw, c)) {
-    gen_out_bwd_c3_kernel<false><<<grid_for(pixels / 4, 256, 148 * 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        fake, real_nchw, hw, dfake_d, l1_scale, static_cast<__nv_bfloat16*>(dpre), pixels, loss_acc);
+  if (gen_out_vec_ok(fake, real_nchw, dfake_d, dpre, ld_f, ld_d, ld_p, hw, c)) {
+    gen_out_bwd_vec_launch<false>(fake, real_nchw, hw, dfake_d, l1_scale, dpre, pixels, c, loss_acc,
+                                  static_cast<cudaStream_t>(stream));
     GAP_LAUNCH_CHECK();
     return 0;
   }
@@ -937,9 +963,9 @@ int gap_gen_out_bwd_u8(const float* fake, int64_t ld_f, const uint8_t* real_hwc,
                        double* loss_acc, void* stream) {
   GAP_CHECK_ARG(fake && real_hwc && dpre && loss_acc && pixels > 0 && c > 0 && hw > 0 && pixels % hw == 0,
                 "gap_gen_out_bwd_u8: bad arguments");
-  if (gen_out_c3_ok(fake, real_hwc, dfake_d, dpre, ld_f, ld_d, ld_p, hw, c) && (reinterpret_cast<uintptr_t>(real_hwc) & 3) == 0) {
-    gen_out_bwd_c3_kernel<true><<<grid_for(pixels / 4, 256, 148 * 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
-        fake, real_hwc, hw, dfake_d, l1_scale, static_cast<__nv_bfloat16*>(dpre), pixels, loss_acc);
+  if (gen_out_vec_ok(fake, real_hwc, dfake_d, dpre, ld_f, ld_d, ld_p, hw, c) && (reinterpret_cast<uintptr_t>(real_hwc) & 3) == 0) {
+    gen_out_bwd_vec_launch<true>(fake, real_hwc, hw, dfake_d, l1_scale, dpre, pixels, c, loss_acc,
+                                 static_cast<cudaStream_t>(stream));
     GAP_LAUNCH_CHECK();
     return 0;
   }

@@ -40,12 +40,13 @@ __device__ __forceinline__ void block_sum_to(double* dst, float v) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// im2col of Conv2d(3 -> C, k3, s1, p1) (double_conv's first conv, models.py:9 via :54):
-//   col[pix][(kh*3+kw)*3 + c] = x[n, y-1+kh, x-1+kw, c]   (27 values, zero padded to 64)
+// im2col of Conv2d(C -> cout, k3, s1, p1), C = 1..4 (double_conv's first conv, models.py:9 via :54):
+//   col[pix][(kh*3+kw)*C + c] = x[n, y-1+kh, x-1+kw, c]   (9*C values, zero padded to 64)
 // x: NHWC bf16 with 4 channel slots per pixel.
 // ------------------------------------------------------------------------------------------------
-__global__ void im2col_k3s1p1_c3_kernel(const bf16* __restrict__ x, long long ld, bf16* __restrict__ col, int n, int h,
-                                        int w) {
+template <int C>
+__global__ void im2col_k3s1p1_kernel(const bf16* __restrict__ x, long long ld, bf16* __restrict__ col, int n, int h,
+                                     int w) {
   const long long total = static_cast<long long>(n) * h * w;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -64,9 +65,8 @@ __global__ void im2col_k3s1p1_c3_kernel(const bf16* __restrict__ x, long long ld
         if (yy >= 0 && yy < h && xx >= 0 && xx < w) {
           const uint2 v = __ldg(reinterpret_cast<const uint2*>(x + ((img * h + yy) * w + xx) * ld));
           const bf16* pv = reinterpret_cast<const bf16*>(&v);
-          row[(kh * 3 + kw) * 3 + 0] = pv[0];
-          row[(kh * 3 + kw) * 3 + 1] = pv[1];
-          row[(kh * 3 + kw) * 3 + 2] = pv[2];
+#pragma unroll
+          for (int c = 0; c < C; ++c) row[(kh * 3 + kw) * C + c] = pv[c];
         }
       }
     }
@@ -676,9 +676,23 @@ extern "C" {
 
 int gap_im2col_k3s1p1_c3(const void* x, int64_t ld, void* col, int n, int h, int w, void* stream) {
   GAP_CHECK_ARG(x && col && n > 0 && h > 0 && w > 0 && ld % 4 == 0, "gap_im2col_k3s1p1_c3: bad arguments");
+  return gap_im2col_k3s1p1_c(x, ld, 3, col, n, h, w, stream);
+}
+
+int gap_im2col_k3s1p1_c(const void* x, int64_t ld, int c, void* col, int n, int h, int w, void* stream) {
+  GAP_CHECK_ARG(c >= 1 && c <= 4, "gap_im2col_k3s1p1_c: c must be 1..4");
+  GAP_CHECK_ARG(x && col && n > 0 && h > 0 && w > 0 && ld % 4 == 0, "gap_im2col_k3s1p1_c: bad arguments");
   const long long total = static_cast<long long>(n) * h * w;
-  im2col_k3s1p1_c3_kernel<<<grid_of(total, 128, 148 * 16), 128, 0, static_cast<cudaStream_t>(stream)>>>(
-      static_cast<const bf16*>(x), ld, static_cast<bf16*>(col), n, h, w);
+  const int grid = grid_of(total, 128, 148 * 16);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const bf16* xi = static_cast<const bf16*>(x);
+  bf16* co = static_cast<bf16*>(col);
+  switch (c) {
+    case 1: im2col_k3s1p1_kernel<1><<<grid, 128, 0, st>>>(xi, ld, co, n, h, w); break;
+    case 2: im2col_k3s1p1_kernel<2><<<grid, 128, 0, st>>>(xi, ld, co, n, h, w); break;
+    case 3: im2col_k3s1p1_kernel<3><<<grid, 128, 0, st>>>(xi, ld, co, n, h, w); break;
+    default: im2col_k3s1p1_kernel<4><<<grid, 128, 0, st>>>(xi, ld, co, n, h, w); break;
+  }
   SI_LAUNCH_OK();
 }
 

@@ -1318,7 +1318,8 @@ struct ThinWgradParams {
   int n, h, w_in, oh, ow, cw;
   float* dw;
   long long ld_m;
-  int c_real;   // 3 (CT = 4) or 6 (CT = 8): channels per tap in the master layout
+  int c_real;   // c0 + c1: channels per tap in the master layout
+  int c0, c1;   // channels of source 0 / source 1 (slots 0..c0-1 and 4..4+c1-1 are real; the rest are dropped)
   float* dbias;
   int tiles_x, tiles_y;
   long long total_tiles;
@@ -1453,8 +1454,8 @@ __global__ void __launch_bounds__(256) thin_conv_wgrad_kernel(const __grid_const
           tap = kh * 4 + 2 * ni + (ncol >> 2);
           slot = ncol & 3;
         }
-        if ((slot & 3) == 3) continue;
-        const int ch = (slot & 3) + (slot >> 2) * 3;
+        if ((slot & 3) >= (slot < 4 ? p.c0 : p.c1)) continue;
+        const int ch = slot < 4 ? slot : p.c0 + slot - 4;
         atomicAdd(p.dw + static_cast<long long>(c0) * p.ld_m + tap * p.c_real + ch, acc[mi][ni][e]);
         atomicAdd(p.dw + static_cast<long long>(c0 + 8) * p.ld_m + tap * p.c_real + ch, acc[mi][ni][2 + e]);
       }
@@ -1701,12 +1702,12 @@ __global__ void __launch_bounds__(kWtThreads, 1) thin_conv_wgrad_tc_kernel(const
       if (CT == 8) {
         const int s8 = m & 7;
         tap = m >> 3;
-        valid = (s8 & 3) != 3;
-        ch = s8 < 3 ? s8 : s8 - 1;
+        valid = (s8 & 3) < (s8 < 4 ? p.c0 : p.c1);
+        ch = s8 < 4 ? s8 : p.c0 + s8 - 4;
       } else {
         const int s4 = m & 3;
         tap = m >> 2;
-        valid = m < 64 && s4 != 3;
+        valid = m < 64 && s4 < p.c0;
         ch = s4;
       }
       float* dst = p.dw + tap * p.c_real + ch;
@@ -1730,15 +1731,16 @@ __global__ void __launch_bounds__(kWtThreads, 1) thin_conv_wgrad_tc_kernel(const
 }
 
 // ------------------------------------------------------------------------------------------------
-// Thin-output ConvTranspose2d(cw -> 3, k4, s2, p1): the generator's last layer (+bias, Tanh; models.py:184,186)
-// and the input gradient of the discriminator's first conv.  Per CTA: a 10 x 18 halo tile of `wide` (8 x 16
-// source pixels + 1 ring) is multiplied by wcol[48 = tap*3 + co][cw] into col[halo pixel][48] (fp32, shared
-// memory) with warp MMAs, then every output pixel of the 16 x 32 output tile sums its 4 taps (col2im inside
-// the CTA; the ring makes the tile self-contained), adds the bias, applies Tanh and is written once.
+// Thin-output ConvTranspose2d(cw -> CO, k4, s2, p1), CO = 1..4: the generator's last layer (+bias, Tanh;
+// models.py:184,186) and the input gradient of the discriminator's first conv (once per source).  Per CTA: a 10 x 18
+// halo tile of `wide` (8 x 16 source pixels + 1 ring) is multiplied by wcol[16*CO = tap*CO + co][cw] into
+// col[halo pixel][16*CO] (fp32, shared memory) with warp MMAs, then every output pixel of the 16 x 32 output tile
+// sums its 4 taps (col2im inside the CTA; the ring makes the tile self-contained), adds the bias, applies Tanh and is
+// written once; output slots >= CO are written as zero.
 // The halo tile arrives by TMA (one 4-D box per 64 channels, out-of-range pixels zero-filled): the per-thread
 // cp.async loop it replaces was 40 % of the kernel's instructions (ncu source page), on an issue-bound kernel.
-// dynamic smem (1 KiB aligned): wide_s[cw/64][192 rows][128 B] (bf16, 128B-swizzled TMA tiles) | w_s[48][cw+8] (bf16) |
-//                               col_s[192][COLS] (fp32) | mbarrier
+// dynamic smem (1 KiB aligned): wide_s[cw/64][192 rows][128 B] (bf16, 128B-swizzled TMA tiles) | w_s[16*CO][cw+8] (bf16) |
+//                               col_s[192][thin_convT_col_stride(CO)] (fp32) | mbarrier
 // ------------------------------------------------------------------------------------------------
 struct ThinConvTParams {
   CUtensorMap tm_wide;   // [n][ih][iw][cw] bf16, box 64 ch x 18 x 10 x 1, 128B swizzle, OOB = zero (the halo ring)
@@ -1751,12 +1753,16 @@ struct ThinConvTParams {
   long long ld_bf;
   float* out_f32;
   long long ld_f;
-  uint8_t* out_u8;   // [n][2ih][2iw][3]: uint8((v*0.5 + 0.5) * 255), the image generate_synthetic_data.py:69-88 saves
+  uint8_t* out_u8;   // [n][2ih][2iw][CO]: uint8((v*0.5 + 0.5) * 255), the image generate_synthetic_data.py:69-88 saves
   int tiles_x, tiles_y;
   long long total_tiles;
 };
 
-constexpr int kColStride = 50;  // fp32 per col_s row (48 used); 50 = 18 mod 32 keeps the col2im reads of 16 neighbouring halo pixels in distinct banks
+// fp32 per col_s row (16*CO used).  In a warp the col2im reads 16 neighbouring halo pixels at one tap column (even
+// lanes) and the next 16 at the column CO lower (odd lanes).  CO = 3: 50 = 18 mod 32 puts the even lanes on the 16 even
+// banks and the odd lanes on the odd ones; CO = 1 likewise with 18.  CO = 2 / 4 read each tap as one float2 / float4:
+// a stride of 18 vectors keeps the 16 (8) lanes of one shared-memory wavefront on distinct 8 (16) byte slots.
+__host__ __device__ constexpr int thin_convT_col_stride(int co) { return co == 3 ? 50 : 18 * co; }
 
 constexpr int kWideBoxRows = 180;               // 10 x 18 halo pixels per box
 constexpr int kWideTileBytes = 192 * 128;       // one 64-channel tile: 192 MMA rows (180 loaded, 12 kept zero)
@@ -1768,20 +1774,24 @@ __device__ __forceinline__ float tanh_fast(float x) {
   return 1.f - __fdividef(2.f, e + 1.f);
 }
 
+template <int CO>
 __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_constant__ ThinConvTParams p) {
+  constexpr int NCOL = 16 * CO;                  // (tap, co) columns
+  constexpr int NT = CO;                         // 8-column n-tiles per warp (a warp owns half of the columns)
+  constexpr int kColStride = thin_convT_col_stride(CO);
   extern __shared__ uint8_t dsm_raw[];
   const uint32_t wide_a = (smem_u32(dsm_raw) + 1023u) & ~1023u;
   uint8_t* dsm = dsm_raw + (wide_a - smem_u32(dsm_raw));
   const int wstride = p.cw + 8;
   const int nbox = p.cw >> 6;
   bf16* w_s = reinterpret_cast<bf16*>(dsm + nbox * kWideTileBytes);
-  float* col_s = reinterpret_cast<float*>(w_s + 48 * wstride);
+  float* col_s = reinterpret_cast<float*>(w_s + NCOL * wstride);
   const uint32_t bar = smem_u32(col_s + 192 * kColStride);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int vshift = p.cw == 64 ? 3 : 4;
   const int oh = 2 * p.ih, ow = 2 * p.iw;
-  const int mg = warp >> 1, nh = warp & 1;   // warp = 3 m-tiles (48 halo pixels) x 3 n-tiles (24 columns)
+  const int mg = warp >> 1, nh = warp & 1;   // warp = 3 m-tiles (48 halo pixels) x NT n-tiles (8*NT columns)
 
   if (tid == 0) {
     tma_prefetch_desc(&p.tm_wide);
@@ -1793,16 +1803,13 @@ __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_consta
     const int b = idx / 96, r = (idx % 96) >> 3, seg = idx & 7;
     *reinterpret_cast<uint4*>(dsm + b * kWideTileBytes + (kWideBoxRows + r) * 128 + seg * 16) = make_uint4(0, 0, 0, 0);
   }
-  for (int idx = tid; idx < (48 << vshift); idx += 256) {
+  for (int idx = tid; idx < (NCOL << vshift); idx += 256) {
     const int r = idx >> vshift, seg = idx & ((1 << vshift) - 1);
     *reinterpret_cast<uint4*>(w_s + r * wstride + seg * 8) = ldg128(p.wcol + static_cast<long long>(r) * p.cw + seg * 8);
   }
-  float bias3[3] = {0.f, 0.f, 0.f};
-  if (p.bias != nullptr) {
-    bias3[0] = __ldg(p.bias);
-    bias3[1] = __ldg(p.bias + 1);
-    bias3[2] = __ldg(p.bias + 2);
-  }
+  float biasv[CO];
+#pragma unroll
+  for (int j = 0; j < CO; ++j) biasv[j] = p.bias != nullptr ? __ldg(p.bias + j) : 0.f;
   const uint32_t w_a = smem_u32(w_s);
   const int kchunks = p.cw >> 4;
   const int tiles_per_img = p.tiles_x * p.tiles_y;
@@ -1827,16 +1834,16 @@ __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_consta
     const int i0 = ty * 8, j0 = tx * 16;
     mbar_wait(bar, phase);
     phase ^= 1u;
-    // ---- col = wide_s (192 x cw) * wcol^T (cw x 48)
-    float acc[3][3][4];
+    // ---- col = wide_s (192 x cw) * wcol^T (cw x 16*CO)
+    float acc[3][NT][4];
 #pragma unroll
     for (int mi = 0; mi < 3; ++mi)
 #pragma unroll
-      for (int ni = 0; ni < 3; ++ni)
+      for (int ni = 0; ni < NT; ++ni)
 #pragma unroll
         for (int j = 0; j < 4; ++j) acc[mi][ni][j] = 0.f;
     for (int kc = 0; kc < kchunks; ++kc) {
-      uint32_t a[3][4], b[4], b4, b5;
+      uint32_t a[3][4], b[NT][2];
 #pragma unroll
       for (int mi = 0; mi < 3; ++mi) {
         // 128B-swizzled tile: 16-byte chunk c of row r lives at chunk (c ^ (r & 7))
@@ -1844,21 +1851,30 @@ __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_consta
         const int chunk = ((kc & 3) << 1) + (lane >> 4);
         ldmatrix_x4(a[mi], wide_a + (kc >> 2) * kWideTileBytes + row * 128 + ((chunk ^ (row & 7)) << 4));
       }
-      ldb_16x16(b, w_a + ((nh * 24) * wstride + kc * 16) * 2, wstride * 2, lane);
-      ldmatrix_x2(b4, b5, w_a + ((nh * 24 + 16 + (lane & 7)) * wstride + kc * 16 + ((lane >> 3) & 1) * 8) * 2);
+      // B fragments: pairs of n-tiles with one x4 load, an odd last n-tile with an x2 load
 #pragma unroll
-      for (int mi = 0; mi < 3; ++mi) {
-        mma_bf16_16816(acc[mi][0], a[mi], b[0], b[1]);
-        mma_bf16_16816(acc[mi][1], a[mi], b[2], b[3]);
-        mma_bf16_16816(acc[mi][2], a[mi], b4, b5);
+      for (int ni = 0; ni + 1 < NT; ni += 2) {
+        uint32_t r4[4];
+        ldb_16x16(r4, w_a + ((nh * NT + ni) * 8 * wstride + kc * 16) * 2, wstride * 2, lane);
+        b[ni][0] = r4[0];
+        b[ni][1] = r4[1];
+        b[ni + 1][0] = r4[2];
+        b[ni + 1][1] = r4[3];
       }
+      if (NT & 1)
+        ldmatrix_x2(b[NT - 1][0], b[NT - 1][1],
+                    w_a + (((nh * NT + NT - 1) * 8 + (lane & 7)) * wstride + kc * 16 + ((lane >> 3) & 1) * 8) * 2);
+#pragma unroll
+      for (int mi = 0; mi < 3; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < NT; ++ni) mma_bf16_16816(acc[mi][ni], a[mi], b[ni][0], b[ni][1]);
     }
 #pragma unroll
     for (int mi = 0; mi < 3; ++mi) {
       const int px0 = (mg * 3 + mi) * 16 + g;
 #pragma unroll
-      for (int ni = 0; ni < 3; ++ni) {
-        const int col = nh * 24 + ni * 8 + 2 * t;
+      for (int ni = 0; ni < NT; ++ni) {
+        const int col = (nh * NT + ni) * 8 + 2 * t;
         *reinterpret_cast<float2*>(col_s + px0 * kColStride + col) = make_float2(acc[mi][ni][0], acc[mi][ni][1]);
         *reinterpret_cast<float2*>(col_s + (px0 + 8) * kColStride + col) = make_float2(acc[mi][ni][2], acc[mi][ni][3]);
       }
@@ -1871,7 +1887,9 @@ __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_consta
       const int pix = tid + k * 256, yl = pix >> 5, xl = pix & 31;
       const int y = 2 * i0 + yl, x = 2 * j0 + xl;
       if (y >= oh || x >= ow) continue;
-      float v[3] = {bias3[0], bias3[1], bias3[2]};
+      float v[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+      for (int j = 0; j < CO; ++j) v[j] = biasv[j];
 #pragma unroll
       for (int a2 = 0; a2 < 2; ++a2) {
         const int kh = ((yl + 1) & 1) + 2 * a2;          // taps with (yl + 1 - kh) even
@@ -1880,25 +1898,35 @@ __global__ void __launch_bounds__(256) thin_convT_fwd_kernel(const __grid_consta
         for (int b2 = 0; b2 < 2; ++b2) {
           const int kw = ((xl + 1) & 1) + 2 * b2;
           const int c = ((xl + 1 - kw) >> 1) + 1;
-          const float* src = col_s + (r * 18 + c) * kColStride + (kh * 4 + kw) * 3;
-          v[0] += src[0];
-          v[1] += src[1];
-          v[2] += src[2];
+          const float* src = col_s + (r * 18 + c) * kColStride + (kh * 4 + kw) * CO;
+          if constexpr (CO == 4) {
+            const float4 q = *reinterpret_cast<const float4*>(src);
+            v[0] += q.x;
+            v[1] += q.y;
+            v[2] += q.z;
+            v[3] += q.w;
+          } else if constexpr (CO == 2) {
+            const float2 q = *reinterpret_cast<const float2*>(src);
+            v[0] += q.x;
+            v[1] += q.y;
+          } else {
+#pragma unroll
+            for (int j = 0; j < CO; ++j) v[j] += src[j];
+          }
         }
       }
       if (p.act == GAP_ACT_TANH) {
-        v[0] = tanh_fast(v[0]);
-        v[1] = tanh_fast(v[1]);
-        v[2] = tanh_fast(v[2]);
+#pragma unroll
+        for (int j = 0; j < CO; ++j) v[j] = tanh_fast(v[j]);
       }
       const long long o = (static_cast<long long>(img) * oh + y) * ow + x;
-      if (p.out_f32) *reinterpret_cast<float4*>(p.out_f32 + o * p.ld_f) = make_float4(v[0], v[1], v[2], 0.f);
-      if (p.out_bf) *reinterpret_cast<uint2*>(p.out_bf + o * p.ld_bf) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], 0.f));
+      if (p.out_f32) *reinterpret_cast<float4*>(p.out_f32 + o * p.ld_f) = make_float4(v[0], v[1], v[2], v[3]);
+      if (p.out_bf) *reinterpret_cast<uint2*>(p.out_bf + o * p.ld_bf) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
       if (p.out_u8) {
 #pragma unroll
-        for (int j = 0; j < 3; ++j) {
+        for (int j = 0; j < CO; ++j) {
           const float u = fminf(fmaxf((v[j] * 0.5f + 0.5f) * 255.f, 0.f), 255.f);
-          p.out_u8[o * 3 + j] = static_cast<uint8_t>(u);   // truncation, like torchvision's to_pil_image (mul(255).byte())
+          p.out_u8[o * CO + j] = static_cast<uint8_t>(u);   // truncation, like torchvision's to_pil_image (mul(255).byte())
         }
       }
     }
@@ -1941,12 +1969,16 @@ __global__ void bce_logits_const_f32_kernel(const float* __restrict__ x, long lo
   }
 }
 
-// uint8 HWC image -> normalised NHWC bf16 with 4 channel slots: (x/255 - 0.5)/0.5 (dataset.py:155-159 on the device)
+// uint8 HWC image [pixel][C] -> normalised NHWC bf16 with 4 channel slots: (x/255 - 0.5)/0.5 (dataset.py:155-159 on the
+// device); slots >= C are written as zero
+template <int C>
 __global__ void u8_hwc_to_nhwc_bf16_kernel(const uint8_t* __restrict__ x, bf16* __restrict__ out, long long ld,
                                            long long pixels) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < pixels; i += (long long)gridDim.x * blockDim.x) {
-    const float a = x[i * 3] * (2.f / 255.f) - 1.f, b = x[i * 3 + 1] * (2.f / 255.f) - 1.f, c = x[i * 3 + 2] * (2.f / 255.f) - 1.f;
-    *reinterpret_cast<uint2*>(out + i * ld) = make_uint2(pack_bf16x2(a, b), pack_bf16x2(c, 0.f));
+    float v[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int j = 0; j < C; ++j) v[j] = x[i * C + j] * (2.f / 255.f) - 1.f;
+    *reinterpret_cast<uint2*>(out + i * ld) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
   }
 }
 
@@ -1959,7 +1991,8 @@ __global__ void u8_hwc_to_nhwc_bf16_kernel(const uint8_t* __restrict__ x, bf16* 
 //   scale = in / out; support = max(scale, 1); center = scale * (i + 0.5)
 //   taps j in [max(0, int(center - support + 0.5)), min(in, int(center + support + 0.5)));
 //   w_j = max(0, 1 - |(j - center + 0.5) / max(scale, 1)|), normalised to sum 1.
-// One thread per output pixel, all three channels; the 2-D weights are the product of the two 1-D ones.
+// One thread per output pixel, all C channels (1..4; slots >= C of the bf16 output are written as zero); the 2-D weights
+// are the product of the two 1-D ones.
 // ------------------------------------------------------------------------------------------------
 struct AaAxis {
   int lo, n;
@@ -1976,6 +2009,7 @@ __device__ __forceinline__ AaAxis aa_axis(int i, int in, float scale) {
   for (int j = 0; j < a.n; ++j) a.total += fmaxf(0.f, 1.f - fabsf((j + a.lo - a.center + 0.5f) * a.inv));
   return a;
 }
+template <int C>
 __global__ void resize_u8_to_nhwc_bf16_kernel(const uint8_t* __restrict__ x, int n, int ih, int iw, int oh, int ow,
                                               bf16* __restrict__ out, long long ld, float* __restrict__ out_nchw) {
   const long long total = static_cast<long long>(n) * oh * ow;
@@ -1984,28 +2018,31 @@ __global__ void resize_u8_to_nhwc_bf16_kernel(const uint8_t* __restrict__ x, int
     const int ox = static_cast<int>(i % ow), oy = static_cast<int>((i / ow) % oh);
     const long long img = i / (static_cast<long long>(ow) * oh);
     const AaAxis ay = aa_axis(oy, ih, sh), ax = aa_axis(ox, iw, sw);
-    float acc[3] = {0.f, 0.f, 0.f};
+    float acc[C];
+#pragma unroll
+    for (int j = 0; j < C; ++j) acc[j] = 0.f;
     for (int jy = 0; jy < ay.n; ++jy) {
       const float wy = fmaxf(0.f, 1.f - fabsf((jy + ay.lo - ay.center + 0.5f) * ay.inv)) / ay.total;
-      const uint8_t* row = x + ((img * ih + ay.lo + jy) * iw + ax.lo) * 3;
-      float r[3] = {0.f, 0.f, 0.f};
+      const uint8_t* row = x + ((img * ih + ay.lo + jy) * iw + ax.lo) * C;
+      float r[C];
+#pragma unroll
+      for (int j = 0; j < C; ++j) r[j] = 0.f;
       for (int jx = 0; jx < ax.n; ++jx) {
         const float wx = fmaxf(0.f, 1.f - fabsf((jx + ax.lo - ax.center + 0.5f) * ax.inv)) / ax.total;
-        r[0] = fmaf(wx, row[jx * 3], r[0]);
-        r[1] = fmaf(wx, row[jx * 3 + 1], r[1]);
-        r[2] = fmaf(wx, row[jx * 3 + 2], r[2]);
+#pragma unroll
+        for (int j = 0; j < C; ++j) r[j] = fmaf(wx, row[jx * C + j], r[j]);
       }
-      acc[0] = fmaf(wy, r[0], acc[0]);
-      acc[1] = fmaf(wy, r[1], acc[1]);
-      acc[2] = fmaf(wy, r[2], acc[2]);
+#pragma unroll
+      for (int j = 0; j < C; ++j) acc[j] = fmaf(wy, r[j], acc[j]);
     }
-    const float a = acc[0] * (2.f / 255.f) - 1.f, b = acc[1] * (2.f / 255.f) - 1.f, c = acc[2] * (2.f / 255.f) - 1.f;
-    if (out != nullptr) *reinterpret_cast<uint2*>(out + i * ld) = make_uint2(pack_bf16x2(a, b), pack_bf16x2(c, 0.f));
-    if (out_nchw != nullptr) {      // what the reference's DataLoader yields: fp32 [n][3][oh][ow]
+    float v[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+    for (int j = 0; j < C; ++j) v[j] = acc[j] * (2.f / 255.f) - 1.f;
+    if (out != nullptr) *reinterpret_cast<uint2*>(out + i * ld) = make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
+    if (out_nchw != nullptr) {      // what the reference's DataLoader yields: fp32 [n][C][oh][ow]
       const long long hw = static_cast<long long>(oh) * ow, pix = static_cast<long long>(oy) * ow + ox;
-      out_nchw[(img * 3 + 0) * hw + pix] = a;
-      out_nchw[(img * 3 + 1) * hw + pix] = b;
-      out_nchw[(img * 3 + 2) * hw + pix] = c;
+#pragma unroll
+      for (int j = 0; j < C; ++j) out_nchw[(img * C + j) * hw + pix] = v[j];
     }
   }
 }
@@ -2324,10 +2361,10 @@ int gap_thin_conv_fwd(const void* src0, int64_t ld0, const void* src1, int64_t l
   return 0;
 }
 
-int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, const void* src1, int64_t ld1,
-                        int n, int h, int w, int cw, float* dw, int64_t ld_m, float* dbias, void* stream) {
+static int thin_conv_wgrad_launch(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, const void* src1,
+                                  int64_t ld1, int c0, int c1, int n, int h, int w, int cw, float* dw, int64_t ld_m,
+                                  float* dbias, void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  GAP_CHECK_ARG(wide && src0 && dw && n > 0 && h > 1 && w > 1, "gap_thin_conv_wgrad: bad arguments");
   if ((cw != 64 && cw != 128) || h % 2 || w % 2 || ld0 % 4 || (src1 && ld1 % 4) || ld_w % 8 ||
       (reinterpret_cast<uintptr_t>(src0) & 7) || (reinterpret_cast<uintptr_t>(src1) & 7) ||
       (reinterpret_cast<uintptr_t>(wide) & 15)) {
@@ -2349,7 +2386,9 @@ int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_
   p.cw = cw;
   p.dw = dw;
   p.ld_m = ld_m;
-  p.c_real = src1 ? 6 : 3;
+  p.c0 = c0;
+  p.c1 = c1;
+  p.c_real = c0 + c1;
   p.dbias = dbias;
   p.tiles_x = (p.ow + 15) / 16;
   p.tiles_y = (p.oh + 7) / 8;
@@ -2412,10 +2451,28 @@ int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_
   return 0;
 }
 
-int gap_thin_convT_fwd(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, const void* wcol, const float* bias,
-                       int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f, uint8_t* out_u8, void* stream) {
+int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, const void* src1, int64_t ld1,
+                        int n, int h, int w, int cw, float* dw, int64_t ld_m, float* dbias, void* stream) {
+  GAP_CHECK_ARG(wide && src0 && dw && n > 0 && h > 1 && w > 1, "gap_thin_conv_wgrad: bad arguments");
+  return thin_conv_wgrad_launch(wide, ld_w, src0, ld0, src1, ld1, 3, src1 ? 3 : 0, n, h, w, cw, dw, ld_m, dbias, stream);
+}
+
+int gap_thin_conv_wgrad_c(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, int c0, const void* src1,
+                          int64_t ld1, int c1, int n, int h, int w, int cw, float* dw, int64_t ld_m, float* dbias,
+                          void* stream) {
+  GAP_CHECK_ARG(c0 >= 1 && c0 <= 4 && (src1 ? (c1 >= 1 && c1 <= 4) : c1 == 0),
+                "gap_thin_conv_wgrad_c: c0 must be 1..4, c1 1..4 with a second source and 0 without");
+  GAP_CHECK_ARG(wide && src0 && dw && n > 0 && h > 1 && w > 1, "gap_thin_conv_wgrad_c: bad arguments");
+  return thin_conv_wgrad_launch(wide, ld_w, src0, ld0, src1, ld1, c0, c1, n, h, w, cw, dw, ld_m, dbias, stream);
+}
+
+}  // extern "C"
+
+template <int CO>
+static int thin_convT_launch(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, const void* wcol, const float* bias,
+                             int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f, uint8_t* out_u8,
+                             void* stream) {
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  GAP_CHECK_ARG(wide && wcol && (out_bf16 || out_f32 || out_u8) && n > 0 && ih > 0 && iw > 0, "gap_thin_convT_fwd: bad arguments");
   GAP_CHECK_ARG(act == GAP_ACT_NONE || act == GAP_ACT_TANH, "gap_thin_convT_fwd: activation must be none or Tanh");
   if ((cw != 64 && cw != 128) || ld_w % 8 || (out_bf16 && ld_bf % 4) || (out_f32 && ld_f % 4) ||
       (reinterpret_cast<uintptr_t>(wide) & 15) || (reinterpret_cast<uintptr_t>(wcol) & 15) ||
@@ -2451,37 +2508,82 @@ int gap_thin_convT_fwd(const void* wide, int64_t ld_w, int n, int ih, int iw, in
     int rc = encode_tmap_bf16(&p.tm_wide, wide, 4, dims, strides, box, nullptr, true);
     if (rc) return rc;
   }
-  const size_t smem = 1024 + static_cast<size_t>(cw / 64) * kWideTileBytes + 48 * static_cast<size_t>(cw + 8) * 2 +
-                      192 * kColStride * 4 + 16;
+  const size_t smem = 1024 + static_cast<size_t>(cw / 64) * kWideTileBytes + 16 * CO * static_cast<size_t>(cw + 8) * 2 +
+                      192 * thin_convT_col_stride(CO) * 4 + 16;
   static bool set = false;
   if (!set) {
-    GAP_CUDA(cudaFuncSetAttribute(thin_convT_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
+    GAP_CUDA(cudaFuncSetAttribute(thin_convT_fwd_kernel<CO>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
     set = true;
   }
   const int grid = static_cast<int>(std::min<long long>(p.total_tiles, static_cast<long long>(debug_get("thin_convT_ctas_per_sm", cw == 64 ? 3 : 2)) * sm_count()));
-  thin_convT_fwd_kernel<<<grid, 256, smem, st>>>(p);
+  thin_convT_fwd_kernel<CO><<<grid, 256, smem, st>>>(p);
   GAP_CUDA(cudaGetLastError());
   return 0;
 }
 
+extern "C" {
+
+int gap_thin_convT_fwd(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, const void* wcol, const float* bias,
+                       int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f, uint8_t* out_u8, void* stream) {
+  GAP_CHECK_ARG(wide && wcol && (out_bf16 || out_f32 || out_u8) && n > 0 && ih > 0 && iw > 0, "gap_thin_convT_fwd: bad arguments");
+  return thin_convT_launch<3>(wide, ld_w, n, ih, iw, cw, wcol, bias, act, out_bf16, ld_bf, out_f32, ld_f, out_u8, stream);
+}
+
+int gap_thin_convT_fwd_c(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, int co, const void* wcol,
+                         const float* bias, int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f,
+                         uint8_t* out_u8, void* stream) {
+  GAP_CHECK_ARG(co >= 1 && co <= 4, "gap_thin_convT_fwd_c: co must be 1..4");
+  GAP_CHECK_ARG(wide && wcol && (out_bf16 || out_f32 || out_u8) && n > 0 && ih > 0 && iw > 0, "gap_thin_convT_fwd_c: bad arguments");
+  switch (co) {
+    case 1: return thin_convT_launch<1>(wide, ld_w, n, ih, iw, cw, wcol, bias, act, out_bf16, ld_bf, out_f32, ld_f, out_u8, stream);
+    case 2: return thin_convT_launch<2>(wide, ld_w, n, ih, iw, cw, wcol, bias, act, out_bf16, ld_bf, out_f32, ld_f, out_u8, stream);
+    case 3: return thin_convT_launch<3>(wide, ld_w, n, ih, iw, cw, wcol, bias, act, out_bf16, ld_bf, out_f32, ld_f, out_u8, stream);
+    default: return thin_convT_launch<4>(wide, ld_w, n, ih, iw, cw, wcol, bias, act, out_bf16, ld_bf, out_f32, ld_f, out_u8, stream);
+  }
+}
+
 int gap_u8_hwc_to_nhwc_bf16(const uint8_t* x, void* out, int64_t out_ld, int64_t pixels, void* stream) {
+  return gap_u8_hwc_to_nhwc_bf16_c(x, 3, out, out_ld, pixels, stream);
+}
+
+int gap_u8_hwc_to_nhwc_bf16_c(const uint8_t* x, int c, void* out, int64_t out_ld, int64_t pixels, void* stream) {
+  GAP_CHECK_ARG(c >= 1 && c <= 4, "gap_u8_hwc_to_nhwc_bf16_c: c must be 1..4");
   GAP_CHECK_ARG(x && out && pixels > 0 && out_ld % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 7) == 0,
                 "gap_u8_hwc_to_nhwc_bf16: bad arguments");
   const int blocks = static_cast<int>(std::min<int64_t>((pixels + 255) / 256, 148 * 16));
-  u8_hwc_to_nhwc_bf16_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(x, static_cast<bf16*>(out), out_ld, pixels);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  bf16* o = static_cast<bf16*>(out);
+  switch (c) {
+    case 1: u8_hwc_to_nhwc_bf16_kernel<1><<<blocks, 256, 0, st>>>(x, o, out_ld, pixels); break;
+    case 2: u8_hwc_to_nhwc_bf16_kernel<2><<<blocks, 256, 0, st>>>(x, o, out_ld, pixels); break;
+    case 3: u8_hwc_to_nhwc_bf16_kernel<3><<<blocks, 256, 0, st>>>(x, o, out_ld, pixels); break;
+    default: u8_hwc_to_nhwc_bf16_kernel<4><<<blocks, 256, 0, st>>>(x, o, out_ld, pixels); break;
+  }
   GAP_CUDA(cudaGetLastError());
   return 0;
 }
 
 int gap_resize_u8_to_nhwc_bf16(const uint8_t* x, int n, int ih, int iw, int oh, int ow, void* out, int64_t out_ld,
                                float* out_nchw_f32, void* stream) {
+  return gap_resize_u8_to_nhwc_bf16_c(x, 3, n, ih, iw, oh, ow, out, out_ld, out_nchw_f32, stream);
+}
+
+int gap_resize_u8_to_nhwc_bf16_c(const uint8_t* x, int c, int n, int ih, int iw, int oh, int ow, void* out, int64_t out_ld,
+                                 float* out_nchw_f32, void* stream) {
+  GAP_CHECK_ARG(c >= 1 && c <= 4, "gap_resize_u8_to_nhwc_bf16_c: c must be 1..4");
   GAP_CHECK_ARG(x && (out || out_nchw_f32) && n > 0 && ih > 0 && iw > 0 && oh > 0 && ow > 0 &&
                     (!out || (out_ld >= 4 && out_ld % 4 == 0)),
                 "gap_resize_u8_to_nhwc_bf16: bad arguments");
   const long long total = static_cast<long long>(n) * oh * ow;
   const int blocks = static_cast<int>(std::min<long long>((total + 255) / 256, 148 * 16));
-  resize_u8_to_nhwc_bf16_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(stream)>>>(
-      x, n, ih, iw, oh, ow, static_cast<bf16*>(out), out_ld, out_nchw_f32);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  bf16* o = static_cast<bf16*>(out);
+  switch (c) {
+    case 1: resize_u8_to_nhwc_bf16_kernel<1><<<blocks, 256, 0, st>>>(x, n, ih, iw, oh, ow, o, out_ld, out_nchw_f32); break;
+    case 2: resize_u8_to_nhwc_bf16_kernel<2><<<blocks, 256, 0, st>>>(x, n, ih, iw, oh, ow, o, out_ld, out_nchw_f32); break;
+    case 3: resize_u8_to_nhwc_bf16_kernel<3><<<blocks, 256, 0, st>>>(x, n, ih, iw, oh, ow, o, out_ld, out_nchw_f32); break;
+    default: resize_u8_to_nhwc_bf16_kernel<4><<<blocks, 256, 0, st>>>(x, n, ih, iw, oh, ow, o, out_ld, out_nchw_f32); break;
+  }
   GAP_CUDA(cudaGetLastError());
   return 0;
 }

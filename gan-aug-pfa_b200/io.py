@@ -1,7 +1,7 @@
 """Host -> device input pipeline for the step loops (SURVEY.md §8(f) rank 2): replaces the reference's per-batch
 `.to(DEVICE)` (train_gan.py:53-54, train.py:137-139) by a double-buffered prefetch on a copy stream.
 
-Batches are tuples of PINNED host tensors — raw uint8 [n, h, w, 3] images (normalised on the device by the first
+Batches are tuples of PINNED host tensors — raw uint8 [n, h, w, C] images (normalised on the device by the first
 kernels, dataset.py:28-29,155-159) or the fp32 NCHW tensors the reference's DataLoader yields.  While iteration i
 computes, batch i+1 is copied into the other staging slot; the consumer calls `release()` once it has enqueued the
 work that reads the current slot, which lets the copy stream refill it two iterations later."""
@@ -17,13 +17,13 @@ from . import ops
 def load_pair_u8(a_u8: torch.Tensor, b_u8: torch.Tensor, size: Tuple[int, int],
                  label: Optional[torch.Tensor] = None):
     """The tensor half of BaseChangeDetectionDataset.__getitem__ (dataset.py:191, transform list at 185-191) on the
-    device, for raw uint8 [n, h, w, 3] image batches of any size: ToTensor -> JointResize(size, BILINEAR; labels
-    NEAREST) -> JointNormalize.  Returns fp32 NCHW [n, 3, H, W] tensors in [-1, 1] — what the reference's DataLoader
+    device, for raw uint8 [n, h, w, C] image batches (C = 1..4) of any size: ToTensor -> JointResize(size, BILINEAR;
+    labels NEAREST) -> JointNormalize.  Returns fp32 NCHW [n, C, H, W] tensors in [-1, 1] — what the reference's DataLoader
     yields and `train_step` / the drop-in modules accept — and the resized int64 label map if one was given."""
     H, W = size
     outs = []
     for x in (a_u8, b_u8):
-        f = torch.empty(x.shape[0], 3, H, W, device=x.device)
+        f = torch.empty(x.shape[0], x.shape[-1], H, W, device=x.device)
         ops.resize_u8_to_nhwc_bf16(x.contiguous(), None, f)
         outs.append(f)
     if label is not None:

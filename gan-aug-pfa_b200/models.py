@@ -21,7 +21,7 @@ import torch
 import torch.nn as nn
 
 from . import ops
-from .pix2pix import DiscriminatorEngine, GeneratorEngine
+from .pix2pix import DiscriminatorEngine, GeneratorEngine, check_image_channels, discriminator_split
 
 
 # ------------------------------------------------------------------------------------------------
@@ -282,6 +282,8 @@ class UNetGenerator(_NativeModule):
     def __init__(self, input_nc, output_nc, num_downs=7, ngf=64, norm_layer=nn.BatchNorm2d, use_dropout=False):
         super().__init__()
         self._norm = norm_kind(norm_layer, use_dropout)
+        check_image_channels("input_nc", input_nc)
+        check_image_channels("output_nc", output_nc)
         self._cfg = (input_nc, output_nc, num_downs, ngf)
         self._use_dropout = bool(use_dropout)
         blk = UnetSkipConnectionBlock(ngf * 8, ngf * 8, input_nc=None, submodule=None, norm_layer=norm_layer,
@@ -304,15 +306,20 @@ class UNetGenerator(_NativeModule):
 
 
 class _DiscriminatorFn(torch.autograd.Function):
+    """The input cat(A, B) is split by discriminator_split: A = the first ceil(input_nc / 2) channels, B = the rest."""
+
     @staticmethod
     def forward(ctx, module, x, grad_mode, *params):
         eng = module._engine()
         n, c, h, w = x.shape
+        if c != sum(eng.split):
+            raise ValueError(f"discriminator input has {c} channels, expected input_nc = {sum(eng.split)}")
+        ca = eng.split[0]
         xd = x.detach().contiguous().float()
         xa = torch.zeros(n, h, w, 4, device=x.device, dtype=torch.bfloat16)
         xb = torch.zeros_like(xa)
-        ops.nchw_to_nhwc_bf16(xd[:, :3].contiguous(), xa)
-        ops.nchw_to_nhwc_bf16(xd[:, 3:].contiguous(), xb)
+        ops.nchw_to_nhwc_bf16(xd[:, :ca].contiguous(), xa)
+        ops.nchw_to_nhwc_bf16(xd[:, ca:].contiguous(), xb)
         logits = eng.forward(xa, xb)
         out = logits.permute(0, 3, 1, 2).clone()
         ctx.module = module
@@ -337,20 +344,23 @@ class _DiscriminatorFn(torch.autograd.Function):
         eng._join_wgrad()
         gx = None
         if ctx.x_grad:
-            gx = torch.empty(n, 6, h, w, device=gout.device)
-            ops.nhwc_to_nchw_f32(eng.dreal, gx, 3, 6, 0)
-            ops.nhwc_to_nchw_f32(eng.dfake, gx, 3, 6, 3)
+            ca, cb = eng.split
+            gx = torch.empty(n, ca + cb, h, w, device=gout.device)
+            ops.nhwc_to_nchw_f32(eng.dreal, gx, ca, ca + cb, 0)
+            ops.nhwc_to_nchw_f32(eng.dfake, gx, cb, ca + cb, ca)
         names = [name for name, _ in module.named_parameters()]
         grads = module._grads_for_autograd(eng, names) if wgrad else [None] * len(names)
         return (None, gx, None, *grads)
 
 
 class NLayerDiscriminator(_NativeModule):
-    """PatchGAN discriminator (models.py:212-247) executing on the native sm_100a kernels."""
+    """PatchGAN discriminator (models.py:212-247) executing on the native sm_100a kernels.  input_nc = 2..8: the input
+    is read as cat(A, B) with A = its first ceil(input_nc / 2) channels (pix2pix.discriminator_split)."""
 
     def __init__(self, input_nc, ndf=64, n_layers=3, norm_layer=nn.BatchNorm2d):
         super().__init__()
         self._norm = norm_kind(norm_layer)
+        discriminator_split(input_nc)
         self._cfg = (input_nc, ndf, n_layers)
         use_bias = False
         kw, padw = 4, 1

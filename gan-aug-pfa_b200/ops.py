@@ -252,14 +252,19 @@ def tanh_bwd(gout_nchw: torch.Tensor, y_nhwc_f32: torch.Tensor, dpre: torch.Tens
 def gen_out_bwd(fake_f32: torch.Tensor, real: torch.Tensor, dfake_d: Optional[torch.Tensor], l1_scale: float,
                 dpre: torch.Tensor, loss_acc: torch.Tensor) -> None:
     """L1 * lambda + Tanh backward.  ``real`` is real_B either as fp32 NCHW (what the reference's DataLoader yields) or
-    as the raw uint8 [n, h, w, 3] image (normalised in the kernel like dataset.py does)."""
-    n, h, w, _ = fake_f32.shape
+    as the raw uint8 [n, h, w, C] image (normalised in the kernel like dataset.py does); C = 1..4 channels, which
+    ``fake_f32`` / ``dfake_d`` / ``dpre`` hold in the first C of their channel slots."""
+    n, h, w, slots = fake_f32.shape
     if real.dtype == torch.uint8:
-        if tuple(real.shape) != (n, h, w, 3) or not real.is_contiguous():
-            raise ValueError("uint8 real_B must be contiguous [n, h, w, 3]")
-        fn, name, c = _lib.lib().gap_gen_out_bwd_u8, "gap_gen_out_bwd_u8", 3
+        c = real.shape[-1]
+        if real.dim() != 4 or tuple(real.shape[:3]) != (n, h, w) or not real.is_contiguous():
+            raise ValueError("uint8 real_B must be contiguous [n, h, w, C]")
+        fn, name = _lib.lib().gap_gen_out_bwd_u8, "gap_gen_out_bwd_u8"
     else:
-        fn, name, c = _lib.lib().gap_gen_out_bwd, "gap_gen_out_bwd", real.shape[1]
+        c = real.shape[1]
+        fn, name = _lib.lib().gap_gen_out_bwd, "gap_gen_out_bwd"
+    if not 1 <= c <= slots:
+        raise ValueError(f"real_B has {c} channels; the generator output holds {slots} channel slots")
     _lib.check(fn(_ptr(fake_f32), fake_f32.stride(2), _ptr(real), h * w, _ptr(dfake_d),
                   0 if dfake_d is None else dfake_d.stride(2), l1_scale, _ptr(dpre), dpre.stride(2), n * h * w, c,
                   _ptr(loss_acc), _stream()), name)
@@ -359,8 +364,9 @@ def cout1_conv_wgrad(dlogits: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, k
 def thin_conv_fwd(s0: torch.Tensor, s1: Optional[torch.Tensor], wpk: torch.Tensor, bias: Optional[torch.Tensor],
                   out1: torch.Tensor, act1: int = ACT_NONE, out2: Optional[torch.Tensor] = None,
                   act2: int = ACT_NONE) -> None:
-    """Conv2d(k4,s2,p1) over one or two 4-slot NHWC sources (3 channels + a zero slot each) -> cw = 64/128
-    channels, fused bias + activation(s); wpk bf16 [cw, 16*CT] with CT = 4 (one source) or 8 (two)."""
+    """Conv2d(k4,s2,p1) over one or two 4-slot NHWC sources (1..4 channels each, unused slots zero) -> cw = 64/128
+    channels, fused bias + activation(s); wpk bf16 [cw, 16*CT] with CT = 4 (one source) or 8 (two), zero in the
+    columns of unused slots."""
     n, h, w, _, ld0 = _nhwc_view(s0)
     ld1 = 0
     if s1 is not None:
@@ -386,9 +392,10 @@ def thin_conv_fwd(s0: torch.Tensor, s1: Optional[torch.Tensor], wpk: torch.Tenso
 
 
 def thin_conv_wgrad(wide: torch.Tensor, s0: torch.Tensor, s1: Optional[torch.Tensor], dw: torch.Tensor, ld_m: int,
-                    dbias: Optional[torch.Tensor] = None) -> None:
+                    dbias: Optional[torch.Tensor] = None, c0: int = 3, c1: Optional[int] = None) -> None:
     """dw[cw][(kh*4+kw)*c + ch] += sum_pix wide[pix][cw] * thin[2*pix+tap-1][ch] (fp32 master layout, row stride
-    ld_m); dbias[cw] += sum_pix wide[pix][cw]."""
+    ld_m); dbias[cw] += sum_pix wide[pix][cw].  c0 / c1: channels of the two sources (c1 defaults to 3 with a second
+    source, 0 without); c = c0 + c1, and source 1's channel s is master channel c0 + s."""
     n, oh, ow, cw, ldw = _nhwc_view(wide)
     n0, h, w, _, ld0 = _nhwc_view(s0)
     if (n0, h, w) != (n, 2 * oh, 2 * ow):
@@ -398,28 +405,42 @@ def thin_conv_wgrad(wide: torch.Tensor, s0: torch.Tensor, s1: Optional[torch.Ten
         n1, h1, w1, _, ld1 = _nhwc_view(s1)
         if (n1, h1, w1) != (n, h, w):
             raise ValueError("sources must share n/h/w")
-    c = 6 if s1 is not None else 3
+    if c1 is None:
+        c1 = 3 if s1 is not None else 0
+    if not 1 <= c0 <= 4 or (s1 is not None and not 1 <= c1 <= 4) or (s1 is None and c1 != 0):
+        raise ValueError(f"channels per source must be 1..4 (c1 = 0 without a second source), got c0={c0} c1={c1}")
+    c = c0 + c1
     if dw.dtype != torch.float32 or dw.numel() < (cw - 1) * ld_m + 16 * c:
         raise ValueError("dw too small")
-    _lib.check(_lib.lib().gap_thin_conv_wgrad(_ptr(wide), ldw, _ptr(s0), ld0, _ptr(s1), ld1, n, h, w, cw, _ptr(dw), ld_m,
-                                              _ptr(dbias), _stream()), "gap_thin_conv_wgrad")
+    if (c0, c1) == (3, 3 if s1 is not None else 0):
+        _lib.check(_lib.lib().gap_thin_conv_wgrad(_ptr(wide), ldw, _ptr(s0), ld0, _ptr(s1), ld1, n, h, w, cw, _ptr(dw),
+                                                  ld_m, _ptr(dbias), _stream()), "gap_thin_conv_wgrad")
+        return
+    _lib.check(_lib.lib().gap_thin_conv_wgrad_c(_ptr(wide), ldw, _ptr(s0), ld0, c0, _ptr(s1), ld1, c1, n, h, w, cw,
+                                                _ptr(dw), ld_m, _ptr(dbias), _stream()), "gap_thin_conv_wgrad_c")
 
 
 def u8_hwc_to_nhwc_bf16(x: torch.Tensor, out: torch.Tensor) -> None:
-    """uint8 [n,h,w,3] -> normalised NHWC bf16 with 4 channel slots (dataset.py:155-159 on the device)."""
-    if x.dtype != torch.uint8 or x.shape[-1] != 3 or not x.is_contiguous() or not x.is_cuda:
-        raise ValueError("expected a contiguous CUDA uint8 [n,h,w,3] tensor")
-    _lib.check(_lib.lib().gap_u8_hwc_to_nhwc_bf16(_ptr(x), _ptr(out), out.stride(2), x.numel() // 3, _stream()),
-               "gap_u8_hwc_to_nhwc_bf16")
+    """uint8 [n,h,w,C] (C = 1..4) -> normalised NHWC bf16 with 4 channel slots, slots >= C zero (dataset.py:155-159 on
+    the device)."""
+    c = x.shape[-1]
+    if x.dtype != torch.uint8 or not 1 <= c <= 4 or not x.is_contiguous() or not x.is_cuda:
+        raise ValueError(f"expected a contiguous CUDA uint8 [n,h,w,C] tensor with C = 1..4, got {x.dtype} {tuple(x.shape)}")
+    if c == 3:
+        _lib.check(_lib.lib().gap_u8_hwc_to_nhwc_bf16(_ptr(x), _ptr(out), out.stride(2), x.numel() // 3, _stream()),
+                   "gap_u8_hwc_to_nhwc_bf16")
+        return
+    _lib.check(_lib.lib().gap_u8_hwc_to_nhwc_bf16_c(_ptr(x), c, _ptr(out), out.stride(2), x.numel() // c, _stream()),
+               "gap_u8_hwc_to_nhwc_bf16_c")
 
 
 def resize_u8_to_nhwc_bf16(x: torch.Tensor, out: Optional[torch.Tensor], out_nchw_f32: Optional[torch.Tensor] = None) -> None:
-    """dataset.py's ToTensor + JointResize(BILINEAR, antialias) + JointNormalize on the device: uint8 [n,ih,iw,3] ->
-    NHWC bf16 [n,oh,ow,4 slots] and / or the fp32 NCHW [n,3,oh,ow] tensor the reference's DataLoader yields (the output
-    tensors' h / w are the target size)."""
-    if x.dtype != torch.uint8 or x.dim() != 4 or x.shape[-1] != 3 or not x.is_contiguous() or not x.is_cuda:
-        raise ValueError("expected a contiguous CUDA uint8 [n,h,w,3] tensor")
-    n = x.shape[0]
+    """dataset.py's ToTensor + JointResize(BILINEAR, antialias) + JointNormalize on the device: uint8 [n,ih,iw,C]
+    (C = 1..4) -> NHWC bf16 [n,oh,ow,4 slots] (slots >= C zero) and / or the fp32 NCHW [n,C,oh,ow] tensor the reference's
+    DataLoader yields (the output tensors' h / w are the target size)."""
+    if x.dtype != torch.uint8 or x.dim() != 4 or not 1 <= x.shape[-1] <= 4 or not x.is_contiguous() or not x.is_cuda:
+        raise ValueError("expected a contiguous CUDA uint8 [n,h,w,C] tensor with C = 1..4")
+    n, c = x.shape[0], x.shape[-1]
     ld = 0
     if out is not None:
         on, oh, ow, _, ld = _nhwc_view(out)
@@ -427,15 +448,19 @@ def resize_u8_to_nhwc_bf16(x: torch.Tensor, out: Optional[torch.Tensor], out_nch
             raise ValueError("output must be NHWC bf16 [n, oh, ow, >=4]")
     if out_nchw_f32 is not None:
         f = out_nchw_f32
-        if f.dtype != torch.float32 or f.dim() != 4 or f.shape[0] != n or f.shape[1] != 3 or not f.is_contiguous() or not f.is_cuda:
-            raise ValueError("out_nchw_f32 must be a contiguous CUDA fp32 [n,3,oh,ow] tensor")
+        if f.dtype != torch.float32 or f.dim() != 4 or f.shape[0] != n or f.shape[1] != c or not f.is_contiguous() or not f.is_cuda:
+            raise ValueError(f"out_nchw_f32 must be a contiguous CUDA fp32 [n,{c},oh,ow] tensor")
         if out is not None and (f.shape[2], f.shape[3]) != (oh, ow):
             raise ValueError("both outputs must have the same size")
         oh, ow = f.shape[2], f.shape[3]
     if out is None and out_nchw_f32 is None:
         raise ValueError("no output given")
-    _lib.check(_lib.lib().gap_resize_u8_to_nhwc_bf16(_ptr(x), n, x.shape[1], x.shape[2], oh, ow, _ptr(out), ld,
-                                                     _ptr(out_nchw_f32), _stream()), "gap_resize_u8_to_nhwc_bf16")
+    if c == 3:
+        _lib.check(_lib.lib().gap_resize_u8_to_nhwc_bf16(_ptr(x), n, x.shape[1], x.shape[2], oh, ow, _ptr(out), ld,
+                                                         _ptr(out_nchw_f32), _stream()), "gap_resize_u8_to_nhwc_bf16")
+        return
+    _lib.check(_lib.lib().gap_resize_u8_to_nhwc_bf16_c(_ptr(x), c, n, x.shape[1], x.shape[2], oh, ow, _ptr(out), ld,
+                                                       _ptr(out_nchw_f32), _stream()), "gap_resize_u8_to_nhwc_bf16_c")
 
 
 def resize_nearest_i64(x: torch.Tensor, out: torch.Tensor) -> None:
@@ -449,18 +474,27 @@ def resize_nearest_i64(x: torch.Tensor, out: torch.Tensor) -> None:
 
 def thin_convT_fwd(wide: torch.Tensor, wcol: torch.Tensor, bias: Optional[torch.Tensor], act: int,
                    out_bf16: Optional[torch.Tensor], out_f32: Optional[torch.Tensor],
-                   out_u8: Optional[torch.Tensor] = None) -> None:
-    """ConvTranspose2d(cw -> 3, k4, s2, p1) (+bias, Tanh) into 4-slot NHWC outputs; wcol bf16 [48 = tap*3+co, cw]."""
+                   out_u8: Optional[torch.Tensor] = None, co: int = 3) -> None:
+    """ConvTranspose2d(cw -> co, k4, s2, p1) (+bias, Tanh), co = 1..4, into 4-slot NHWC outputs (slots >= co written
+    as zero); wcol bf16 [16*co = tap*co + c, cw]; out_u8 uint8 [n, 2ih, 2iw, co]."""
+    if not 1 <= co <= 4:
+        raise ValueError(f"co must be 1..4, got {co}")
     n, ih, iw, cw, ldw = _nhwc_view(wide)
-    if wcol.dtype != torch.bfloat16 or tuple(wcol.shape) != (48, cw) or not wcol.is_contiguous():
-        raise ValueError(f"wcol must be contiguous bf16 [48, {cw}]")
+    if wcol.dtype != torch.bfloat16 or tuple(wcol.shape) != (16 * co, cw) or not wcol.is_contiguous():
+        raise ValueError(f"wcol must be contiguous bf16 [{16 * co}, {cw}]")
     for o, dt in ((out_bf16, torch.bfloat16), (out_f32, torch.float32)):
         if o is not None and (o.dtype != dt or tuple(o.shape[:3]) != (n, 2 * ih, 2 * iw) or o.shape[3] < 4):
             raise ValueError("output must be [n, 2ih, 2iw, >=4]")
-    _lib.check(_lib.lib().gap_thin_convT_fwd(_ptr(wide), ldw, n, ih, iw, cw, _ptr(wcol), _ptr(bias), act, _ptr(out_bf16),
-                                             0 if out_bf16 is None else out_bf16.stride(2), _ptr(out_f32),
-                                             0 if out_f32 is None else out_f32.stride(2), _ptr(out_u8), _stream()),
-               "gap_thin_convT_fwd")
+    if out_u8 is not None and (out_u8.dtype != torch.uint8 or tuple(out_u8.shape) != (n, 2 * ih, 2 * iw, co)
+                               or not out_u8.is_contiguous()):
+        raise ValueError(f"out_u8 must be a contiguous uint8 [{n}, {2 * ih}, {2 * iw}, {co}] tensor")
+    args = (n, ih, iw, cw) + (() if co == 3 else (co,)) + (
+        _ptr(wcol), _ptr(bias), act, _ptr(out_bf16), 0 if out_bf16 is None else out_bf16.stride(2), _ptr(out_f32),
+        0 if out_f32 is None else out_f32.stride(2), _ptr(out_u8), _stream())
+    if co == 3:
+        _lib.check(_lib.lib().gap_thin_convT_fwd(_ptr(wide), ldw, *args), "gap_thin_convT_fwd")
+    else:
+        _lib.check(_lib.lib().gap_thin_convT_fwd_c(_ptr(wide), ldw, *args), "gap_thin_convT_fwd_c")
 
 
 def bn_finalize(stats, count, gamma, beta, eps, momentum, repeat, running_mean, running_var, nbt, scale, shift,
@@ -660,6 +694,17 @@ def _px(t: torch.Tensor) -> int:
 def im2col_k3s1p1_c3(x: torch.Tensor, col: torch.Tensor) -> None:
     n, h, w, _, ld = _nhwc_view(x)
     _lib.check(_lib.lib().gap_im2col_k3s1p1_c3(_ptr(x), ld, _ptr(col), n, h, w, _stream()), "gap_im2col_k3s1p1_c3")
+
+
+def im2col_k3s1p1(x: torch.Tensor, col: torch.Tensor, c: int) -> None:
+    """col[pix][(kh*3+kw)*c + ch] (9*c values, zero padded to 64) of the first c = 1..4 channel slots of x."""
+    if not 1 <= c <= 4:
+        raise ValueError(f"c must be 1..4, got {c}")
+    if c == 3:
+        im2col_k3s1p1_c3(x, col)
+        return
+    n, h, w, _, ld = _nhwc_view(x)
+    _lib.check(_lib.lib().gap_im2col_k3s1p1_c(_ptr(x), ld, c, _ptr(col), n, h, w, _stream()), "gap_im2col_k3s1p1_c")
 
 
 def maxpool2x2_fwd(x: torch.Tensor, out: torch.Tensor) -> None:

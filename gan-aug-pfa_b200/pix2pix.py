@@ -34,6 +34,26 @@ BN_EPS = 1e-5
 BN_MOMENTUM = 0.1
 IN_EPS = 1e-5           # nn.InstanceNorm2d default
 LAMBDA_L1 = 100.0  # train_gan.py:33
+# Image tensors on the hot path are NHWC bf16 with IMAGE_SLOTS channel slots: an image of 1..4 channels fills the first
+# ones and the rest stay zero.  The discriminator sees cat(A, B) as two such sources.
+IMAGE_SLOTS = 4
+
+
+def check_image_channels(what: str, c: int) -> int:
+    """`c` if it fits one 4-slot image tensor, else NotImplementedError naming the supported range."""
+    if not isinstance(c, int) or not 1 <= c <= IMAGE_SLOTS:
+        raise NotImplementedError(f"{what} = {c!r} is not implemented natively: images of 1 to {IMAGE_SLOTS} channels are")
+    return c
+
+
+def discriminator_split(input_nc: int) -> Tuple[int, int]:
+    """Channels of the two sources of a discriminator over cat(A, B) with `input_nc` channels: A = the first
+    ceil(input_nc / 2), B = the rest (3 | 3 for the reference's 6).  NotImplementedError outside 2..8."""
+    if not isinstance(input_nc, int) or not 2 <= input_nc <= 2 * IMAGE_SLOTS:
+        raise NotImplementedError(f"input_nc = {input_nc!r} is not implemented natively by the discriminator: 2 to "
+                                  f"{2 * IMAGE_SLOTS} channels are (two sources of up to {IMAGE_SLOTS} channels each)")
+    ca = (input_nc + 1) // 2
+    return ca, input_nc - ca
 
 
 def _pad4(n: int) -> int:
@@ -385,7 +405,8 @@ class _Net:
 # Generator
 # ================================================================================================
 class GeneratorEngine(_Net):
-    """UNetGenerator(input_nc=3, output_nc=3, num_downs, ngf, BatchNorm2d or InstanceNorm2d, use_dropout)."""
+    """UNetGenerator(input_nc, output_nc, num_downs, ngf, BatchNorm2d or InstanceNorm2d, use_dropout) with
+    input_nc, output_nc in 1..4 (default 3, 3)."""
 
     _BUFFER_ATTRS = ("S", "x_nhwc", "A", "R", "Rin", "yd", "yu", "fake_bf", "fake_f32", "dpre", "gR", "gRin", "gA",
                      "dyu", "dyd", "xin", "out_cat")
@@ -408,25 +429,31 @@ class GeneratorEngine(_Net):
         self.dropout_calls = 0          # forward counter: every forward draws fresh masks
         self._drop_off: Dict[int, int] = {}
         if spec is None:
-            if input_nc != 3 or output_nc != 3:
-                raise NotImplementedError("the native generator supports input_nc = output_nc = 3")
+            check_image_channels("input_nc", input_nc)
+            check_image_channels("output_nc", output_nc)
             if ngf % 64 != 0 or num_downs < 5:
                 raise NotImplementedError("ngf must be a multiple of 64 and num_downs >= 5")
             spec = GeneratorSpec(input_nc, output_nc, num_downs, ngf, norm=norm)
         else:
             if use_dropout:
                 raise NotImplementedError("stand-alone blocks with dropout are not implemented natively")
-            if any(c % 64 for c in spec.C) or (not spec.virtual0 and (spec.input_nc != 3 or spec.output_nc != 3)):
-                raise NotImplementedError("native blocks need channel counts that are multiples of 64 (3 at the image side)")
+            if any(c % 64 for c in spec.C):
+                raise NotImplementedError("native blocks need channel counts that are multiples of 64 (1 to 4 at the "
+                                          "image side)")
+            if not spec.virtual0:
+                check_image_channels("input_nc", spec.input_nc)
+                check_image_channels("output_nc", spec.output_nc)
         self.spec = sp = spec
+        self.input_nc, self.output_nc = sp.input_nc, sp.output_nc
         self.virtual0 = v0 = sp.virtual0
         self.L = L = sp.L
         self.C = C = sp.C
         self.k_down, self.k_dbn, self.k_up, self.k_ubn = sp.k_down, sp.k_dbn, sp.k_up, sp.k_ubn
         # flat-buffer order = order in which gradients complete in backward (DP buckets)
+        ic, oc = self.input_nc, self.output_nc
         if not v0:
-            self._reg_small(self.k_up[0] + ".weight", 2 * C[0], 3, 64)
-            self._reg_vec(self.k_up[0] + ".bias", 3)
+            self._reg_small(self.k_up[0] + ".weight", 2 * C[0], oc, 64)
+            self._reg_vec(self.k_up[0] + ".bias", oc)
         # ubn / dbn: the norm layers (_BN or _IN); with InstanceNorm each conv's bias segment follows its weight
         norm_reg = self._reg_in if inst else self._reg_bn
         self.ubn: List[Optional[_BN]] = [None] * L
@@ -444,7 +471,7 @@ class GeneratorEngine(_Net):
             if self.k_dbn[j] is not None:
                 self.dbn[j] = norm_reg(self.k_dbn[j], C[j])
         if not v0:
-            self._reg_small(self.k_down[0] + ".weight", C[0], 3, 64)
+            self._reg_small(self.k_down[0] + ".weight", C[0], ic, 64)
             if inst:
                 self._reg_vec(self.k_down[0] + ".bias", C[0])
         self.store.allocate(device)
@@ -459,8 +486,8 @@ class GeneratorEngine(_Net):
         self.w_u_fwd = [None]
         self.w_u_dg = [None]
         if not v0:
-            self.w_u_T2 = torch.zeros(48, 2 * C[0], **bf)        # last ConvTranspose2d, forward: [(kh*4+kw)*3 + co][Cin]
-            # thin-layer operands [rows][16 taps x 4 channel slots] (3 channels + a zero slot)
+            self.w_u_T2 = torch.zeros(16 * oc, 2 * C[0], **bf)   # last ConvTranspose2d, forward: [(kh*4+kw)*oc + co][Cin]
+            # thin-layer operands [rows][16 taps x 4 channel slots] (input_nc / output_nc channels, zero slots after)
             self.w_d_thin = torch.zeros(C[0], 64, **bf)          # first conv, models.py:177
             self.w_u_thin = torch.zeros(2 * C[0], 64, **bf)      # last ConvTranspose2d seen from its dgrad
         else:
@@ -496,10 +523,11 @@ class GeneratorEngine(_Net):
             plan.add(p, o, self.w_d_dg[j], 2, 4, ci, ci, (2, 2), co, co, 4 * co, (1, 16 * ci, 4 * ci, ci))
         if not self.virtual0:
             k0 = off(self.k_up[0] + ".weight")
-            c2 = 2 * C[0]
-            plan.add(p, k0, self.w_u_T2, 0, 1, 48, 48, (1, 1), c2, c2, c2, (1, 64, 0, 0))
-            plan.add(p, off(self.k_down[0] + ".weight"), self.w_d_thin, 0, 1, C[0], C[0], (4, 4), 3, 4, 64, (64, 1, 12, 3))
-            plan.add(p, k0, self.w_u_thin, 0, 1, c2, c2, (4, 4), 3, 4, 64, (64, 1, 12, 3))
+            c2, ic, oc = 2 * C[0], self.input_nc, self.output_nc
+            plan.add(p, k0, self.w_u_T2, 0, 1, 16 * oc, 16 * oc, (1, 1), c2, c2, c2, (1, 64, 0, 0))
+            plan.add(p, off(self.k_down[0] + ".weight"), self.w_d_thin, 0, 1, C[0], C[0], (4, 4), ic, 4, 64,
+                     (64, 1, 4 * ic, ic))
+            plan.add(p, k0, self.w_u_thin, 0, 1, c2, c2, (4, 4), oc, 4, 64, (64, 1, 4 * oc, oc))
         for j in range(1, L):
             ci = C[j] if j == L - 1 else 2 * C[j]
             co = C[j - 1]
@@ -554,9 +582,11 @@ class GeneratorEngine(_Net):
         """Size the buffers for x and convert it into self.x_nhwc (NHWC bf16, 4 channel slots); returns that tensor."""
         u8_in = x_nchw.dtype == torch.uint8
         if u8_in:
-            n, h, w, _ = x_nchw.shape
+            n, h, w, c = x_nchw.shape
         else:
-            n, _, h, w = x_nchw.shape
+            n, c, h, w = x_nchw.shape
+        if c != self.input_nc:
+            raise ValueError(f"generator input has {c} channels, expected input_nc = {self.input_nc}")
         self._alloc(n, h, w)
         if u8_in:
             ops.u8_hwc_to_nhwc_bf16(x_nchw, self.x_nhwc)
@@ -567,11 +597,12 @@ class GeneratorEngine(_Net):
     @_on_device
     def forward(self, x_nchw: torch.Tensor, bn_repeat: int = 1, out_u8: Optional[torch.Tensor] = None,
                 x_ready: bool = False) -> torch.Tensor:
-        """x: fp32 NCHW on the device, or uint8 NHWC [n,h,w,3] (normalised on the device like dataset.py:155-159).
-        Returns fake as fp32 NHWC [n,h,w,4] (channel 3 is padding); the bf16 copy is self.fake_bf.  bn_repeat=2
-        folds the reference's second identical forward.  out_u8 (uint8 [n,h,w,3]) additionally receives the image
-        generate_synthetic_data.py:69-88 saves, written by the last layer's epilogue.  x_ready: prepare_input(x) has
-        already run (the trainer converts the input before it forks the generator onto its own stream)."""
+        """x: fp32 NCHW on the device, or uint8 NHWC [n,h,w,input_nc] (normalised on the device like dataset.py:155-159).
+        Returns fake as fp32 NHWC [n,h,w,4] (channels >= output_nc are zero padding); the bf16 copy is self.fake_bf.
+        bn_repeat=2 folds the reference's second identical forward.  out_u8 (uint8 [n,h,w,output_nc]) additionally
+        receives the image generate_synthetic_data.py:69-88 saves, written by the last layer's epilogue.  x_ready:
+        prepare_input(x) has already run (the trainer converts the input before it forks the generator onto its own
+        stream)."""
         self._join_wgrad()
         v0 = self.virtual0
         if v0:
@@ -632,7 +663,7 @@ class GeneratorEngine(_Net):
         if v0:
             return self.out_cat
         ops.thin_convT_fwd(self.R[0], self.w_u_T2, self.param(self.k_up[0] + ".bias"), ACT_TANH, self.fake_bf, self.fake_f32,
-                           out_u8)
+                           out_u8, co=self.output_nc)
         self.dropout_calls += 1
         return self.fake_f32
 
@@ -647,8 +678,8 @@ class GeneratorEngine(_Net):
             out = torch.empty(n, 2 * self.C[0], h, w, device=self.dev)
             ops.nhwc_to_nchw_f32(self.out_cat, out, 2 * self.C[0])
             return out
-        out = torch.empty(n, 3, h, w, device=self.dev)
-        ops.nhwc_to_nchw_f32(self.fake_f32, out, 3)
+        out = torch.empty(n, self.output_nc, h, w, device=self.dev)
+        ops.nhwc_to_nchw_f32(self.fake_f32, out, self.output_nc)
         return out
 
     # -- backward -------------------------------------------------------------------------------
@@ -666,8 +697,8 @@ class GeneratorEngine(_Net):
         # outermost up-conv (a stand-alone inner block starts from gR[0] = the gradient of its concatenated output)
 
         def _w0():
-            ops.thin_conv_wgrad(self.R[0], self.dpre, None, gseg(self.k_up[0] + ".weight"), 64)
-            ops.colsum_bf16(self.dpre, 3, self.grad(self.k_up[0] + ".bias"))
+            ops.thin_conv_wgrad(self.R[0], self.dpre, None, gseg(self.k_up[0] + ".weight"), 64, c0=self.output_nc)
+            ops.colsum_bf16(self.dpre, self.output_nc, self.grad(self.k_up[0] + ".bias"))
         if not v0:
             self._fork_wgrad(_w0)
             self._ready(self.k_up[0] + ".weight", self.k_up[0] + ".bias", side=True)
@@ -741,7 +772,7 @@ class GeneratorEngine(_Net):
             return
         dbias0 = self.grad(self.k_down[0] + ".bias") if inst else None
         self._fork_wgrad(lambda: ops.thin_conv_wgrad(self.dyd[0], self.x_nhwc, None, gseg(self.k_down[0] + ".weight"), 64,
-                                                     dbias=dbias0))
+                                                     dbias=dbias0, c0=self.input_nc))
         self._ready(self.k_down[0] + ".weight", *((self.k_down[0] + ".bias",) if inst else ()), side=True)
 
 
@@ -749,7 +780,9 @@ class GeneratorEngine(_Net):
 # Discriminator
 # ================================================================================================
 class DiscriminatorEngine(_Net):
-    """NLayerDiscriminator(input_nc=6, ndf, n_layers, BatchNorm2d or InstanceNorm2d)."""
+    """NLayerDiscriminator(input_nc, ndf, n_layers, BatchNorm2d or InstanceNorm2d) over cat(A, B), input_nc in 2..8:
+    forward takes A and B as two 4-slot sources of split = (channels of A, channels of B) channels, by default
+    discriminator_split(input_nc) (3 | 3 for the reference's 6)."""
 
     # BatchNorm + LeakyReLU of the last normalised layer (models.py:239-240) applied inside the Cout = 1 head's forward
     # and wgrad kernels instead of a separate pass that writes H (63 MB written + re-read per forward at batch 64)
@@ -758,20 +791,25 @@ class DiscriminatorEngine(_Net):
     _BUFFER_ATTRS = ("hs", "ws", "H", "y", "logits", "z_ws", "dlogits", "gH", "dy", "dfake", "_xa", "_xb")
 
     def __init__(self, device, input_nc: int = 6, ndf: int = 64, n_layers: int = 3, init: bool = True,
-                 norm: str = "batch") -> None:
+                 norm: str = "batch", split: Optional[Tuple[int, int]] = None) -> None:
         super().__init__(device, norm)
         if self.norm == "instance":
             # the head's kernels take per-channel (scale, shift) only; InstanceNorm's are per image: H is materialised
             self.fuse_head = False
-        if input_nc != 6:
-            raise NotImplementedError("the native discriminator supports input_nc = 6 (cat of two RGB images)")
+        if split is None:
+            split = discriminator_split(input_nc)
+        else:
+            split = (check_image_channels("split[0]", split[0]), check_image_channels("split[1]", split[1]))
+            if sum(split) != input_nc:
+                raise ValueError(f"split {split} does not add up to input_nc = {input_nc}")
+        self.split = split
         if ndf % 64 != 0 or n_layers < 1:
             raise NotImplementedError("ndf must be a multiple of 64")
         self.spec = sp = DiscriminatorSpec(input_nc, ndf, n_layers, norm=self.norm)
         self.nl = n_layers
         self.C = C = sp.C
         self.k_conv, self.k_bn, self.n_conv = sp.k_conv, sp.k_bn, sp.n_conv
-        self._reg_small(self.k_conv[0] + ".weight", C[0], 6, 128)
+        self._reg_small(self.k_conv[0] + ".weight", C[0], input_nc, 128)
         self._reg_vec(self.k_conv[0] + ".bias", C[0])
         self.bn: List[Optional[_BN]] = [None] * self.n_conv
         for k in range(1, n_layers + 1):
@@ -787,9 +825,10 @@ class DiscriminatorEngine(_Net):
         self.w_fwd = [None] + [torch.zeros(1, C[k], 16 * C[k - 1], **bf) for k in range(1, n_layers + 1)]
         self.w_fwd.append(torch.zeros(1, 1, 16 * C[-1], **bf))
         self.w_dg = [None]
-        # first conv seen from its input gradient: [(kh*4+kw)*3 + ch][64]; B half (channels 3..5) and A half
-        self.w_T2 = torch.zeros(48, C[0], **bf)
-        self.w_T2a = torch.zeros(48, C[0], **bf)
+        # first conv seen from its input gradient: [(kh*4+kw)*c + ch][64] per source; B (channels ca..) and A (0..ca-1)
+        ca, cb = split
+        self.w_T2 = torch.zeros(16 * cb, C[0], **bf)
+        self.w_T2a = torch.zeros(16 * ca, C[0], **bf)
         for k in range(1, n_layers + 1):
             if k < n_layers:
                 self.w_dg.append(torch.zeros(4, C[k - 1], 4 * C[k], **bf))     # stride 2: four phases
@@ -818,11 +857,15 @@ class DiscriminatorEngine(_Net):
         C, p, off = self.C, self.store.p, self.store.off
         plan = ops.PackPlan()
         o = off(self.k_conv[0] + ".weight")
-        plan.add(p, o, self.w_thin, 0, 1, C[0], C[0], (4, 4), 3, 8, 128, (128, 1, 24, 6))
-        plan.add(p, o + 3, self.w_thin, 0, 1, C[0], C[0], (4, 4), 3, 8, 128, (128, 1, 24, 6), out_off=4)
+        ca, cb = self.split
+        c = ca + cb
+        plan.add(p, o, self.w_thin, 0, 1, C[0], C[0], (4, 4), ca, 8, 128, (128, 1, 4 * c, c))
+        plan.add(p, o + ca, self.w_thin, 0, 1, C[0], C[0], (4, 4), cb, 8, 128, (128, 1, 4 * c, c), out_off=4)
         for tap in range(16):
-            plan.add(p, o + 6 * tap + 3, self.w_T2, 0, 1, 3, 3, (1, 1), C[0], C[0], C[0], (1, 128, 0, 0), out_off=3 * tap * C[0])
-            plan.add(p, o + 6 * tap, self.w_T2a, 0, 1, 3, 3, (1, 1), C[0], C[0], C[0], (1, 128, 0, 0), out_off=3 * tap * C[0])
+            plan.add(p, o + c * tap + ca, self.w_T2, 0, 1, cb, cb, (1, 1), C[0], C[0], C[0], (1, 128, 0, 0),
+                     out_off=cb * tap * C[0])
+            plan.add(p, o + c * tap, self.w_T2a, 0, 1, ca, ca, (1, 1), C[0], C[0], C[0], (1, 128, 0, 0),
+                     out_off=ca * tap * C[0])
         for k in range(1, self.n_conv):
             ci = C[k - 1]
             co = 1 if k == self.n_conv - 1 else C[k]
@@ -869,8 +912,8 @@ class DiscriminatorEngine(_Net):
 
     @_on_device
     def forward(self, xa: torch.Tensor, xb: torch.Tensor) -> torch.Tensor:
-        """xa, xb: NHWC bf16 [n,h,w,>=3] (the two halves of torch.cat((A, B), 1), train_gan.py:57,59,66).
-        Returns fp32 logits [n,h',w',1]."""
+        """xa, xb: NHWC bf16 [n,h,w,4 slots] holding split[0] / split[1] channels, the rest zero (the two halves of
+        torch.cat((A, B), 1), train_gan.py:57,59,66).  Returns fp32 logits [n,h',w',1]."""
         n, h, w, _ = xa.shape
         self._join_wgrad()
         self._alloc(n, h, w)
@@ -901,7 +944,8 @@ class DiscriminatorEngine(_Net):
     @_on_device
     def backward(self, wgrad: bool, input_grad: bool, input_grad_a: bool = False, final_hook=None) -> Optional[torch.Tensor]:
         """Consumes self.dlogits (fp32 [n, h', w']).  wgrad=False skips every parameter gradient (the G step);
-        input_grad=True returns d(loss)/d(xb) as fp32 NHWC.  The last conv's bias gradient (sum of dlogits) is
+        input_grad=True returns d(loss)/d(xb) as fp32 NHWC [n,h,w,4] (channels >= split[1] zero); input_grad_a also
+        writes d(loss)/d(xa) into self.dreal.  The last conv's bias gradient (sum of dlogits) is
         produced by whoever wrote dlogits (gap_bce_logits_const_f32 / gap_sum_f32).  final_hook(offset, stream): called
         when this pass has enqueued the last contribution to every gradient from `offset` to the end of the flat buffer
         (the buffer is in forward order, backward finalises it from the tail): the data-parallel reducer starts reducing
@@ -954,12 +998,13 @@ class DiscriminatorEngine(_Net):
         if wgrad:
             self._fork_wgrad(lambda: ops.thin_conv_wgrad(self.dy[0], self._xa, self._xb,
                                                          self.store.seg(g, self.k_conv[0] + ".weight"), 128,
-                                                         dbias=self.grad(self.k_conv[0] + ".bias")))
+                                                         dbias=self.grad(self.k_conv[0] + ".bias"), c0=self.split[0],
+                                                         c1=self.split[1]))
         if input_grad:
-            ops.thin_convT_fwd(self.dy[0], self.w_T2, None, ACT_NONE, None, self.dfake)
+            ops.thin_convT_fwd(self.dy[0], self.w_T2, None, ACT_NONE, None, self.dfake, co=self.split[1])
             if input_grad_a:
                 self.dreal = torch.zeros_like(self.dfake)
-                ops.thin_convT_fwd(self.dy[0], self.w_T2a, None, ACT_NONE, None, self.dreal)
+                ops.thin_convT_fwd(self.dy[0], self.w_T2a, None, ACT_NONE, None, self.dreal, co=self.split[0])
             return self.dfake
         return None
 
@@ -975,14 +1020,19 @@ class Pix2PixTrainer:
 
     def __init__(self, device, lr_g: float = 1e-4, lr_d: float = 1e-4, beta1: float = 0.5, num_downs: int = 7,
                  ngf: int = 64, ndf: int = 64, n_layers: int = 3, allreduce=None, world: int = 1,
-                 bucket_elems: int = 8 << 20, use_dropout: bool = False, norm: str = "batch") -> None:
+                 bucket_elems: int = 8 << 20, use_dropout: bool = False, norm: str = "batch", input_nc: int = 3,
+                 output_nc: int = 3) -> None:
         """norm: "batch" (nn.BatchNorm2d, the reference default) or "instance" (nn.InstanceNorm2d, pix2pix's
-        `--norm instance`) in both networks."""
+        `--norm instance`) in both networks.  input_nc / output_nc (1..4): channels of real_A and of real_B / fake_B;
+        the discriminator sees cat(A, B) with A as its first input_nc channels."""
         self.dev = torch.device(device)
         self.norm = norm
+        self.input_nc = check_image_channels("input_nc", input_nc)
+        self.output_nc = check_image_channels("output_nc", output_nc)
         # construction order G then D fixes the seeded weights (train_gan.py:138-139)
-        self.G = GeneratorEngine(self.dev, 3, 3, num_downs, ngf, use_dropout=use_dropout, norm=norm)
-        self.D = DiscriminatorEngine(self.dev, 6, ndf, n_layers, norm=norm)
+        self.G = GeneratorEngine(self.dev, input_nc, output_nc, num_downs, ngf, use_dropout=use_dropout, norm=norm)
+        self.D = DiscriminatorEngine(self.dev, input_nc + output_nc, ndf, n_layers, norm=norm,
+                                     split=(input_nc, output_nc))
         self.lr_g, self.lr_d, self.betas = lr_g, lr_d, (beta1, 0.999)
         self.loss_acc = torch.zeros(4, device=self.dev, dtype=torch.float64)  # d_real, d_fake, g_gan, l1 (re-zeroed by
         self.loss_out = torch.zeros(2, device=self.dev, dtype=torch.float64)  # gap_gan_losses at the end of each step)
@@ -1055,7 +1105,7 @@ class Pix2PixTrainer:
     def train_step(self, real_A: torch.Tensor, real_B: torch.Tensor,
                    loss_host: Optional[torch.Tensor] = None) -> torch.Tensor:
         """real_A / real_B: fp32 NCHW in [-1, 1] on the device (what the reference's DataLoader yields), or BOTH as raw
-        uint8 [n, h, w, 3] images: the ToTensor + JointNormalize of dataset.py:28-29,155-159 then runs on the device
+        uint8 [n, h, w, input_nc] / [n, h, w, output_nc] images: the ToTensor + JointNormalize of dataset.py:28-29,155-159 then runs on the device
         inside the first kernels (4x less host->device traffic).  Returns a device tensor [loss_d, loss_g] (fp64); no
         host synchronisation happens here.  loss_host: a PINNED host fp64[2] tensor — the step's last kernel then stores
         the two losses straight into host memory (zero-copy over PCIe; valid once the stream has passed that kernel) and
@@ -1066,8 +1116,12 @@ class Pix2PixTrainer:
             raise ValueError("real_A and real_B must both be fp32 NCHW or both uint8 NHWC")
         if u8:
             n, h, w, _ = real_A.shape
+            cb = real_B.shape[-1]
         else:
             n, _, h, w = real_A.shape
+            cb = real_B.shape[1]
+        if cb != self.output_nc:
+            raise ValueError(f"real_B has {cb} channels, expected output_nc = {self.output_nc}")
         if self.a_nhwc is None or self.a_nhwc.shape[:3] != (n, h, w):
             self.a_nhwc = torch.zeros(n, h, w, 4, device=self.dev, dtype=torch.bfloat16)
             self.b_nhwc = torch.zeros_like(self.a_nhwc)
@@ -1121,7 +1175,7 @@ class Pix2PixTrainer:
         logits = D.forward(a_nhwc, G.fake_bf)              # :66 (updated D)
         ops.bce_logits_const_f32(logits, 1.0, 1.0 / cnt, D.dlogits, self.loss_acc[2:3])   # :67
         dfake = D.backward(wgrad=False, input_grad=True)
-        numel = n * 3 * h * w
+        numel = n * self.output_nc * h * w
         ops.gen_out_bwd(G.fake_f32, real_B, dfake, LAMBDA_L1 / numel, G.dpre, self.loss_acc[3:4])  # :68-70
         if self.g_reducer is not None:
             self.g_reducer.begin()

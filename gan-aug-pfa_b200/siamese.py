@@ -43,17 +43,20 @@ class _Saved:
 
 
 class SiameseEngine(_Net):
-    """SiameseUNet(n_channels=3, n_classes=1)."""
+    """SiameseUNet(n_channels, n_classes=1), n_channels = 1..4 (default 3)."""
 
     def __init__(self, device, n_channels: int = 3, n_classes: int = 1) -> None:
         super().__init__(device)
-        if n_channels != 3 or n_classes != 1:
-            raise NotImplementedError("the native Siamese U-Net supports n_channels = 3, n_classes = 1")
+        if n_classes != 1:
+            raise NotImplementedError("the native Siamese U-Net supports n_classes = 1")
+        if not isinstance(n_channels, int) or not 1 <= n_channels <= 4:
+            raise NotImplementedError(f"n_channels = {n_channels!r} is not implemented natively: images of 1 to 4 "
+                                      "channels are")
         self.n_channels, self.n_classes = n_channels, n_classes
         self.key_order: List[str] = []
         self.conv_meta: Dict[str, Tuple[int, int, int]] = {}      # conv key -> (cout, cin, k)
         # ---- registration in the reference's module order (models.py:54-90) = state_dict order
-        cin = 3
+        cin = n_channels
         for name, c in ENC:
             self._reg_double_conv(name, cin, c)
             cin = c
@@ -72,8 +75,8 @@ class SiameseEngine(_Net):
         self.w_fwd: Dict[str, torch.Tensor] = {}
         self.w_dg: Dict[str, torch.Tensor] = {}
         for key, (co, ci, k) in self.conv_meta.items():
-            if ci == 3:
-                self.w_fwd[key] = torch.zeros(1, co, 64, **bf)          # im2col form, K = 27 padded to 64; no dgrad
+            if ci <= 4:
+                self.w_fwd[key] = torch.zeros(1, co, 64, **bf)          # im2col form, K = 9*ci padded to 64; no dgrad
                 continue
             self.w_fwd[key] = torch.zeros(1, co, k * k * ci, **bf)
             self.w_dg[key] = torch.zeros(1, ci, k * k * co, **bf)
@@ -86,8 +89,8 @@ class SiameseEngine(_Net):
 
     # -- registration ------------------------------------------------------------------------------
     def _reg_convk(self, key: str, cout: int, cin: int, k: int, bias: bool) -> None:
-        if cin == 3:      # [cout][(kh*3+kw)*3 + c] padded to 64
-            self._reg(key + ".weight", cout * 64, (cout, 3, k, k), (64, 1, 3 * k, 3))
+        if cin <= 4:      # the image-side first conv: [cout][(kh*3+kw)*cin + c] padded to 64
+            self._reg(key + ".weight", cout * 64, (cout, cin, k, k), (64, 1, cin * k, cin))
         else:             # [cout][kh][kw][cin]
             self._reg(key + ".weight", cout * k * k * cin, (cout, cin, k, k), (k * k * cin, 1, k * cin, cin))
         self.conv_meta[key] = (cout, cin, k)
@@ -123,7 +126,7 @@ class SiameseEngine(_Net):
             p, off = self.store.p, self.store.off
             for key, (co, ci, k) in self.conv_meta.items():
                 o = off(key + ".weight")
-                if ci == 3:
+                if ci <= 4:
                     plan.add(p, o, self.w_fwd[key], 0, 1, co, co, (1, 1), 64, 64, 64, (64, 1, 0, 0))
                     continue
                 kk = k * k
@@ -207,17 +210,17 @@ class SiameseEngine(_Net):
         if not self.training:
             # eval (train.py:151, evaluate.py:146): BatchNorm folds into the conv epilogue; nothing is kept for backward
             self._bn_stats(bn, sv, n * h * w)
-            if ci == 3:
+            if ci <= 4:
                 ops.conv_gemm([x], self.w_fwd[key], ops.geom_conv_fwd(1, 1, 0), out, co, (h, w), act=ACT_RELU,
-                              scale=sv.scale, bias=sv.shift, flops=2.0 * n * h * w * co * 27)
+                              scale=sv.scale, bias=sv.shift, flops=2.0 * n * h * w * co * 9 * ci)
             else:
                 ops.conv_gemm([x], self.w_fwd[key], ops.geom_conv_fwd(3, 1, 1), out, co, (h, w), act=ACT_RELU,
                               scale=sv.scale, bias=sv.shift)
             return {"bn": bn, "sv": sv, "y": y}
         stats = bn.stats
-        if ci == 3:
+        if ci <= 4:
             ops.conv_gemm([x], self.w_fwd[key], ops.geom_conv_fwd(1, 1, 0), y, co, (h, w), stats=stats,
-                          flops=2.0 * n * h * w * co * 27)
+                          flops=2.0 * n * h * w * co * 9 * ci)
         else:
             ops.conv_gemm([x], self.w_fwd[key], ops.geom_conv_fwd(3, 1, 1), y, co, (h, w), stats=stats)
         self._bn_stats(bn, sv, n * h * w)
@@ -236,9 +239,9 @@ class SiameseEngine(_Net):
             wseg = self.store.seg(self.store.g, key + ".weight")
             # weight gradients are off the critical path: they run on the side stream (tensor-bound) underneath the
             # HBM-bound BatchNorm / pooling / gate passes of the layers that follow
-            if ci == 3:
+            if ci <= 4:
                 self._fork_wgrad(lambda: ops.conv_wgrad(dy, x, wseg, (1, 1), 1, (0, 0), 64, 0,
-                                                        flops=2.0 * n * h * w * co * 27))
+                                                        flops=2.0 * n * h * w * co * 9 * ci))
                 return
             self._fork_wgrad(lambda: ops.conv_wgrad(dy, x, wseg, (3, 3), 1, (-1, -1), 9 * ci, ci))
             if gx is None:
@@ -333,8 +336,10 @@ class SiameseEngine(_Net):
         """forward_encoder (models.py:92-102) for branch p: 4 x (double_conv + MaxPool2d(2)) + bottleneck; the features
         land in the channel slots p of the concatenated skip buffers S[0..4]."""
         n = x.shape[0]
+        if x.shape[1] != self.n_channels:
+            raise ValueError(f"input has {x.shape[1]} channels, expected n_channels = {self.n_channels}")
         ops.nchw_to_nhwc_bf16(x.contiguous().float(), self.x_in[p])
-        ops.im2col_k3s1p1_c3(self.x_in[p], self.col[p])
+        ops.im2col_k3s1p1(self.x_in[p], self.col[p], self.n_channels)
         src, gsrc = self.col[p], None
         for lvl, (name, c) in enumerate(ENC):
             out = self.S[lvl][..., p * c:(p + 1) * c]

@@ -220,9 +220,13 @@ int gap_cout1_conv_wgrad(const float* dlogits, int n, int oh, int ow, const void
  * conv (models.py:177, outermost block), the discriminator's first conv over cat(A, B) (models.py:223,
  * train_gan.py:57,59,66) and the input gradient of the generator's last ConvTranspose2d (models.py:184).
  *   out1[pix][co] = act1(bias[co] + sum_{tap,slot} in[2*pix+tap-1][slot] * wpk[co][tap*CT + slot]),  out2 likewise
- * src0 / src1: NHWC bf16 with 4 channel slots used per pixel (3 channels + a zero slot; ld % 4 == 0);
+ * src0 / src1: NHWC bf16 with 4 channel slots used per pixel (1..4 channels, the rest zero slots; ld % 4 == 0);
  * src1 == NULL -> CT = 4, else CT = 8 with src1's slots at 4..7.  wpk: bf16 [cw][16*CT]; cw = 64 or 128;
  * activations: none / LeakyReLU / ReLU.  out2 may be NULL.
+ * The kernel sums over every slot, so it serves any channel count of up to 4 per source provided BOTH the packed
+ * weights of unused slots AND the unused activation slots are zero (0 * NaN = NaN): every producer of a 4-slot image
+ * tensor (the converters below, gap_nchw_f32_to_nhwc_bf16 on zero-initialised buffers, gap_thin_convT_fwd[_c],
+ * gap_gen_out_bwd[_u8]) leaves the slots past its channel count zero.
  * ---------------------------------------------------------------------------------------------- */
 int gap_thin_conv_fwd(const void* src0, int64_t ld0, const void* src1, int64_t ld1, int n, int h, int w, const void* wpk,
                       const float* bias, int cw, void* out1, int64_t ldo1, int act1, void* out2, int64_t ldo2, int act2,
@@ -236,6 +240,12 @@ int gap_thin_conv_fwd(const void* src0, int64_t ld0, const void* src1, int64_t l
  * dbias may be NULL. */
 int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, const void* src1, int64_t ld1,
                         int n, int h, int w, int cw, float* dw, int64_t ld_m, float* dbias, void* stream);
+/* The same with c0 / c1 channels in source 0 / source 1 (c0 = 1..4; c1 = 1..4 with src1, 0 without): slots past a
+ * source's channel count are dropped and slot s of source 1 is master channel c0 + s, in the layout
+ * [cw][(kh*4+kw)*(c0+c1) + ch].  gap_thin_conv_wgrad is c0 = 3, c1 = src1 ? 3 : 0. */
+int gap_thin_conv_wgrad_c(const void* wide, int64_t ld_w, const void* src0, int64_t ld0, int c0, const void* src1,
+                          int64_t ld1, int c1, int n, int h, int w, int cw, float* dw, int64_t ld_m, float* dbias,
+                          void* stream);
 
 /* Thin-output ConvTranspose2d(cw -> 3, k4, s2, p1) (+bias, Tanh): the generator's last layer
  * (models.py:184,186), and — with the first conv's weights — the input gradient of the discriminator's first
@@ -243,11 +253,19 @@ int gap_thin_conv_wgrad(const void* wide, int64_t ld_w, const void* src0, int64_
  * [n, 2ih, 2iw, 4 slots] in bf16 and / or fp32 (slot 3 is written as zero); act = GAP_ACT_NONE or GAP_ACT_TANH. */
 int gap_thin_convT_fwd(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, const void* wcol, const float* bias,
                        int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f, uint8_t* out_u8, void* stream);
+/* ConvTranspose2d(cw -> co, k4, s2, p1) for co = 1..4: wcol bf16 [16*co = (kh*4+kw)*co + c][cw], bias [co] (may be
+ * NULL), outputs [n, 2ih, 2iw, 4 slots] with slots >= co written as zero, out_u8 [n][2ih][2iw][co].
+ * gap_thin_convT_fwd is co = 3. */
+int gap_thin_convT_fwd_c(const void* wide, int64_t ld_w, int n, int ih, int iw, int cw, int co, const void* wcol,
+                         const float* bias, int act, void* out_bf16, int64_t ld_bf, float* out_f32, int64_t ld_f,
+                         uint8_t* out_u8, void* stream);
 /* SURVEY.md §8(f) ranks 1-2 (the I/O either side of the generator): out_u8 above, if not NULL, receives the image
  * generate_synthetic_data.py:69-88 writes to PNG — uint8 [n][2ih][2iw][3] = byte((v*0.5 + 0.5) * 255) — straight from
  * the last layer's epilogue; gap_u8_hwc_to_nhwc_bf16 is dataset.py's ToTensor + Normalize(0.5, 0.5) (dataset.py:155-159)
  * on the device: uint8 HWC [pixels][3] -> NHWC bf16 with 4 channel slots, x*(2/255) - 1. */
 int gap_u8_hwc_to_nhwc_bf16(const uint8_t* x, void* out, int64_t out_ld, int64_t pixels, void* stream);
+/* The same for c = 1..4 channels per pixel (uint8 HWC [pixels][c]); slots >= c are written as zero. */
+int gap_u8_hwc_to_nhwc_bf16_c(const uint8_t* x, int c, void* out, int64_t out_ld, int64_t pixels, void* stream);
 /* The same with dataset.py's JointResize in front (dataset.py:136-153; ToTensor -> resize(BILINEAR) -> Normalize): uint8
  * HWC [n][ih][iw][3] -> antialiased bilinear resize (torchvision's tensor path = F.interpolate(mode="bilinear",
  * align_corners=False, antialias=True)) -> x*2 - 1 -> NHWC bf16 [n][oh][ow][4 slots] and / or (out_nchw_f32) the fp32
@@ -255,6 +273,10 @@ int gap_u8_hwc_to_nhwc_bf16(const uint8_t* x, void* out, int64_t out_ld, int64_t
  * label half of JointResize (InterpolationMode.NEAREST on the int64 {0,1} map, dataset.py:143-146). */
 int gap_resize_u8_to_nhwc_bf16(const uint8_t* x, int n, int ih, int iw, int oh, int ow, void* out, int64_t out_ld,
                                float* out_nchw_f32, void* stream);
+/* The same for c = 1..4 channels per pixel (uint8 HWC [n][ih][iw][c]; out_nchw_f32 [n][c][oh][ow]); bf16 slots >= c are
+ * written as zero.  gap_resize_u8_to_nhwc_bf16 is c = 3. */
+int gap_resize_u8_to_nhwc_bf16_c(const uint8_t* x, int c, int n, int ih, int iw, int oh, int ow, void* out,
+                                 int64_t out_ld, float* out_nchw_f32, void* stream);
 int gap_resize_nearest_i64(const int64_t* x, int n, int ih, int iw, int oh, int ow, int64_t* out, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
@@ -263,6 +285,9 @@ int gap_resize_nearest_i64(const int64_t* x, int n, int ih, int iw, int oh, int 
  * ---------------------------------------------------------------------------------------------- */
 /* im2col of Conv2d(3 -> C, k3, s1, p1) (models.py:9 through :54): col[pix][(kh*3+kw)*3 + c], padded to 64 */
 int gap_im2col_k3s1p1_c3(const void* x, int64_t ld, void* col, int n, int h, int w, void* stream);
+/* The same for c = 1..4 input channels: col[pix][(kh*3+kw)*c + ch], 9*c values padded to 64 (gap_im2col_k3s1p1_c3 is
+ * c = 3) */
+int gap_im2col_k3s1p1_c(const void* x, int64_t ld, int c, void* col, int n, int h, int w, void* stream);
 /* nn.MaxPool2d(2) (models.py:58).  Backward sends the gradient to the first maximum in scan order. */
 int gap_maxpool2x2_fwd(const void* x, int64_t ldx, void* out, int64_t ldo, int n, int h, int w, int c, void* stream);
 int gap_maxpool2x2_bwd(const void* x, int64_t ldx, const void* gout, int64_t ldg, void* gin, int64_t ldi, int n, int h,
