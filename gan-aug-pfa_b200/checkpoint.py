@@ -91,7 +91,8 @@ def load_trainer_state(trainer, state: dict, restore_rng: bool = True) -> dict:
 
 def siamese_state(engine, extra: Optional[dict] = None) -> dict:
     torch.cuda.synchronize(engine.dev)
-    return {"format": FORMAT, "kind": "siamese", "channels": {"n_channels": engine.n_channels}, "net": _net_state(engine),
+    return {"format": FORMAT, "kind": "siamese", "channels": {"n_channels": engine.n_channels},
+            "n_classes": engine.n_classes, "net": _net_state(engine),
             "rng": _rng_state(engine.dev), "extra": extra or {}}
 
 
@@ -102,6 +103,10 @@ def load_siamese_state(engine, state: dict, restore_rng: bool = True) -> dict:
     if ch != engine.n_channels:
         raise ValueError(f"checkpoint was written by a Siamese U-Net with n_channels={ch}; this one has "
                          f"n_channels={engine.n_channels}")
+    k = state.get("n_classes", 1)           # checkpoints written before multi-class support are n_classes = 1 runs
+    if k != engine.n_classes:
+        raise ValueError(f"checkpoint was written by a Siamese U-Net with n_classes={k}; this one has "
+                         f"n_classes={engine.n_classes}")
     _load_net(engine, state["net"])
     if restore_rng:
         _set_rng_state(state["rng"], engine.dev)

@@ -504,7 +504,8 @@ class _SiameseFn(torch.autograd.Function):
         logits = eng.forward(x1.detach(), x2.detach())
         ctx.module = module
         ctx.shape = tuple(logits.shape)
-        return logits.unsqueeze(1).clone()
+        # n_classes = 1: the [n, h, w] map as [n, 1, h, w]; n_classes > 1: the [n, K, h, w] class planes as they are
+        return logits.unsqueeze(1).clone() if logits.dim() == 3 else logits.clone()
 
     @staticmethod
     def backward(ctx, gout):
@@ -518,9 +519,13 @@ class _SiameseFn(torch.autograd.Function):
 
 
 class SiameseUNet(_NativeModule):
-    """Siamese U-Net with attention gates (models.py:47-145) executing on the native sm_100a kernels."""
+    """Siamese U-Net with attention gates (models.py:47-145) executing on the native sm_100a kernels.  n_classes = 1
+    returns [n, 1, h, w] logits for the sigmoid losses; n_classes = 2..16 returns [n, K, h, w] logits for
+    nn.CrossEntropyLoss / torch.argmax(dim=1)."""
 
     def __init__(self, n_channels, n_classes):
+        from .siamese import check_n_classes
+        check_n_classes(n_classes)
         super().__init__()
         self.n_channels = n_channels
         self.n_classes = n_classes

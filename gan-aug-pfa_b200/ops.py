@@ -812,3 +812,139 @@ def seg_confusion(logits: torch.Tensor, labels: torch.Tensor, counts: torch.Tens
         raise ValueError("seg_confusion needs CUDA tensors (there is no CPU path)")
     _lib.check(_lib.lib().gap_seg_confusion(_ptr(logits), _ptr(labels), 1 if labels.dtype == torch.int64 else 0, n,
                                             logits.numel() // n, _ptr(counts), _stream()), "gap_seg_confusion")
+
+
+# ------------------------------------------------------------------------------------------------
+# Multi-class head of SiameseUNet(n_channels, n_classes), K = 1..16 (gap_b200.h "Multi-class head"): fp32 class
+# planes [n][K][h][w]; head input NHWC bf16 [n][h][w][64]
+# ------------------------------------------------------------------------------------------------
+MAX_CLASSES = 16
+
+
+def _check_k(k: int, what: str) -> None:
+    if not isinstance(k, int) or not 1 <= k <= MAX_CLASSES:
+        raise ValueError(f"{what}: the number of classes must be an int in 1..{MAX_CLASSES}, got {k!r}")
+
+
+def _head_input(x: torch.Tensor, what: str) -> tuple[int, int]:
+    """(n, hw) of an NHWC bf16 [n, h, w, 64] head input (a channel slice of a wider buffer is fine)."""
+    if x.dim() != 4 or x.shape[-1] != 64 or x.dtype != torch.bfloat16 or x.stride(-1) != 1:
+        raise ValueError(f"{what}: x must be NHWC bf16 [n, h, w, 64], got {tuple(x.shape)} {x.dtype}")
+    n, h, w, _ = x.shape
+    if x.stride(1) != w * x.stride(2) or x.stride(0) != h * x.stride(1) or x.stride(2) % 8 or x.data_ptr() % 16:
+        raise ValueError(f"{what}: x must have 16-byte aligned rows of a whole number of 8-element vectors")
+    return n, h * w
+
+
+def _planes(t: torch.Tensor, n: int, k: int, hw: int, what: str, name: str) -> None:
+    if t.dtype != torch.float32 or not t.is_contiguous() or t.numel() != n * k * hw or t.shape[0] != n:
+        raise ValueError(f"{what}: {name} must be contiguous fp32 class planes [n={n}, K={k}, h, w], got "
+                         f"{tuple(t.shape)} {t.dtype}")
+
+
+def _head_weight(w: torch.Tensor, k: int, what: str) -> None:
+    if w.dtype != torch.float32 or not w.is_contiguous() or w.numel() != k * 64:
+        raise ValueError(f"{what}: the weight must be contiguous fp32 [K={k}, 64], got {tuple(w.shape)} {w.dtype}")
+
+
+def _cuda(what: str, *ts: Optional[torch.Tensor]) -> None:
+    if not all(t.is_cuda for t in ts if t is not None):
+        raise ValueError(f"{what} needs CUDA tensors (there is no CPU path)")
+
+
+def conv1x1_ck_fwd(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, out: torch.Tensor,
+                   pred: Optional[torch.Tensor] = None) -> None:
+    """out [n, K, h, w] fp32 = Conv2d(64 -> K, 1)(x) + bias; pred (uint8 [n, h, w], optional) = argmax over K."""
+    what = "conv1x1_ck_fwd"
+    n, hw = _head_input(x, what)
+    k = out.shape[1] if out.dim() == 4 else -1
+    _check_k(k, what)
+    _planes(out, n, k, hw, what, "out")
+    _head_weight(w, k, what)
+    if bias.dtype != torch.float32 or not bias.is_contiguous() or bias.numel() != k:
+        raise ValueError(f"{what}: bias must be contiguous fp32 [{k}]")
+    if pred is not None and (pred.dtype != torch.uint8 or not pred.is_contiguous() or pred.numel() != n * hw):
+        raise ValueError(f"{what}: pred must be contiguous uint8 [n, h, w]")
+    _cuda(what, x, w, bias, out, pred)
+    _lib.check(_lib.lib().gap_conv1x1_ck_fwd(_ptr(x), x.stride(2), _ptr(w), _ptr(bias), k, n, hw, _ptr(out), _ptr(pred),
+                                             _stream()), "gap_conv1x1_ck_fwd")
+
+
+def conv1x1_ck_dgrad(dl: torch.Tensor, w: torch.Tensor, gx: torch.Tensor) -> None:
+    """gx [n, h, w, 64] bf16 (written) = sum_c dl[:, c] * w[c]."""
+    what = "conv1x1_ck_dgrad"
+    n, hw = _head_input(gx, what)
+    k = dl.shape[1] if dl.dim() == 4 else -1
+    _check_k(k, what)
+    _planes(dl, n, k, hw, what, "dl")
+    _head_weight(w, k, what)
+    _cuda(what, dl, w, gx)
+    _lib.check(_lib.lib().gap_conv1x1_ck_dgrad(_ptr(dl), _ptr(w), k, n, hw, _ptr(gx), gx.stride(2), _stream()),
+               "gap_conv1x1_ck_dgrad")
+
+
+def conv1x1_ck_wgrad(dl: torch.Tensor, x: torch.Tensor, dw: torch.Tensor, db: Optional[torch.Tensor]) -> None:
+    """dw [K, 64] += sum_pix dl[c, pix] * x[pix]; db [K] += sum_pix dl[c, pix] (fp32, accumulated)."""
+    what = "conv1x1_ck_wgrad"
+    n, hw = _head_input(x, what)
+    k = dl.shape[1] if dl.dim() == 4 else -1
+    _check_k(k, what)
+    _planes(dl, n, k, hw, what, "dl")
+    _head_weight(dw, k, what)
+    if db is not None and (db.dtype != torch.float32 or not db.is_contiguous() or db.numel() != k):
+        raise ValueError(f"{what}: db must be contiguous fp32 [{k}]")
+    _cuda(what, dl, x, dw, db)
+    _lib.check(_lib.lib().gap_conv1x1_ck_wgrad(_ptr(dl), _ptr(x), x.stride(2), k, n, hw, _ptr(dw), _ptr(db), _stream()),
+               "gap_conv1x1_ck_wgrad")
+
+
+def _labels(labels: torch.Tensor, n: int, hw: int, what: str) -> None:
+    if labels.dtype != torch.int64 or not labels.is_contiguous() or labels.numel() != n * hw:
+        raise ValueError(f"{what}: labels must be contiguous int64 [n, h, w] matching the logits")
+
+
+def seg_ce_loss(logits: torch.Tensor, labels: torch.Tensor, class_weight: Optional[torch.Tensor], ignore_index: int,
+                sums2: torch.Tensor, bad_labels: torch.Tensor, grad: Optional[torch.Tensor], grad_scale: float,
+                loss: torch.Tensor) -> None:
+    """nn.CrossEntropyLoss(weight=class_weight, ignore_index=ignore_index) on fp32 class planes [n, K, h, w] against
+    int64 labels [n, h, w]: loss (fp64 [1], written) and grad = grad_scale * d(loss)/d(logits).  bad_labels (int64 [1])
+    counts the labels outside [0, K) that are not ignore_index; they contribute nothing."""
+    what = "seg_ce_loss"
+    if logits.dim() != 4:
+        raise ValueError(f"{what}: logits must be class planes [n, K, h, w], got {tuple(logits.shape)}")
+    n, k = logits.shape[0], logits.shape[1]
+    hw = logits.shape[2] * logits.shape[3]
+    _check_k(k, what)
+    _planes(logits, n, k, hw, what, "logits")
+    _labels(labels, n, hw, what)
+    if grad is not None:
+        _planes(grad, n, k, hw, what, "grad")
+    if class_weight is not None and (class_weight.dtype != torch.float32 or not class_weight.is_contiguous()
+                                     or class_weight.numel() != k):
+        raise ValueError(f"{what}: class_weight must be contiguous fp32 [{k}]")
+    if sums2.dtype != torch.float64 or sums2.numel() < 2 or loss.dtype != torch.float64 or loss.numel() < 1:
+        raise ValueError(f"{what}: sums2 must be fp64 [2] and loss fp64 [1]")
+    if bad_labels.dtype != torch.int64 or bad_labels.numel() < 1:
+        raise ValueError(f"{what}: bad_labels must be int64 [1]")
+    _cuda(what, logits, labels, class_weight, sums2, bad_labels, grad, loss)
+    _lib.check(_lib.lib().gap_seg_ce_loss(_ptr(logits), _ptr(labels), k, n, hw, _ptr(class_weight), int(ignore_index),
+                                          _ptr(sums2), _ptr(bad_labels), _ptr(grad), grad_scale, _ptr(loss), _stream()),
+               "gap_seg_ce_loss")
+
+
+def seg_confusion_ck(logits: torch.Tensor, labels: torch.Tensor, ignore_index: int, counts: torch.Tensor) -> None:
+    """counts [n, K, K] (int64, accumulated) += per-sample confusion matrix: rows = label, columns = argmax over the
+    K planes of logits [n, K, h, w]; labels equal to ignore_index or outside [0, K) are skipped."""
+    what = "seg_confusion_ck"
+    if logits.dim() != 4:
+        raise ValueError(f"{what}: logits must be class planes [n, K, h, w], got {tuple(logits.shape)}")
+    n, k = logits.shape[0], logits.shape[1]
+    hw = logits.shape[2] * logits.shape[3]
+    _check_k(k, what)
+    _planes(logits, n, k, hw, what, "logits")
+    _labels(labels, n, hw, what)
+    if counts.dtype != torch.int64 or tuple(counts.shape) != (n, k, k) or not counts.is_contiguous():
+        raise ValueError(f"{what}: counts must be a contiguous int64 [n={n}, {k}, {k}] tensor")
+    _cuda(what, logits, labels, counts)
+    _lib.check(_lib.lib().gap_seg_confusion_ck(_ptr(logits), _ptr(labels), k, n, hw, int(ignore_index), _ptr(counts),
+                                               _stream()), "gap_seg_confusion_ck")

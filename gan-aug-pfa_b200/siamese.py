@@ -11,6 +11,11 @@ channel slots of the concatenated skip buffers S_k = [conv_k(x1) | conv_k(x2)] a
 D_k = [upsample(prev) | attention(S_k)], so no torch.cat ever copies.  The shared encoder runs twice, so its
 BatchNorm layers keep one set of saved statistics per pass (and update their running buffers twice, like the
 reference).  Single-channel maps (psi, logits) are fp32.
+
+Classes: n_classes = K = 1..16.  The logits and their gradient are fp32 class planes [n][K][h][w] (NCHW, what
+nn.CrossEntropyLoss and torch.argmax(dim=1) expect; for K = 1 the same memory as the [n][h][w] map, which keeps its
+shape).  K = 1 runs the single-channel conv_last kernels and the sigmoid losses; K > 1 runs the gap_conv1x1_ck_* head
+kernels and softmax cross-entropy (`kind="ce"`).
 """
 from __future__ import annotations
 
@@ -23,8 +28,16 @@ from .ops import ACT_NONE, ACT_RELU
 from .pix2pix import BN_EPS, BN_MOMENTUM, _BN, _Net, _on_device
 
 ENC = (("dconv_down1", 64), ("dconv_down2", 128), ("dconv_down3", 256), ("dconv_down4", 512), ("bottleneck", 1024))
+MAX_CLASSES = ops.MAX_CLASSES
 DEC = (("att3", "dconv_up3", 2048, 1024, 512), ("att2", "dconv_up2", 512, 512, 256), ("att1", "dconv_up1", 256, 256, 128),
        ("att_last", "dconv_last", 128, 128, 64))      # (gate, block, F_g, F_l, block out channels)
+
+
+def check_n_classes(n_classes) -> None:
+    """NotImplementedError unless n_classes is an int in 1..16 (the classes the native head kernels cover)."""
+    if isinstance(n_classes, bool) or not isinstance(n_classes, int) or not 1 <= n_classes <= MAX_CLASSES:
+        raise NotImplementedError(f"n_classes = {n_classes!r} is not implemented natively: 1 to {MAX_CLASSES} classes "
+                                  "are")
 
 
 def _k(name: str, leaf: str) -> str:
@@ -43,12 +56,11 @@ class _Saved:
 
 
 class SiameseEngine(_Net):
-    """SiameseUNet(n_channels, n_classes=1), n_channels = 1..4 (default 3)."""
+    """SiameseUNet(n_channels, n_classes), n_channels = 1..4 (default 3), n_classes = 1..16 (default 1)."""
 
     def __init__(self, device, n_channels: int = 3, n_classes: int = 1) -> None:
         super().__init__(device)
-        if n_classes != 1:
-            raise NotImplementedError("the native Siamese U-Net supports n_classes = 1")
+        check_n_classes(n_classes)
         if not isinstance(n_channels, int) or not 1 <= n_channels <= 4:
             raise NotImplementedError(f"n_channels = {n_channels!r} is not implemented natively: images of 1 to 4 "
                                       "channels are")
@@ -64,8 +76,8 @@ class SiameseEngine(_Net):
             self._reg_gate(gate, fg, fl, fl // 2)
         for _, block, fg, fl, cout in DEC:
             self._reg_double_conv(block, fg + fl, cout)
-        self._reg("conv_last.weight", 64, (1, 64, 1, 1), (64, 1, 1, 1))
-        self._reg_vec("conv_last.bias", 1)
+        self._reg("conv_last.weight", n_classes * 64, (n_classes, 64, 1, 1), (64, 1, 1, 1))
+        self._reg_vec("conv_last.bias", n_classes)
         self.key_order += ["conv_last.weight", "conv_last.bias"]
         self.store.allocate(device)
         for bn in self.bns.values():
@@ -86,6 +98,11 @@ class SiameseEngine(_Net):
         self._marks: Dict[int, int] = {}     # tape index -> flat-buffer offset from which every gradient is final once
         #                                      that entry has run (the backward pass finalises the buffer tail first)
         self.reducer = None                  # parallel.TailReducer when data parallel (see train_step)
+        # cross-entropy (n_classes > 1): fp64 workspace, and the count of labels outside [0, K) that are not
+        # ignore_index (they contribute nothing to the loss; the count is never reset by the engine)
+        self.ce_sums = torch.zeros(2, device=device, dtype=torch.float64)
+        self.bad_labels = torch.zeros(1, device=device, dtype=torch.int64)
+        self._cw_cache = (None, None)
 
     # -- registration ------------------------------------------------------------------------------
     def _reg_convk(self, key: str, cout: int, cin: int, k: int, bias: bool) -> None:
@@ -157,8 +174,9 @@ class SiameseEngine(_Net):
             hh, ww = h >> lvl, w >> lvl
             self.D.append(z(hh, ww, fg + fl))
             self.gD.append(z(hh, ww, fg + fl))
-        self.logits = torch.empty(n, h, w, device=dev)
-        self.dlogits = torch.zeros(n, h, w, device=dev)
+        planes = (n, h, w) if self.n_classes == 1 else (n, self.n_classes, h, w)
+        self.logits = torch.empty(*planes, device=dev)
+        self.dlogits = torch.zeros(*planes, device=dev)
         self.tmp: Dict[Tuple[int, ...], torch.Tensor] = {}
         self.saved: Dict[Tuple[str, int], _Saved] = {}
         self.loss_sums = torch.zeros(4, device=dev, dtype=torch.float64)
@@ -375,8 +393,9 @@ class SiameseEngine(_Net):
         self._tape = []
 
     @_on_device
-    def forward(self, x1: torch.Tensor, x2: torch.Tensor) -> torch.Tensor:
-        """x1, x2: fp32 NCHW on the device.  Returns fp32 logits [n, h, w] (n_classes = 1)."""
+    def forward(self, x1: torch.Tensor, x2: torch.Tensor, pred: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """x1, x2: fp32 NCHW on the device.  Returns fp32 logits [n, h, w] (n_classes = 1) or class planes
+        [n, K, h, w] (n_classes = K > 1); pred (uint8 [n, h, w], K > 1 only) receives the argmax class map."""
         n, _, h, w = x1.shape
         self._alloc(n, h, w)
         self._tape = []
@@ -399,17 +418,46 @@ class SiameseEngine(_Net):
             self._double_conv(d, block, out, 0, gd, gout)
             prev, gprev = out, gout
         self._last, self._glast = prev, gprev
-        ops.conv1x1_cout1_fwd(prev, self.store.seg(self.store.p, "conv_last.weight"), self.param("conv_last.bias"),
-                              self.logits.view(-1))
+        if self.n_classes == 1:
+            ops.conv1x1_cout1_fwd(prev, self.store.seg(self.store.p, "conv_last.weight"), self.param("conv_last.bias"),
+                                  self.logits.view(-1))
+        else:
+            ops.conv1x1_ck_fwd(prev, self.store.seg(self.store.p, "conv_last.weight"), self.param("conv_last.bias"),
+                               self.logits, pred)
         return self.logits
+
+    @_on_device
+    def predict(self, x1: torch.Tensor, x2: torch.Tensor, out_u8: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Eval-mode forward (BatchNorm with the running statistics) that returns the uint8 class map [n, h, w]: the
+        argmax over the K class planes, ties to the lowest class as torch.argmax(dim=1).  n_classes > 1 only."""
+        if self.n_classes == 1:
+            raise ValueError("predict() returns the argmax over n_classes > 1 planes; with n_classes = 1 threshold the "
+                             "logits of forward()")
+        n, _, h, w = x1.shape
+        if out_u8 is None:
+            out_u8 = torch.empty(n, h, w, device=self.dev, dtype=torch.uint8)
+        was = self.training
+        self.training = False
+        try:
+            self.forward(x1, x2, pred=out_u8)
+        finally:
+            self.training = was
+            self._tape = []
+        return out_u8
 
     # -- backward --------------------------------------------------------------------------------------
     @_on_device
     def backward(self) -> None:
-        """Consumes self.dlogits (fp32 [n, h, w]); accumulates every parameter gradient."""
-        dl = self.dlogits.view(-1)
-        ops.conv1x1_cout1_wgrad(dl, self._last, self.store.seg(self.store.g, "conv_last.weight"), self.grad("conv_last.bias"))
-        ops.conv1x1_cout1_dgrad(dl, self.store.seg(self.store.p, "conv_last.weight"), self._glast)
+        """Consumes self.dlogits (fp32 [n, h, w] or [n, K, h, w]); accumulates every parameter gradient."""
+        if self.n_classes == 1:
+            dl = self.dlogits.view(-1)
+            ops.conv1x1_cout1_wgrad(dl, self._last, self.store.seg(self.store.g, "conv_last.weight"),
+                                    self.grad("conv_last.bias"))
+            ops.conv1x1_cout1_dgrad(dl, self.store.seg(self.store.p, "conv_last.weight"), self._glast)
+        else:
+            ops.conv1x1_ck_wgrad(self.dlogits, self._last, self.store.seg(self.store.g, "conv_last.weight"),
+                                 self.grad("conv_last.bias"))
+            ops.conv1x1_ck_dgrad(self.dlogits, self.store.seg(self.store.p, "conv_last.weight"), self._glast)
         for idx in range(len(self._tape) - 1, -1, -1):
             self._tape[idx]()
             if self.reducer is not None and idx in self._marks:
@@ -419,10 +467,37 @@ class SiameseEngine(_Net):
         self._tape = []
 
     # -- one training iteration (train.py:137-146) ------------------------------------------------------
-    def loss_and_grad(self, labels: torch.Tensor, kind: str = "combined", **kw) -> torch.Tensor:
-        """CombinedLoss (train.py:82-105) or FocalDiceLoss (train.py:108-128) on self.logits; writes d(loss)/d(logits)
-        into self.dlogits and returns the loss as a device fp64 scalar tensor."""
-        if kind == "combined":
+    def _class_weight(self, class_weight) -> Optional[torch.Tensor]:
+        if class_weight is None:
+            return None
+        if isinstance(class_weight, torch.Tensor) and class_weight.device == self.dev:
+            return class_weight.detach().float().contiguous()
+        key = tuple(float(v) for v in (class_weight.tolist() if isinstance(class_weight, torch.Tensor) else class_weight))
+        if self._cw_cache[0] != key:         # one upload per distinct weight vector, not one per step
+            self._cw_cache = (key, torch.tensor(key, device=self.dev, dtype=torch.float32))
+        return self._cw_cache[1]
+
+    def loss_and_grad(self, labels: torch.Tensor, kind: Optional[str] = None, **kw) -> torch.Tensor:
+        """The loss on self.logits; writes d(loss)/d(logits) into self.dlogits and returns the loss as a device fp64
+        scalar tensor.  n_classes = 1: kind "combined" (CombinedLoss, train.py:82-105; the default) or "focal_dice"
+        (FocalDiceLoss, train.py:108-128).  n_classes > 1: kind "ce" (the default), nn.CrossEntropyLoss(
+        weight=class_weight, ignore_index=ignore_index) with class_weight a length-K sequence or device tensor."""
+        k = self.n_classes
+        if kind is None:
+            kind = "combined" if k == 1 else "ce"
+        if (kind == "ce") != (k > 1) and kind in ("ce", "combined", "focal_dice"):
+            raise ValueError(f"loss kind {kind!r} does not apply to n_classes = {k}: use kind='ce' with n_classes > 1 "
+                             "and 'combined' or 'focal_dice' with n_classes = 1")
+        if kind == "ce":
+            unknown = set(kw) - {"class_weight", "ignore_index"}
+            if unknown:
+                raise ValueError(f"kind='ce' takes class_weight and ignore_index, not {sorted(unknown)}")
+            cw = self._class_weight(kw.get("class_weight"))
+            if cw is not None and cw.numel() != k:
+                raise ValueError(f"class_weight has {cw.numel()} entries; n_classes = {k}")
+            ops.seg_ce_loss(self.logits, labels.contiguous(), cw, int(kw.get("ignore_index", -100)), self.ce_sums,
+                            self.bad_labels, self.dlogits, 1.0, self.loss_out)
+        elif kind == "combined":
             alpha = kw.get("alpha", 0.5)
             ops.seg_loss(self.logits, labels, 0, alpha, 1.0 - alpha, kw.get("pos_weight", 9.0), kw.get("smooth", 1.0), 0.0,
                          0.0, self.loss_sums, self.dlogits, 1.0, self.loss_out)
@@ -436,10 +511,15 @@ class SiameseEngine(_Net):
 
     @_on_device
     def train_step(self, img1: torch.Tensor, img2: torch.Tensor, labels: torch.Tensor, lr: float = 1.0152e-4,
-                   weight_decay: float = 1.118e-5, kind: str = "combined", grad_scale: float = 1.0, allreduce=None,
+                   weight_decay: float = 1.118e-5, kind: Optional[str] = None, grad_scale: float = 1.0, allreduce=None,
                    **loss_kw) -> torch.Tensor:
         """zero_grad -> forward -> criterion -> backward -> AdamW step (train.py:140-144).  Data parallel: set
-        `self.reducer = parallel.TailReducer(self.store.g)` (or pass `allreduce`) and grad_scale = 1 / world."""
+        `self.reducer = parallel.TailReducer(self.store.g)` (or pass `allreduce`) and grad_scale = 1 / world.  kind: see
+        loss_and_grad ("combined" for n_classes = 1, "ce" for n_classes > 1 by default)."""
+        if kind is None:
+            kind = "combined" if self.n_classes == 1 else "ce"
+        if (kind == "ce") != (self.n_classes > 1) and kind in ("ce", "combined", "focal_dice"):
+            self.loss_and_grad(None, kind)          # raises the pairing error before any work is enqueued
         self.training = True
         self.zero_grad()
         self.forward(img1, img2)

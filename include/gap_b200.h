@@ -334,6 +334,33 @@ int gap_seg_loss(const float* logits, const int64_t* labels, int64_t n, int mode
                  float pos_weight, float smooth, float gamma, float focal_alpha, double* sums4, float* grad,
                  float grad_scale, double* loss, void* stream);
 
+/* Multi-class head of SiameseUNet(n_channels, n_classes), K = n_classes = 1..16 (seg_head.cu).
+ * Layout: logits and their gradient are fp32 class planes [n][K][hw] (NCHW: what nn.CrossEntropyLoss and
+ * torch.argmax(dim=1) take; for K = 1 the same memory as the [n][hw] map of the single-class path).  The head input
+ * x is the NHWC bf16 output of dconv_last, [n*hw][64] with row stride ldx (a multiple of 8); w is the fp32 master
+ * conv_last.weight [K][64] (rounded to bf16 in the kernels), bias [K].
+ *   fwd:   out[n][c][p] = bias[c] + sum_ch w[c][ch] * x[pix][ch];  pred (optional, uint8 [n][hw]) = argmax over c
+ *          (ties to the lowest index, NaN above everything, as torch.argmax)
+ *   dgrad: gx[pix][ch] = sum_c dl[c][pix] * w[c][ch], bf16, written (not accumulated) into channels 0..63 of rows ldg apart
+ *   wgrad: dw[c][ch] += sum_pix dl[c][pix] * x[pix][ch], db[c] += sum_pix dl[c][pix] (db optional) */
+int gap_conv1x1_ck_fwd(const void* x, int64_t ldx, const float* w, const float* bias, int k, int n, int64_t hw,
+                       float* out, uint8_t* pred, void* stream);
+int gap_conv1x1_ck_dgrad(const float* dl, const float* w, int k, int n, int64_t hw, void* gx, int64_t ldg, void* stream);
+int gap_conv1x1_ck_wgrad(const float* dl, const void* x, int64_t ldx, int k, int n, int64_t hw, float* dw, float* db,
+                         void* stream);
+/* nn.CrossEntropyLoss(weight=class_weight, ignore_index, reduction="mean") over the K planes against int64 labels
+ * [n][hw]: loss[0] = sum w[y] * (logsumexp - x[y]) / sum w[y] over labels != ignore_index (NaN when there are none);
+ * grad (may be NULL) = grad_scale * d(loss)/d(logits) in the plane layout.  class_weight fp32 [K] or NULL (all 1).
+ * A label outside [0, K) that is not ignore_index contributes nothing and adds 1 to *bad_labels (never zeroed here).
+ * sums2 is a 2-double workspace.  No host synchronisation. */
+int gap_seg_ce_loss(const float* logits, const int64_t* labels, int k, int n, int64_t hw, const float* class_weight,
+                    int64_t ignore_index, double* sums2, int64_t* bad_labels, float* grad, float grad_scale,
+                    double* loss, void* stream);
+/* Per-sample K x K confusion matrix: counts[n][label][argmax_c logits] += 1 (int64, accumulated: the caller zeroes it
+ * once); pixels whose label is ignore_index or outside [0, K) are skipped.  n < 65536. */
+int gap_seg_confusion_ck(const float* logits, const int64_t* labels, int k, int n, int64_t hw, int64_t ignore_index,
+                         int64_t* counts, void* stream);
+
 /* evaluate.py:34-64 calculate_metrics, device side: per-sample counts[n][4] += [TP, FP, FN, TN] of
  * (sigmoid(logits) > 0.5) against {0,1} labels (int64 when labels_are_i64, else fp32); logits are [n][hw] fp32.
  * The caller zeroes counts once and may accumulate several batches; the ratios are formed on the host. */
