@@ -1,12 +1,12 @@
 // Multi-class head of the Siamese U-Net: SiameseUNet(n_channels, n_classes) with n_classes = K = 1..16
-// (models.py:90 `conv_last = nn.Conv2d(64, n_classes, 1)`), nn.CrossEntropyLoss on its output and the per-sample
-// K x K confusion matrix.
+// (models.py:90 `conv_last = nn.Conv2d(64, n_classes, 1)`), nn.CrossEntropyLoss on its output, the softmax CE / focal
+// + multi-class Dice losses and the per-sample K x K confusion matrix.
 //
 // Layout: the logits and their gradient are fp32 class planes [n][K][hw] (NCHW, what nn.CrossEntropyLoss and
 // torch.argmax(dim=1) expect); for K = 1 that is the [n][hw] map of the single-class path.  The head input is the
 // NHWC bf16 output of dconv_last, [pix][64] with a row stride of ldx elements.
 //
-// All five kernels are HBM-bound (the head input alone is 128 B per pixel, the planes 4K B).  The conv kernels run
+// All these kernels are HBM-bound (the head input alone is 128 B per pixel, the planes 4K B).  The conv kernels run
 // on warp MMAs (mma.sync m16n8k16, bf16 in, fp32 accumulate) with the operands read straight from global memory into
 // fragments: the reduction axis of an MMA may be permuted freely as long as A and B agree, and so may the columns
 // of the result, so each kernel picks the permutation under which every lane loads and stores whole 16-byte vectors.
@@ -386,6 +386,233 @@ __global__ void ce_finish_kernel(const CeArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// Softmax point term + multi-class Dice over the K planes, p = softmax(x), V = pixels with y != ignore, 0 <= y < K:
+//   loss = w_point * Point + (1 - w_point) * Dice,   Dice = 1 - 1/(K-1) sum_{k>=1} (2 I_k + s) / (P_k + T_k + s)
+//   I_k = sum_V p_k [y=k], P_k = sum_V p_k, T_k = sum_V [y=k]  (whole batch; class 0 is not a Dice class)
+//   mode 0: Point = sum_V w[y] (-log p_y) / sum_V w[y]                   (nn.CrossEntropyLoss(weight, ignore_index))
+//   mode 1: Point = sum_V a[y] (1 - p_y)^gamma (-log p_y) / |V|          (softmax focal loss, a = class_weight)
+// Pass 1 (stats) reads planes and labels once and accumulates the fp64 sums [num, norm, I_1.., P_1.., T_1..]
+// (3(K-1)+2 of them) and the out-of-range label count; pass 2 derives the per-class Dice coefficients from the sums in
+// every CTA (no finalize launch, no host sync), recomputes the softmax and writes the gradient; block 0 writes the loss.
+// ------------------------------------------------------------------------------------------------
+constexpr int kDiceSums = 3 * (kMaxClasses - 1) + 2;
+
+struct DiceArgs {
+  const float* x;
+  const long long* labels;
+  const float* weight;     // [K] or NULL (all 1)
+  long long ignore;
+  int k, mode;
+  long long hw, npix;
+  float w_point, gamma, smooth;
+  double* sums;            // [3(K-1)+2]
+  long long* bad;          // += out-of-range labels
+  float* grad;             // may be NULL
+  float grad_scale;
+  double* loss;
+};
+
+// (1 - q)^gamma (-log q) and its log-ratio helper for the focal term, from r = sum_{c != y} p_c (accurate for confident
+// pixels, where 1 - q cancels) and nll_lse = lse - x_y (accurate for unlikely labels, where log1p(-r) rounds)
+__device__ __forceinline__ float focal_nll(float r, float nll_lse) { return r < 0.5f ? -log1pf(-r) : nll_lse; }
+__device__ __forceinline__ float focal_logq_over_r(float r, float nll_lse) {   // log(q) / r, -> -1 at r = 0
+  return r == 0.f ? -1.f : (r < 0.5f ? log1pf(-r) / r : -nll_lse / r);
+}
+__device__ __forceinline__ float pow_gamma(float r, float gamma) { return gamma == 2.f ? r * r : powf(r, gamma); }
+
+template <int K>
+__global__ void __launch_bounds__(256) dice_stats_kernel(const DiceArgs a) {
+  const int k = K > 0 ? K : a.k;
+  float I[kMaxClasses], P[kMaxClasses], T[kMaxClasses];
+#pragma unroll
+  for (int c = 0; c < kMaxClasses; ++c) I[c] = P[c] = T[c] = 0.f;
+  float num = 0.f, norm = 0.f;
+  unsigned int nbad = 0;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < a.npix;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long y = a.labels[i];
+    if (y == a.ignore) continue;
+    if (y < 0 || y >= k) {
+      ++nbad;
+      continue;
+    }
+    const long long base = i + (i / a.hw) * (k - 1) * a.hw;
+    float v[kMaxClasses];
+    float m = -INFINITY, xy = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        v[c] = a.x[base + c * a.hw];
+        m = fmaxf(m, v[c]);
+        if (c == y) xy = v[c];
+      }
+    }
+    float se = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        v[c] = expf(v[c] - m);
+        se += v[c];
+      }
+    }
+    const float inv_se = 1.f / se;
+    float r = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        const float p = v[c] * inv_se;
+        P[c] += p;
+        if (c == y) {
+          I[c] += p;
+          T[c] += 1.f;
+        } else {
+          r += p;
+        }
+      }
+    }
+    const float nll_lse = m + logf(se) - xy;
+    const float wy = a.weight ? __ldg(a.weight + y) : 1.f;
+    if (a.mode == 0) {
+      num += wy * nll_lse;
+      norm += wy;
+    } else {
+      num += wy * pow_gamma(r, a.gamma) * focal_nll(r, nll_lse);
+      norm += 1.f;
+    }
+  }
+  // CTA reduction in fp64: warp shuffles, then one slot per (sum, warp) in shared memory, one atomic per sum
+  __shared__ double red[kDiceSums][8];
+  __shared__ unsigned int red_bad[8];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int nsum = 3 * (k - 1) + 2;
+  auto put = [&](int s, float v) {
+    const double d = warp_sum_d(static_cast<double>(v));
+    if (lane == 0) red[s][wid] = d;
+  };
+  put(0, num);
+  put(1, norm);
+#pragma unroll
+  for (int c = 1; c < kMaxClasses; ++c) {
+    if (c < k) {
+      put(1 + c, I[c]);
+      put(k + c, P[c]);
+      put(2 * k - 1 + c, T[c]);
+    }
+  }
+  for (int o = 16; o > 0; o >>= 1) nbad += __shfl_xor_sync(0xffffffffu, nbad, o);
+  if (lane == 0) red_bad[wid] = nbad;
+  __syncthreads();
+  const int nw = blockDim.x >> 5;
+  for (int s = threadIdx.x; s < nsum; s += blockDim.x) {
+    double t = 0.0;
+    for (int w = 0; w < nw; ++w) t += red[s][w];
+    if (t != 0.0) atomicAdd(a.sums + s, t);
+  }
+  if (threadIdx.x == 0) {
+    unsigned long long b = 0;
+    for (int w = 0; w < nw; ++w) b += red_bad[w];
+    if (b) atomicAdd(reinterpret_cast<unsigned long long*>(a.bad), b);
+  }
+}
+
+template <int K>
+__global__ void __launch_bounds__(256) dice_grad_kernel(const DiceArgs a) {
+  const int k = K > 0 ? K : a.k;
+  // g_c = A_c [y=c] + B_c is d(Dice)/d(p_c) at a counted pixel (A_0 = B_0 = 0)
+  __shared__ float sA[kMaxClasses], sB[kMaxClasses];
+  __shared__ float s_inv_norm;
+  const double* S = a.sums;
+  if (threadIdx.x < kMaxClasses) {
+    const int c = threadIdx.x;
+    float A = 0.f, B = 0.f;
+    if (c >= 1 && c < k) {
+      const double U = S[k + c] + S[2 * k - 1 + c] + a.smooth;
+      A = static_cast<float>(-2.0 / ((k - 1) * U));
+      B = static_cast<float>((2.0 * S[1 + c] + a.smooth) / ((k - 1) * U * U));
+    }
+    sA[c] = A;
+    sB[c] = B;
+  }
+  if (threadIdx.x == 0) {
+    s_inv_norm = static_cast<float>(1.0 / S[1]);
+    if (blockIdx.x == 0) {
+      double ratio = 0.0;
+      for (int c = 1; c < k; ++c) ratio += (2.0 * S[1 + c] + a.smooth) / (S[k + c] + S[2 * k - 1 + c] + a.smooth);
+      const double dice = 1.0 - ratio / (k - 1);
+      a.loss[0] = a.w_point * (S[0] / S[1]) + (1.0 - a.w_point) * dice;
+    }
+  }
+  if (a.grad == nullptr) return;
+  __syncthreads();
+  float A[kMaxClasses], B[kMaxClasses];
+#pragma unroll
+  for (int c = 0; c < kMaxClasses; ++c) {
+    A[c] = c < k ? sA[c] : 0.f;
+    B[c] = c < k ? sB[c] : 0.f;
+  }
+  const float inv_norm = s_inv_norm;
+  const float wp = a.grad_scale * a.w_point, wd = a.grad_scale * (1.f - a.w_point);
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < a.npix;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long base = i + (i / a.hw) * (k - 1) * a.hw;
+    const long long y = a.labels[i];
+    if (y == a.ignore || y < 0 || y >= k) {
+#pragma unroll
+      for (int c = 0; c < kMaxClasses; ++c)
+        if (c < k) a.grad[base + c * a.hw] = 0.f;
+      continue;
+    }
+    float v[kMaxClasses];
+    float m = -INFINITY, xy = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        v[c] = a.x[base + c * a.hw];
+        m = fmaxf(m, v[c]);
+        if (c == y) xy = v[c];
+      }
+    }
+    float se = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        v[c] = expf(v[c] - m);
+        se += v[c];
+      }
+    }
+    const float inv_se = 1.f / se;
+    float sg = 0.f, r = 0.f, q = 0.f;
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        v[c] *= inv_se;                    // v now holds p
+        sg += v[c] * ((c == y ? A[c] : 0.f) + B[c]);
+        if (c == y) q = v[c];
+        else r += v[c];
+      }
+    }
+    const float wy = a.weight ? __ldg(a.weight + y) : 1.f;
+    // point term: d/dx_c = fp * (p_c - [c=y])
+    float fp;
+    if (a.mode == 0) {
+      fp = wy * inv_norm;
+    } else {
+      const float nll_lse = m + logf(se) - xy;
+      fp = -wy * pow_gamma(r, a.gamma) * (a.gamma * q * focal_logq_over_r(r, nll_lse) - 1.f) * inv_norm;
+    }
+#pragma unroll
+    for (int c = 0; c < kMaxClasses; ++c) {
+      if (c < k) {
+        const float g = (c == y ? A[c] : 0.f) + B[c];
+        const float dpoint = fp * (v[c] - (c == y ? 1.f : 0.f));
+        const float ddice = v[c] * (g - sg);
+        a.grad[base + c * a.hw] = wp * dpoint + wd * ddice;
+      }
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // Per-sample K x K confusion matrix: counts[n][label][argmax_c logits[n][c][pix]] += 1 over pixels whose label is in
 // [0, K) (ignore_index and out-of-range labels are skipped).  gridDim.y = samples; a warp adds equal bins once
 // (__match_any_sync), shared-memory histograms, one 64-bit atomic per non-empty bin and CTA.
@@ -497,6 +724,30 @@ int gap_seg_ce_loss(const float* logits, const int64_t* labels, int k, int n, in
   }
   GAP_CUDA(cudaGetLastError());
   ce_finish_kernel<<<1, 32, 0, st>>>(a);
+  CK_LAUNCH_OK();
+}
+
+int gap_seg_softmax_dice(const float* logits, const int64_t* labels, int k, int n, int64_t hw, int mode, float w_point,
+                         float gamma, float smooth, const float* class_weight, int64_t ignore_index, double* sums,
+                         int64_t* bad_labels, float* grad, float grad_scale, double* loss, void* stream) {
+  GAP_CHECK_ARG(k >= 2 && k <= kMaxClasses, "gap_seg_softmax_dice: k must be 2..16, got %d", k);
+  GAP_CHECK_ARG(logits && labels && sums && bad_labels && loss && n > 0 && hw > 0 && (mode == 0 || mode == 1),
+                "gap_seg_softmax_dice: bad arguments");
+  GAP_CHECK_ARG(smooth > 0.f && gamma >= 0.f && w_point >= 0.f && w_point <= 1.f,
+                "gap_seg_softmax_dice: need smooth > 0, gamma >= 0 and 0 <= w_point <= 1");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const long long npix = static_cast<long long>(n) * hw;
+  DiceArgs a{logits, reinterpret_cast<const long long*>(labels), class_weight, ignore_index, k, mode, hw, npix,
+             w_point, gamma, smooth, sums, reinterpret_cast<long long*>(bad_labels), grad, grad_scale, loss};
+  GAP_CUDA(cudaMemsetAsync(sums, 0, sizeof(double) * (3 * (k - 1) + 2), st));
+  const int gs = ck_grid(npix, 256, 148 * 4);
+  const int gg = grad ? ck_grid(npix, 256, 148 * 8) : 1;      // without a gradient only block 0 (the loss) runs
+  switch (k) {     // the common small class counts get fully unrolled plane loops
+    case 2: dice_stats_kernel<2><<<gs, 256, 0, st>>>(a); dice_grad_kernel<2><<<gg, 256, 0, st>>>(a); break;
+    case 3: dice_stats_kernel<3><<<gs, 256, 0, st>>>(a); dice_grad_kernel<3><<<gg, 256, 0, st>>>(a); break;
+    case 7: dice_stats_kernel<7><<<gs, 256, 0, st>>>(a); dice_grad_kernel<7><<<gg, 256, 0, st>>>(a); break;
+    default: dice_stats_kernel<0><<<gs, 256, 0, st>>>(a); dice_grad_kernel<0><<<gg, 256, 0, st>>>(a); break;
+  }
   CK_LAUNCH_OK();
 }
 

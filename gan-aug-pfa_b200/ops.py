@@ -932,6 +932,56 @@ def seg_ce_loss(logits: torch.Tensor, labels: torch.Tensor, class_weight: Option
                "gap_seg_ce_loss")
 
 
+DICE_SUMS = 3 * (MAX_CLASSES - 1) + 2      # fp64 workspace of seg_softmax_dice_loss for any K
+
+
+def check_dice_args(what: str, w_point, gamma, smooth) -> None:
+    """The keyword ranges of the softmax Dice losses (ValueError otherwise)."""
+    if not 0.0 <= float(w_point) <= 1.0:
+        raise ValueError(f"{what}: the point-term weight must be in [0, 1], got {w_point!r}")
+    if not float(gamma) >= 0.0:
+        raise ValueError(f"{what}: gamma must be >= 0, got {gamma!r}")
+    if not float(smooth) > 0.0:
+        raise ValueError(f"{what}: smooth must be > 0, got {smooth!r}")
+
+
+def seg_softmax_dice_loss(logits: torch.Tensor, labels: torch.Tensor, mode: int, w_point: float, gamma: float,
+                          smooth: float, class_weight: Optional[torch.Tensor], ignore_index: int, sums: torch.Tensor,
+                          bad_labels: torch.Tensor, grad: Optional[torch.Tensor], grad_scale: float,
+                          loss: torch.Tensor) -> None:
+    """w_point * Point + (1 - w_point) * Dice on fp32 class planes [n, K, h, w] (K = 2..16) against int64 labels
+    [n, h, w]; Dice = 1 - mean over classes 1..K-1 of (2 I_k + smooth) / (P_k + T_k + smooth) over the whole batch.
+    mode 0: Point = nn.CrossEntropyLoss(weight=class_weight, ignore_index); mode 1: Point = the softmax focal loss
+    mean a[y] (1 - p_y)^gamma (-log p_y), a = class_weight.  loss (fp64 [1]) is written, grad = grad_scale *
+    d(loss)/d(logits); sums is an fp64 workspace of >= 3(K-1)+2; bad_labels (int64 [1]) counts the labels outside
+    [0, K) that are not ignore_index (they contribute nothing)."""
+    what = "seg_softmax_dice_loss"
+    if mode not in (0, 1):
+        raise ValueError(f"{what}: mode must be 0 (cross-entropy) or 1 (focal), got {mode!r}")
+    check_dice_args(what, w_point, gamma, smooth)
+    if logits.dim() != 4:
+        raise ValueError(f"{what}: logits must be class planes [n, K, h, w], got {tuple(logits.shape)}")
+    n, k = logits.shape[0], logits.shape[1]
+    hw = logits.shape[2] * logits.shape[3]
+    if not 2 <= k <= MAX_CLASSES:
+        raise ValueError(f"{what}: the number of classes must be in 2..{MAX_CLASSES}, got {k}")
+    _planes(logits, n, k, hw, what, "logits")
+    _labels(labels, n, hw, what)
+    if grad is not None:
+        _planes(grad, n, k, hw, what, "grad")
+    if class_weight is not None and (class_weight.dtype != torch.float32 or not class_weight.is_contiguous()
+                                     or class_weight.numel() != k):
+        raise ValueError(f"{what}: class_weight must be contiguous fp32 [{k}]")
+    if sums.dtype != torch.float64 or sums.numel() < 3 * (k - 1) + 2 or loss.dtype != torch.float64 or loss.numel() < 1:
+        raise ValueError(f"{what}: sums must be fp64 [>= {3 * (k - 1) + 2}] and loss fp64 [1]")
+    if bad_labels.dtype != torch.int64 or bad_labels.numel() < 1:
+        raise ValueError(f"{what}: bad_labels must be int64 [1]")
+    _cuda(what, logits, labels, class_weight, sums, bad_labels, grad, loss)
+    _lib.check(_lib.lib().gap_seg_softmax_dice(_ptr(logits), _ptr(labels), k, n, hw, mode, w_point, gamma, smooth,
+                                               _ptr(class_weight), int(ignore_index), _ptr(sums), _ptr(bad_labels),
+                                               _ptr(grad), grad_scale, _ptr(loss), _stream()), "gap_seg_softmax_dice")
+
+
 def seg_confusion_ck(logits: torch.Tensor, labels: torch.Tensor, ignore_index: int, counts: torch.Tensor) -> None:
     """counts [n, K, K] (int64, accumulated) += per-sample confusion matrix: rows = label, columns = argmax over the
     K planes of logits [n, K, h, w]; labels equal to ignore_index or outside [0, K) are skipped."""

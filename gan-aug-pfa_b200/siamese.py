@@ -15,7 +15,8 @@ reference).  Single-channel maps (psi, logits) are fp32.
 Classes: n_classes = K = 1..16.  The logits and their gradient are fp32 class planes [n][K][h][w] (NCHW, what
 nn.CrossEntropyLoss and torch.argmax(dim=1) expect; for K = 1 the same memory as the [n][h][w] map, which keeps its
 shape).  K = 1 runs the single-channel conv_last kernels and the sigmoid losses; K > 1 runs the gap_conv1x1_ck_* head
-kernels and softmax cross-entropy (`kind="ce"`).
+kernels and softmax cross-entropy (`kind="ce"`), or softmax cross-entropy / focal loss with a multi-class Dice term
+(`kind="ce_dice"` / `"softmax_focal_dice"`, gap_seg_softmax_dice).
 """
 from __future__ import annotations
 
@@ -29,6 +30,10 @@ from .pix2pix import BN_EPS, BN_MOMENTUM, _BN, _Net, _on_device
 
 ENC = (("dconv_down1", 64), ("dconv_down2", 128), ("dconv_down3", 256), ("dconv_down4", 512), ("bottleneck", 1024))
 MAX_CLASSES = ops.MAX_CLASSES
+MULTI_KINDS = ("ce", "ce_dice", "softmax_focal_dice")       # loss kinds of n_classes > 1
+SINGLE_KINDS = ("combined", "focal_dice")                   # loss kinds of n_classes = 1
+DICE_KW = {"ce_dice": {"alpha": 0.5, "smooth": 1.0, "class_weight": None, "ignore_index": -100},
+           "softmax_focal_dice": {"beta": 0.5, "gamma": 2.0, "smooth": 1.0, "class_weight": None, "ignore_index": -100}}
 DEC = (("att3", "dconv_up3", 2048, 1024, 512), ("att2", "dconv_up2", 512, 512, 256), ("att1", "dconv_up1", 256, 256, 128),
        ("att_last", "dconv_last", 128, 128, 64))      # (gate, block, F_g, F_l, block out channels)
 
@@ -101,6 +106,7 @@ class SiameseEngine(_Net):
         # cross-entropy (n_classes > 1): fp64 workspace, and the count of labels outside [0, K) that are not
         # ignore_index (they contribute nothing to the loss; the count is never reset by the engine)
         self.ce_sums = torch.zeros(2, device=device, dtype=torch.float64)
+        self.dice_sums = torch.zeros(ops.DICE_SUMS, device=device, dtype=torch.float64)     # the Dice kinds' sums
         self.bad_labels = torch.zeros(1, device=device, dtype=torch.int64)
         self._cw_cache = (None, None)
 
@@ -477,17 +483,41 @@ class SiameseEngine(_Net):
             self._cw_cache = (key, torch.tensor(key, device=self.dev, dtype=torch.float32))
         return self._cw_cache[1]
 
+    def _check_kind(self, kind: str) -> None:
+        k = self.n_classes
+        if (kind in MULTI_KINDS and k == 1) or (kind in SINGLE_KINDS and k > 1):
+            raise ValueError(f"loss kind {kind!r} does not apply to n_classes = {k}: use kind='ce' with n_classes > 1 "
+                             "(or 'ce_dice', 'softmax_focal_dice') and 'combined' or 'focal_dice' with n_classes = 1")
+
+    def _dice_args(self, kind: str, kw: dict) -> dict:
+        """The keywords of a Dice kind with their defaults, checked (ValueError) before any launch."""
+        unknown = set(kw) - set(DICE_KW[kind])
+        if unknown:
+            raise ValueError(f"kind={kind!r} takes {', '.join(DICE_KW[kind])}, not {sorted(unknown)}")
+        args = dict(DICE_KW[kind], **kw)
+        w_point = args["alpha"] if kind == "ce_dice" else args["beta"]
+        ops.check_dice_args(f"kind={kind!r}", w_point, args.get("gamma", 0.0), args["smooth"])
+        cw = self._class_weight(args["class_weight"])
+        if cw is not None and cw.numel() != self.n_classes:
+            raise ValueError(f"class_weight has {cw.numel()} entries; n_classes = {self.n_classes}")
+        return dict(mode=0 if kind == "ce_dice" else 1, w_point=float(w_point), gamma=float(args.get("gamma", 0.0)),
+                    smooth=float(args["smooth"]), class_weight=cw, ignore_index=int(args["ignore_index"]))
+
     def loss_and_grad(self, labels: torch.Tensor, kind: Optional[str] = None, **kw) -> torch.Tensor:
         """The loss on self.logits; writes d(loss)/d(logits) into self.dlogits and returns the loss as a device fp64
         scalar tensor.  n_classes = 1: kind "combined" (CombinedLoss, train.py:82-105; the default) or "focal_dice"
         (FocalDiceLoss, train.py:108-128).  n_classes > 1: kind "ce" (the default), nn.CrossEntropyLoss(
-        weight=class_weight, ignore_index=ignore_index) with class_weight a length-K sequence or device tensor."""
+        weight=class_weight, ignore_index=ignore_index) with class_weight a length-K sequence or device tensor;
+        kind "ce_dice" (alpha * CE + (1 - alpha) * Dice; alpha=0.5, smooth=1.0, class_weight, ignore_index) or
+        "softmax_focal_dice" (beta * Focal + (1 - beta) * Dice; beta=0.5, gamma=2.0, smooth=1.0, class_weight as the
+        focal per-class factor, ignore_index), the K-class forms of CombinedLoss and FocalDiceLoss.  Their Dice term is
+        1 - the mean over classes 1..K-1 (class 0, "no change", is excluded) of (2 I_k + smooth) / (P_k + T_k + smooth),
+        summed over this batch.  Data parallel: each rank's Dice uses its own batch (as the binary "combined" and
+        "focal_dice" do) and the gradients are averaged by the reducer; there is no cross-rank Dice."""
         k = self.n_classes
         if kind is None:
             kind = "combined" if k == 1 else "ce"
-        if (kind == "ce") != (k > 1) and kind in ("ce", "combined", "focal_dice"):
-            raise ValueError(f"loss kind {kind!r} does not apply to n_classes = {k}: use kind='ce' with n_classes > 1 "
-                             "and 'combined' or 'focal_dice' with n_classes = 1")
+        self._check_kind(kind)
         if kind == "ce":
             unknown = set(kw) - {"class_weight", "ignore_index"}
             if unknown:
@@ -497,6 +527,11 @@ class SiameseEngine(_Net):
                 raise ValueError(f"class_weight has {cw.numel()} entries; n_classes = {k}")
             ops.seg_ce_loss(self.logits, labels.contiguous(), cw, int(kw.get("ignore_index", -100)), self.ce_sums,
                             self.bad_labels, self.dlogits, 1.0, self.loss_out)
+        elif kind in DICE_KW:
+            a = self._dice_args(kind, kw)
+            ops.seg_softmax_dice_loss(self.logits, labels.contiguous(), a["mode"], a["w_point"], a["gamma"], a["smooth"],
+                                      a["class_weight"], a["ignore_index"], self.dice_sums, self.bad_labels, self.dlogits,
+                                      1.0, self.loss_out)
         elif kind == "combined":
             alpha = kw.get("alpha", 0.5)
             ops.seg_loss(self.logits, labels, 0, alpha, 1.0 - alpha, kw.get("pos_weight", 9.0), kw.get("smooth", 1.0), 0.0,
@@ -518,8 +553,9 @@ class SiameseEngine(_Net):
         loss_and_grad ("combined" for n_classes = 1, "ce" for n_classes > 1 by default)."""
         if kind is None:
             kind = "combined" if self.n_classes == 1 else "ce"
-        if (kind == "ce") != (self.n_classes > 1) and kind in ("ce", "combined", "focal_dice"):
-            self.loss_and_grad(None, kind)          # raises the pairing error before any work is enqueued
+        self._check_kind(kind)                  # the pairing error before any work is enqueued
+        if kind in DICE_KW:
+            self._dice_args(kind, loss_kw)      # and the keyword errors of the Dice kinds
         self.training = True
         self.zero_grad()
         self.forward(img1, img2)

@@ -356,6 +356,18 @@ int gap_conv1x1_ck_wgrad(const float* dl, const void* x, int64_t ldx, int k, int
 int gap_seg_ce_loss(const float* logits, const int64_t* labels, int k, int n, int64_t hw, const float* class_weight,
                     int64_t ignore_index, double* sums2, int64_t* bad_labels, float* grad, float grad_scale,
                     double* loss, void* stream);
+/* Softmax point term + multi-class Dice over the K = 2..16 planes against int64 labels [n][hw], p = softmax(logits):
+ *   loss[0] = w_point * Point + (1 - w_point) * Dice,  Dice = 1 - 1/(K-1) sum_{k=1..K-1} (2 I_k + s) / (P_k + T_k + s)
+ * with I_k = sum p_k [y=k], P_k = sum p_k, T_k = sum [y=k] over the counted pixels of the whole batch (y != ignore_index,
+ * 0 <= y < K; class 0 is not a Dice class) and s = smooth > 0.
+ *   mode 0: Point = nn.CrossEntropyLoss(weight=class_weight, ignore_index) (weighted mean, normalised by sum w[y])
+ *   mode 1: Point = sum a[y] (1 - p_y)^gamma (-log p_y) / (counted pixels), a = class_weight (NULL: all 1), gamma >= 0
+ * grad (may be NULL) = grad_scale * d(loss)/d(logits), zero at pixels that are not counted.  An all-ignored batch gives a
+ * NaN loss and a zero gradient.  A label outside [0, K) that is not ignore_index adds 1 to *bad_labels (never zeroed
+ * here).  sums is a fp64 workspace of 3(K-1)+2 doubles.  0 <= w_point <= 1.  No host synchronisation. */
+int gap_seg_softmax_dice(const float* logits, const int64_t* labels, int k, int n, int64_t hw, int mode, float w_point,
+                         float gamma, float smooth, const float* class_weight, int64_t ignore_index, double* sums,
+                         int64_t* bad_labels, float* grad, float grad_scale, double* loss, void* stream);
 /* Per-sample K x K confusion matrix: counts[n][label][argmax_c logits] += 1 (int64, accumulated: the caller zeroes it
  * once); pixels whose label is ignore_index or outside [0, K) are skipped.  n < 65536. */
 int gap_seg_confusion_ck(const float* logits, const int64_t* labels, int k, int n, int64_t hw, int64_t ignore_index,
