@@ -135,6 +135,9 @@ _SIGNATURES = {
     "gap_seg_ce_loss": (C.c_int, [_P, _P, _I, _I, _L, _P, _L, _P, _P, _P, _F, _P, _P]),
     "gap_seg_softmax_dice": (C.c_int, [_P, _P, _I, _I, _L, _I, _F, _F, _F, _P, _L, _P, _P, _P, _F, _P, _P]),
     "gap_seg_confusion_ck": (C.c_int, [_P, _P, _I, _I, _L, _L, _P, _P]),
+    "gap_scene_gather": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "gap_scene_blend": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "gap_scene_finalize": (C.c_int, [_P, _P, _I, _L, _P, _I, _P, _L, _P, _P]),
     "gap_bn_finalize": (C.c_int, [_P, _I, _D, _P, _P, _F, _F, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gap_bn_eval_scale_shift": (C.c_int, [_I, _P, _P, _P, _P, _F, _P, _P, _P]),
     "gap_bn_act": (C.c_int, [_P, _L, _P, _P, _L, _I, _P, _L, _I, _P, _L, _I, _P]),

@@ -557,3 +557,10 @@ class SiameseUNet(_NativeModule):
 
     def forward(self, x1, x2):
         return _SiameseFn.apply(self, x1, x2, *self.parameters())
+
+    def predict_scene(self, img1, img2, tile=256, overlap=64, batch=8, return_probs=False, labels=None,
+                      ignore_index=-100):
+        """Sliding-window change map of a whole scene at its own resolution (SiameseEngine.predict_scene): always in
+        eval mode, whatever mode the module is in; no autograd.  Returns a siamese.SceneResult(pred, probs, confusion)."""
+        return self._engine().predict_scene(img1, img2, tile=tile, overlap=overlap, batch=batch,
+                                            return_probs=return_probs, labels=labels, ignore_index=ignore_index)

@@ -998,3 +998,102 @@ def seg_confusion_ck(logits: torch.Tensor, labels: torch.Tensor, ignore_index: i
     _cuda(what, logits, labels, counts)
     _lib.check(_lib.lib().gap_seg_confusion_ck(_ptr(logits), _ptr(labels), k, n, hw, int(ignore_index), _ptr(counts),
                                                _stream()), "gap_seg_confusion_ck")
+
+
+# ------------------------------------------------------------------------------------------------
+# Sliding-window scene inference (gap_b200.h "Sliding-window inference"): a tile grid is (ay, ax), each axis the tuple
+# (len, ext, step, n) of siamese.scene_axis
+# ------------------------------------------------------------------------------------------------
+def _scene_grid_args(grid, what: str) -> tuple:
+    (h, ey, sy, ny), (w, ex, sx, nx) = grid
+    if ey % 16 or ex % 16 or min(h, w, ey, ex, sy, sx, ny, nx) < 1:
+        raise ValueError(f"{what}: bad tile grid {grid!r}")
+    return h, w, ey, ex, sy, sx, ny, nx
+
+
+def _scene_input(x: torch.Tensor, c: int, h: int, w: int, what: str, name: str) -> bool:
+    """True for a uint8 [h, w, c] scene, False for an fp32 [c, h, w] one (ValueError otherwise)."""
+    if x.dtype == torch.uint8 and tuple(x.shape) == (h, w, c) and x.is_contiguous():
+        return True
+    if x.dtype == torch.float32 and tuple(x.shape) == (c, h, w) and x.is_contiguous():
+        return False
+    raise ValueError(f"{what}: {name} must be a contiguous uint8 [{h}, {w}, {c}] or fp32 [{c}, {h}, {w}] scene, got "
+                     f"{x.dtype} {tuple(x.shape)}")
+
+
+def scene_gather(img1: torch.Tensor, img2: torch.Tensor, grid, tile0: int, out1: torch.Tensor, out2: torch.Tensor) -> None:
+    """Tiles tile0 .. tile0 + batch - 1 of both scenes (uint8 [H, W, C] normalised as dataset.py does, or fp32 [C, H, W]
+    rounded to bf16) -> out1 / out2, dense NHWC bf16 [batch, E_y, E_x, 4]; slots >= C and tiles past the grid are zero."""
+    what = "scene_gather"
+    h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    c = img1.shape[-1] if img1.dtype == torch.uint8 else img1.shape[0]
+    if not 1 <= c <= 4:
+        raise ValueError(f"{what}: scenes of 1 to 4 channels are supported, got {c}")
+    u8 = _scene_input(img1, c, h, w, what, "img1")
+    if _scene_input(img2, c, h, w, what, "img2") != u8:
+        raise ValueError(f"{what}: img1 and img2 must have the same dtype")
+    batch = out1.shape[0]
+    for name, o in (("out1", out1), ("out2", out2)):
+        if o.dtype != torch.bfloat16 or tuple(o.shape) != (batch, ey, ex, 4) or not o.is_contiguous():
+            raise ValueError(f"{what}: {name} must be a contiguous bf16 [batch, {ey}, {ex}, 4] tensor, got "
+                             f"{o.dtype} {tuple(o.shape)}")
+        if o.data_ptr() % 8:
+            raise ValueError(f"{what}: {name} must be 8-byte aligned (each 4-slot pixel is one 8-byte store)")
+    if not 0 <= tile0 < ny * nx:
+        raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
+    _cuda(what, img1, img2, out1, out2)
+    _lib.check(_lib.lib().gap_scene_gather(_ptr(img1), _ptr(img2), int(u8), c, h, w, ey, ex, sy, sx, ny, nx, int(tile0),
+                                           batch, _ptr(out1), _ptr(out2), _stream()), "gap_scene_gather")
+
+
+def scene_blend(logits: torch.Tensor, grid, tile0: int, acc: torch.Tensor, wsum: torch.Tensor) -> None:
+    """Window-weighted probabilities of one batch of tile logits (fp32 [batch, E_y, E_x] for K = 1, [batch, K, E_y, E_x]
+    for K > 1) -> acc [K, H, W] += w * p, wsum [H, W] += w (fp32) at every scene pixel the batch covers."""
+    what = "scene_blend"
+    h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    k = 1 if logits.dim() == 3 else (logits.shape[1] if logits.dim() == 4 else -1)
+    _check_k(k, what)
+    batch = logits.shape[0]
+    if logits.dtype != torch.float32 or not logits.is_contiguous() or tuple(logits.shape[-2:]) != (ey, ex):
+        raise ValueError(f"{what}: logits must be contiguous fp32 [batch, (K,) {ey}, {ex}], got {logits.dtype} "
+                         f"{tuple(logits.shape)}")
+    if acc.dtype != torch.float32 or tuple(acc.shape) != (k, h, w) or not acc.is_contiguous():
+        raise ValueError(f"{what}: acc must be a contiguous fp32 [{k}, {h}, {w}] tensor")
+    if wsum.dtype != torch.float32 or tuple(wsum.shape) != (h, w) or not wsum.is_contiguous():
+        raise ValueError(f"{what}: wsum must be a contiguous fp32 [{h}, {w}] tensor")
+    if not 0 <= tile0 < ny * nx:
+        raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
+    _cuda(what, logits, acc, wsum)
+    _lib.check(_lib.lib().gap_scene_blend(_ptr(logits), k, h, w, ey, ex, sy, sx, ny, nx, int(tile0), batch, _ptr(acc),
+                                          _ptr(wsum), _stream()), "gap_scene_blend")
+
+
+def scene_finalize(acc: torch.Tensor, wsum: torch.Tensor, pred: torch.Tensor, write_probs: bool,
+                   labels: Optional[torch.Tensor] = None, ignore_index: int = -100,
+                   counts: Optional[torch.Tensor] = None) -> None:
+    """pred (uint8 [H, W]) = argmax of acc / wsum over K (K = 1: > 0.5); write_probs: acc becomes the probabilities in
+    place.  With labels (int64 [H, W]) counts (int64, accumulated) += the [K, K] confusion matrix (K = 1: [TP, FP, FN,
+    TN]) over pixels whose label is not ignore_index and lies in [0, K) ({0, 1} for K = 1)."""
+    what = "scene_finalize"
+    if acc.dim() != 3:
+        raise ValueError(f"{what}: acc must be fp32 [K, H, W], got {tuple(acc.shape)}")
+    k, h, w = acc.shape
+    _check_k(k, what)
+    if acc.dtype != torch.float32 or not acc.is_contiguous():
+        raise ValueError(f"{what}: acc must be a contiguous fp32 [K, H, W] tensor")
+    if wsum.dtype != torch.float32 or tuple(wsum.shape) != (h, w) or not wsum.is_contiguous():
+        raise ValueError(f"{what}: wsum must be a contiguous fp32 [{h}, {w}] tensor")
+    if pred.dtype != torch.uint8 or tuple(pred.shape) != (h, w) or not pred.is_contiguous():
+        raise ValueError(f"{what}: pred must be a contiguous uint8 [{h}, {w}] tensor")
+    if (labels is None) != (counts is None):
+        raise ValueError(f"{what}: labels and counts go together")
+    if labels is not None:
+        if labels.dtype != torch.int64 or tuple(labels.shape) != (h, w) or not labels.is_contiguous():
+            raise ValueError(f"{what}: labels must be a contiguous int64 [{h}, {w}] tensor")
+        shape = (4,) if k == 1 else (k, k)
+        if counts.dtype != torch.int64 or tuple(counts.shape) != shape or not counts.is_contiguous():
+            raise ValueError(f"{what}: counts must be a contiguous int64 {list(shape)} tensor")
+    _cuda(what, acc, wsum, pred, labels, counts)
+    _lib.check(_lib.lib().gap_scene_finalize(_ptr(acc), _ptr(wsum), k, h * w, _ptr(pred), int(bool(write_probs)),
+                                             _ptr(labels), int(ignore_index), _ptr(counts), _stream()),
+               "gap_scene_finalize")

@@ -20,7 +20,7 @@ kernels and softmax cross-entropy (`kind="ce"`), or softmax cross-entropy / foca
 """
 from __future__ import annotations
 
-from typing import Callable, Dict, List, Optional, Tuple
+from typing import Callable, Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 
@@ -43,6 +43,45 @@ def check_n_classes(n_classes) -> None:
     if isinstance(n_classes, bool) or not isinstance(n_classes, int) or not 1 <= n_classes <= MAX_CLASSES:
         raise NotImplementedError(f"n_classes = {n_classes!r} is not implemented natively: 1 to {MAX_CLASSES} classes "
                                   "are")
+
+
+def scene_axis(length: int, tile: int, overlap: int) -> Tuple[List[int], int]:
+    """The tile origins along one scene axis of `length` pixels and the tile extent E (predict_scene's grid; csrc/scene.cu
+    derives the same origins on the device).  length <= tile: one tile at 0 with E = ceil16(length), whose reads past
+    the scene clamp to its last row / column.  Otherwise E = tile, step S = tile - overlap and
+    n = ceil((length - tile) / S) + 1 tiles at min(i*S, length - tile): the last one is snapped to the edge."""
+    if length <= tile:
+        return [0], -(-length // 16) * 16
+    step = tile - overlap
+    n = -(-(length - tile) // step) + 1
+    return [min(i * step, length - tile) for i in range(n)], tile
+
+
+def scene_window(extent: int) -> torch.Tensor:
+    """The 1-D blending window of a tile axis, fp64 [extent]: g(t) = exp(-(t + 0.5 - E/2)^2 / (2 sigma^2)), sigma = E/8
+    (nnU-Net's choice); a tile's weight is g_y(ty) * g_x(tx).  Its smallest value is about exp(-8), so every covered
+    pixel has a positive weight sum, and with overlap 0 it cancels (plain stitching)."""
+    t = torch.arange(extent, dtype=torch.float64)
+    sigma = extent / 8
+    return torch.exp(-(t + 0.5 - extent / 2) ** 2 / (2 * sigma ** 2))
+
+
+def _scene_grid(h: int, w: int, tile: int, overlap: int):
+    """((len, ext, step, n) of the y axis, same of the x axis): the grid in the form the scene kernels take."""
+    out = []
+    for length in (h, w):
+        origins, ext = scene_axis(length, tile, overlap)
+        out.append((length, ext, tile - overlap if len(origins) > 1 else ext, len(origins)))
+    return tuple(out)
+
+
+class SceneResult(NamedTuple):
+    """predict_scene's result; fields that were not asked for are None.
+    pred: uint8 [H, W] class map (K = 1: 0/1).  probs: fp32 [K, H, W] blended probabilities (K = 1: the sigmoid).
+    confusion: int64 [K, K] (rows = label, columns = prediction) or, K = 1, [TP, FP, FN, TN]."""
+    pred: torch.Tensor
+    probs: Optional[torch.Tensor]
+    confusion: Optional[torch.Tensor]
 
 
 def _k(name: str, leaf: str) -> str:
@@ -356,13 +395,15 @@ class SiameseEngine(_Net):
         self._tape.append(backward)
 
     # -- forward ---------------------------------------------------------------------------------------
-    def _encode(self, p: int, x: torch.Tensor) -> None:
+    def _encode(self, p: int, x: Optional[torch.Tensor]) -> None:
         """forward_encoder (models.py:92-102) for branch p: 4 x (double_conv + MaxPool2d(2)) + bottleneck; the features
-        land in the channel slots p of the concatenated skip buffers S[0..4]."""
-        n = x.shape[0]
-        if x.shape[1] != self.n_channels:
-            raise ValueError(f"input has {x.shape[1]} channels, expected n_channels = {self.n_channels}")
-        ops.nchw_to_nhwc_bf16(x.contiguous().float(), self.x_in[p])
+        land in the channel slots p of the concatenated skip buffers S[0..4].  x: the fp32 NCHW input, or None when
+        x_in[p] already holds it (staged by the scene gather)."""
+        n = self.x_in[p].shape[0]
+        if x is not None:
+            if x.shape[1] != self.n_channels:
+                raise ValueError(f"input has {x.shape[1]} channels, expected n_channels = {self.n_channels}")
+            ops.nchw_to_nhwc_bf16(x.contiguous().float(), self.x_in[p])
         ops.im2col_k3s1p1(self.x_in[p], self.col[p], self.n_channels)
         src, gsrc = self.col[p], None
         for lvl, (name, c) in enumerate(ENC):
@@ -404,9 +445,14 @@ class SiameseEngine(_Net):
         [n, K, h, w] (n_classes = K > 1); pred (uint8 [n, h, w], K > 1 only) receives the argmax class map."""
         n, _, h, w = x1.shape
         self._alloc(n, h, w)
+        return self._forward_from((x1, x2), pred)
+
+    def _forward_from(self, xs, pred: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """forward() from the inputs on: xs = (x1, x2) fp32 NCHW, converted into x_in as each encoder pass starts, or
+        (None, None) when x_in already holds the batch (the staged path of predict_scene)."""
         self._tape = []
         self._marks = {}
-        for p, x in enumerate((x1, x2)):
+        for p, x in enumerate(xs):
             self._encode(p, x)
         prev, gprev = self.S[4], self.gS[4]          # bottleneck pair (2048 channels)
         self._marks[len(self._tape)] = self.store.off(DEC[0][0] + ".W_g.0.weight")   # gates, decoder blocks, conv_last
@@ -450,6 +496,97 @@ class SiameseEngine(_Net):
             self.training = was
             self._tape = []
         return out_u8
+
+    def _scene_input(self, x, name: str):
+        """(is_uint8, h, w) of a predict_scene input, ValueError unless it is uint8 [H, W, C] (host or device) or fp32
+        [C, H, W] on the engine's device, with C = n_channels."""
+        if not isinstance(x, torch.Tensor) or x.dim() != 3:
+            raise ValueError(f"{name} must be a uint8 [H, W, C] or fp32 [C, H, W] tensor, got "
+                             f"{getattr(x, 'shape', type(x))}")
+        if x.dtype == torch.uint8:
+            h, w, c = x.shape
+        elif x.dtype == torch.float32:
+            c, h, w = x.shape
+            if x.device.type != self.dev.type or (self.dev.index is not None and x.device.index != self.dev.index):
+                raise ValueError(f"{name}: an fp32 [C, H, W] scene must be on the engine's device {self.dev}, got "
+                                 f"{x.device}")
+        else:
+            raise ValueError(f"{name} must be uint8 [H, W, C] or fp32 [C, H, W], got {x.dtype}")
+        if c != self.n_channels:
+            raise ValueError(f"{name} has {c} channels, expected n_channels = {self.n_channels}")
+        if h < 1 or w < 1:
+            raise ValueError(f"{name} is empty: {tuple(x.shape)}")
+        return x.dtype == torch.uint8, h, w
+
+    @_on_device
+    def predict_scene(self, img1: torch.Tensor, img2: torch.Tensor, tile: int = 256, overlap: int = 64, batch: int = 8,
+                      return_probs: bool = False, labels: Optional[torch.Tensor] = None,
+                      ignore_index: int = -100) -> SceneResult:
+        """A change map of a whole scene of any size at its own resolution, by sliding-window inference.
+
+        img1, img2: the two images of the scene, either uint8 [H, W, C] as PIL / numpy give them (host or device;
+        normalised on the device as dataset.py's ToTensor + Normalize(0.5, 0.5); a host scene is copied to the device
+        once) or fp32 [C, H, W] on the device, already normalised (what forward() takes).  C = n_channels, the same
+        shape for both, any H, W >= 1.
+
+        The scene is cut into tiles of tile x tile pixels that overlap by `overlap` (scene_axis: an axis shorter than
+        the tile gets one tile of its own length rounded up to 16, padded by repeating the edge), and the tiles run
+        `batch` at a time through the eval-mode network (BatchNorm with the running statistics, as predict()).  Their
+        softmax (K = 1: sigmoid) probabilities are blended with the Gaussian window of scene_window:
+        p = sum_tiles w * p_tile / sum_tiles w, summed in ascending tile index, so the result does not depend on
+        `batch`.  pred is the argmax of p (ties to the lowest class) or, for K = 1, p > 0.5.
+
+        return_probs: also return p (fp32 [K, H, W]).  labels (int64 [H, W]): also return the confusion counts of pred
+        against them at full resolution: [K, K] (rows = label; metrics.multiclass_metrics takes it) or, for K = 1,
+        [TP, FP, FN, TN] (metrics.metrics_from_counts); pixels labelled ignore_index or outside [0, K) ({0, 1} for
+        K = 1) are not counted.
+
+        Memory: (K + 1) * 4 bytes per scene pixel of accumulators (which become probs), and the engine's activation
+        buffers sized for `batch` tiles; like any call at a new shape this may re-allocate them.  Everything runs on
+        the current stream without a host synchronisation.  The `training` flag is restored afterwards and no
+        parameter, gradient or BatchNorm buffer changes.  Bad arguments raise ValueError before any work is enqueued."""
+        for name, v in (("tile", tile), ("overlap", overlap), ("batch", batch)):
+            if isinstance(v, bool) or not isinstance(v, int):
+                raise ValueError(f"{name} must be an int, got {v!r}")
+        if tile < 16 or tile % 16:
+            raise ValueError(f"tile must be a multiple of 16 and at least 16, got {tile}")
+        if not 0 <= overlap < tile:
+            raise ValueError(f"overlap must be in [0, tile = {tile}), got {overlap}")
+        if batch < 1:
+            raise ValueError(f"batch must be >= 1, got {batch}")
+        u8, h, w = self._scene_input(img1, "img1")
+        if self._scene_input(img2, "img2")[0] != u8 or img2.shape != img1.shape:
+            raise ValueError(f"img1 and img2 must have the same dtype and shape, got {img1.dtype} "
+                             f"{tuple(img1.shape)} and {img2.dtype} {tuple(img2.shape)}")
+        if labels is not None and (not isinstance(labels, torch.Tensor) or labels.dtype != torch.int64
+                                   or tuple(labels.shape) != (h, w)):
+            raise ValueError(f"labels must be an int64 [{h}, {w}] tensor, got "
+                             f"{getattr(labels, 'dtype', type(labels))} {tuple(getattr(labels, 'shape', ()))}")
+        k = self.n_classes
+        grid = _scene_grid(h, w, tile, overlap)
+        (_, ey, _, ny), (_, ex, _, nx) = grid
+        img1, img2 = img1.to(self.dev).contiguous(), img2.to(self.dev).contiguous()
+        if labels is not None:
+            labels = labels.to(self.dev).contiguous()
+        acc = torch.empty(k, h, w, device=self.dev)              # every pixel is written by the batch of its first tile
+        wsum = torch.empty(h, w, device=self.dev)
+        pred = torch.empty(h, w, device=self.dev, dtype=torch.uint8)
+        conf = None
+        if labels is not None:
+            conf = torch.zeros((4,) if k == 1 else (k, k), device=self.dev, dtype=torch.int64)
+        was = self.training
+        self.training = False
+        try:
+            self._alloc(batch, ey, ex)
+            for t0 in range(0, ny * nx, batch):                 # the last batch is padded with zero tiles
+                ops.scene_gather(img1, img2, grid, t0, self.x_in[0], self.x_in[1])
+                self._forward_from((None, None))
+                ops.scene_blend(self.logits, grid, t0, acc, wsum)
+            ops.scene_finalize(acc, wsum, pred, return_probs, labels, ignore_index, conf)
+        finally:
+            self.training = was
+            self._tape = []
+        return SceneResult(pred, acc if return_probs else None, conf)
 
     # -- backward --------------------------------------------------------------------------------------
     @_on_device

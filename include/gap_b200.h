@@ -373,6 +373,30 @@ int gap_seg_softmax_dice(const float* logits, const int64_t* labels, int k, int 
 int gap_seg_confusion_ck(const float* logits, const int64_t* labels, int k, int n, int64_t hw, int64_t ignore_index,
                          int64_t* counts, void* stream);
 
+/* Sliding-window inference over a whole scene (scene.cu, SiameseEngine.predict_scene).  Each axis of the tile grid is
+ * (len, ext, step, n): the scene length, the tile extent (a multiple of 16), the step between tile origins and the tile
+ * count; tile i of an axis starts at n == 1 ? 0 : min(i*step, len - ext) (n == 1 needs len <= ext and reads past len
+ * clamp to the last row / column; n > 1 needs len > ext).  Tiles are numbered row-major, t = ty*nx + tx.  Blending
+ * window w = g(ty) g(tx), g(t) = exp(-(t + 0.5 - ext/2)^2 / (2 (ext/8)^2)).
+ * gather: tiles tile0 .. tile0+batch-1 of both scenes -> NHWC bf16 [batch][ey][ex][4 slots] (out1 / out2, dense);
+ *   src_u8: uint8 HWC [h][w][c] normalised as gap_u8_hwc_to_nhwc_bf16_c, else fp32 CHW [c][h][w] rounded as
+ *   gap_nchw_f32_to_nhwc_bf16; slots >= c and tiles >= ny*nx (padding of the last batch) are written as zero.
+ *   out1 / out2 must be 8-byte aligned: each 4-slot pixel is one 8-byte store. */
+int gap_scene_gather(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy, int sx,
+                     int ny, int nx, int tile0, int batch, void* out1, void* out2, void* stream);
+/* blend: logits fp32 [batch][k][ey][ex] (k = 1: sigmoid, else softmax over the k planes) of tiles tile0 .. -> for every
+ * scene pixel, over the covering tiles of this batch in ascending index: acc[c][pixel] += w * p_c, wsum[pixel] += w
+ * (fp32 [k][h][w] and [h][w]).  A pixel whose first covering tile of the grid is in this batch starts from zero, so the
+ * accumulators need no clearing when the batches run in order.  No floating-point atomics: deterministic. */
+int gap_scene_blend(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx, int tile0,
+                    int batch, float* acc, float* wsum, void* stream);
+/* finalize: p = acc / wsum over `pixels`; pred (uint8) = argmax_c p (ties to the lowest class) or, k = 1, p > 0.5;
+ * write_probs: acc is overwritten with p.  labels (int64, optional, with counts): counts += k > 1 ? [label][pred] (k*k)
+ * : [TP, FP, FN, TN] (label 1 positive, 0 negative); ignore_index and labels outside [0, k) ({0, 1} for k = 1) are not
+ * counted.  The caller zeroes counts. */
+int gap_scene_finalize(float* acc, const float* wsum, int k, int64_t pixels, uint8_t* pred, int write_probs,
+                       const int64_t* labels, int64_t ignore_index, int64_t* counts, void* stream);
+
 /* evaluate.py:34-64 calculate_metrics, device side: per-sample counts[n][4] += [TP, FP, FN, TN] of
  * (sigmoid(logits) > 0.5) against {0,1} labels (int64 when labels_are_i64, else fp32); logits are [n][hw] fp32.
  * The caller zeroes counts once and may accumulate several batches; the ratios are formed on the host. */
