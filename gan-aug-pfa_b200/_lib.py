@@ -138,6 +138,9 @@ _SIGNATURES = {
     "gap_scene_gather": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "gap_scene_blend": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "gap_scene_finalize": (C.c_int, [_P, _P, _I, _L, _P, _I, _P, _L, _P, _P]),
+    "gap_scene_gather_one": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
+    "gap_scene_blend_image": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "gap_scene_finalize_image": (C.c_int, [_P, _P, _I, _L, _P, _I, _P]),
     "gap_bn_finalize": (C.c_int, [_P, _I, _D, _P, _P, _F, _F, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "gap_bn_eval_scale_shift": (C.c_int, [_I, _P, _P, _P, _P, _F, _P, _P, _P]),
     "gap_bn_act": (C.c_int, [_P, _L, _P, _P, _L, _I, _P, _L, _I, _P, _L, _I, _P]),

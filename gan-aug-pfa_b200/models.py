@@ -304,6 +304,11 @@ class UNetGenerator(_NativeModule):
     def forward(self, input):
         return _GeneratorFn.apply(self, input, torch.is_grad_enabled(), *self.parameters())
 
+    def translate_scene(self, img, tile=256, overlap=64, batch=32, return_float=False):
+        """Sliding-window image of a whole scene at its own resolution (GeneratorEngine.translate_scene): always in eval
+        mode, whatever mode the module is in; no autograd.  Returns a pix2pix.SceneImage(image, values)."""
+        return self._engine().translate_scene(img, tile=tile, overlap=overlap, batch=batch, return_float=return_float)
+
 
 class _DiscriminatorFn(torch.autograd.Function):
     """The input cat(A, B) is split by discriminator_split: A = the first ceil(input_nc / 2) channels, B = the rest."""

@@ -1002,7 +1002,7 @@ def seg_confusion_ck(logits: torch.Tensor, labels: torch.Tensor, ignore_index: i
 
 # ------------------------------------------------------------------------------------------------
 # Sliding-window scene inference (gap_b200.h "Sliding-window inference"): a tile grid is (ay, ax), each axis the tuple
-# (len, ext, step, n) of siamese.scene_axis
+# (len, ext, step, n) of scene._scene_grid
 # ------------------------------------------------------------------------------------------------
 def _scene_grid_args(grid, what: str) -> tuple:
     (h, ey, sy, ny), (w, ex, sx, nx) = grid
@@ -1097,3 +1097,74 @@ def scene_finalize(acc: torch.Tensor, wsum: torch.Tensor, pred: torch.Tensor, wr
     _lib.check(_lib.lib().gap_scene_finalize(_ptr(acc), _ptr(wsum), k, h * w, _ptr(pred), int(bool(write_probs)),
                                              _ptr(labels), int(ignore_index), _ptr(counts), _stream()),
                "gap_scene_finalize")
+
+
+def scene_gather_one(img: torch.Tensor, grid, tile0: int, out: torch.Tensor) -> None:
+    """Tiles tile0 .. tile0 + batch - 1 of one scene (uint8 [H, W, C] normalised as dataset.py does, or fp32 [C, H, W]
+    rounded to bf16) -> out, dense NHWC bf16 [batch, E_y, E_x, 4] (the generator's input batch); slots >= C and tiles
+    past the grid are zero."""
+    what = "scene_gather_one"
+    h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    c = (img.shape[-1] if img.dtype == torch.uint8 else img.shape[0]) if img.dim() == 3 else 0
+    if not 1 <= c <= 4:
+        raise ValueError(f"{what}: scenes of 1 to 4 channels are supported, got {img.dtype} {tuple(img.shape)}")
+    u8 = _scene_input(img, c, h, w, what, "img")
+    batch = out.shape[0]
+    if out.dtype != torch.bfloat16 or tuple(out.shape) != (batch, ey, ex, 4) or not out.is_contiguous():
+        raise ValueError(f"{what}: out must be a contiguous bf16 [batch, {ey}, {ex}, 4] tensor, got {out.dtype} "
+                         f"{tuple(out.shape)}")
+    if out.data_ptr() % 8:
+        raise ValueError(f"{what}: out must be 8-byte aligned (each 4-slot pixel is one 8-byte store)")
+    if not 0 <= tile0 < ny * nx:
+        raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
+    _cuda(what, img, out)
+    _lib.check(_lib.lib().gap_scene_gather_one(_ptr(img), int(u8), c, h, w, ey, ex, sy, sx, ny, nx, int(tile0), batch,
+                                               _ptr(out), _stream()), "gap_scene_gather_one")
+
+
+SCENE_MAX_WINDOW = 12288        # ey + ex of gap_scene_blend_image: its window table lives in shared memory
+
+
+def scene_blend_image(fake: torch.Tensor, grid, tile0: int, acc: torch.Tensor, wsum: torch.Tensor) -> None:
+    """Window-weighted generator outputs of one batch of tiles (fp32 [batch, E_y, E_x, 4], channels >= C unused) ->
+    acc [C, H, W] += w * v, wsum [H, W] += w (fp32) at every scene pixel the batch covers; C = acc.shape[0] in 1..4."""
+    what = "scene_blend_image"
+    h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    if acc.dim() != 3 or not 1 <= acc.shape[0] <= 4:
+        raise ValueError(f"{what}: acc must be fp32 [C, {h}, {w}] with C in 1..4, got {tuple(acc.shape)}")
+    c = acc.shape[0]
+    if acc.dtype != torch.float32 or tuple(acc.shape) != (c, h, w) or not acc.is_contiguous():
+        raise ValueError(f"{what}: acc must be a contiguous fp32 [{c}, {h}, {w}] tensor")
+    if wsum.dtype != torch.float32 or tuple(wsum.shape) != (h, w) or not wsum.is_contiguous():
+        raise ValueError(f"{what}: wsum must be a contiguous fp32 [{h}, {w}] tensor")
+    batch = fake.shape[0] if fake.dim() == 4 else 0
+    if fake.dtype != torch.float32 or tuple(fake.shape) != (batch, ey, ex, 4) or not fake.is_contiguous() or batch < 1:
+        raise ValueError(f"{what}: fake must be a contiguous fp32 [batch, {ey}, {ex}, 4] tensor, got {fake.dtype} "
+                         f"{tuple(fake.shape)}")
+    if fake.data_ptr() % 16:
+        raise ValueError(f"{what}: fake must be 16-byte aligned (each 4-slot pixel is one 16-byte load)")
+    if ey + ex > SCENE_MAX_WINDOW:
+        raise ValueError(f"{what}: tile extents {ey} + {ex} exceed {SCENE_MAX_WINDOW}")
+    if not 0 <= tile0 < ny * nx:
+        raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
+    _cuda(what, fake, acc, wsum)
+    _lib.check(_lib.lib().gap_scene_blend_image(_ptr(fake), c, h, w, ey, ex, sy, sx, ny, nx, int(tile0), batch,
+                                                _ptr(acc), _ptr(wsum), _stream()), "gap_scene_blend_image")
+
+
+def scene_finalize_image(acc: torch.Tensor, wsum: torch.Tensor, image: torch.Tensor, write_float: bool) -> None:
+    """image (uint8 [H, W, C]) = uint8(clamp((v * 0.5 + 0.5) * 255, 0, 255)), truncated, of v = acc / wsum;
+    write_float: acc (fp32 [C, H, W]) becomes v in place."""
+    what = "scene_finalize_image"
+    if acc.dim() != 3 or not 1 <= acc.shape[0] <= 4:
+        raise ValueError(f"{what}: acc must be fp32 [C, H, W] with C in 1..4, got {tuple(acc.shape)}")
+    c, h, w = acc.shape
+    if acc.dtype != torch.float32 or not acc.is_contiguous():
+        raise ValueError(f"{what}: acc must be a contiguous fp32 [C, H, W] tensor")
+    if wsum.dtype != torch.float32 or tuple(wsum.shape) != (h, w) or not wsum.is_contiguous():
+        raise ValueError(f"{what}: wsum must be a contiguous fp32 [{h}, {w}] tensor")
+    if image.dtype != torch.uint8 or tuple(image.shape) != (h, w, c) or not image.is_contiguous():
+        raise ValueError(f"{what}: image must be a contiguous uint8 [{h}, {w}, {c}] tensor")
+    _cuda(what, acc, wsum, image)
+    _lib.check(_lib.lib().gap_scene_finalize_image(_ptr(acc), _ptr(wsum), c, h * w, _ptr(image),
+                                                   int(bool(write_float)), _stream()), "gap_scene_finalize_image")

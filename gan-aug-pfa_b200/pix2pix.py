@@ -22,12 +22,13 @@ from __future__ import annotations
 
 import functools
 from dataclasses import dataclass
-from typing import Dict, List, Optional, Tuple
+from typing import Dict, List, NamedTuple, Optional, Tuple
 
 import torch
 
 from . import ops
 from .ops import ACT_LRELU, ACT_NONE, ACT_RELU, ACT_TANH
+from .scene import _scene_grid
 from .spec import DiscriminatorSpec, GeneratorSpec
 
 BN_EPS = 1e-5
@@ -54,6 +55,13 @@ def discriminator_split(input_nc: int) -> Tuple[int, int]:
                                   f"{2 * IMAGE_SLOTS} channels are (two sources of up to {IMAGE_SLOTS} channels each)")
     ca = (input_nc + 1) // 2
     return ca, input_nc - ca
+
+
+class SceneImage(NamedTuple):
+    """translate_scene's result.  image: uint8 [H, W, output_nc], the picture generate_synthetic_data.py saves.
+    values: the blended fp32 Tanh outputs [output_nc, H, W] in [-1, 1] (return_float=True), else None."""
+    image: torch.Tensor
+    values: Optional[torch.Tensor]
 
 
 def _pad4(n: int) -> int:
@@ -666,6 +674,93 @@ class GeneratorEngine(_Net):
                            out_u8, co=self.output_nc)
         self.dropout_calls += 1
         return self.fake_f32
+
+    def _scene_input(self, img) -> Tuple[bool, int, int]:
+        """(is_uint8, h, w) of a translate_scene input, ValueError unless it is uint8 [H, W, input_nc] (host or device)
+        or fp32 [input_nc, H, W] on the engine's device."""
+        if not isinstance(img, torch.Tensor) or img.dim() != 3:
+            raise ValueError(f"img must be a uint8 [H, W, C] or fp32 [C, H, W] tensor, got "
+                             f"{getattr(img, 'shape', type(img))}")
+        if img.dtype == torch.uint8:
+            h, w, c = img.shape
+        elif img.dtype == torch.float32:
+            c, h, w = img.shape
+            if img.device.type != self.dev.type or (self.dev.index is not None and img.device.index != self.dev.index):
+                raise ValueError(f"img: an fp32 [C, H, W] scene must be on the engine's device {self.dev}, got "
+                                 f"{img.device}")
+        else:
+            raise ValueError(f"img must be uint8 [H, W, C] or fp32 [C, H, W], got {img.dtype}")
+        if c != self.input_nc:
+            raise ValueError(f"img has {c} channels, expected input_nc = {self.input_nc}")
+        if h < 1 or w < 1:
+            raise ValueError(f"img is empty: {tuple(img.shape)}")
+        return img.dtype == torch.uint8, h, w
+
+    @_on_device
+    def translate_scene(self, img: torch.Tensor, tile: int = 256, overlap: int = 64, batch: int = 32,
+                        return_float: bool = False) -> SceneImage:
+        """The generator's image of a whole scene of any size at its own resolution, by sliding-window inference: the
+        synthetic second image of a pair that lines up pixel for pixel with the first one and with its labels.
+
+        img: uint8 [H, W, input_nc] as PIL / numpy give it (host or device; normalised on the device as dataset.py's
+        ToTensor + Normalize(0.5, 0.5); a host scene is copied to the device once), or fp32 [input_nc, H, W] on the
+        device, already normalised (what forward() takes, rounded to bf16 as forward() does).  Any H, W >= 1.
+
+        The scene is cut into tiles of tile x tile pixels that overlap by `overlap` (scene.scene_axis: an axis shorter
+        than the tile gets one tile of its own length rounded up to 2^depth, padded by repeating the edge), and the
+        tiles run `batch` at a time through the eval-mode generator: BatchNorm with the running statistics, no dropout.
+        Their Tanh outputs are blended with the Gaussian window of scene.scene_window, v = sum_tiles w * v_tile /
+        sum_tiles w, summed in ascending tile index, so the blend does not depend on `batch`.  An InstanceNorm
+        generator normalises each tile by its own statistics, which is what a generator trained on crops of the tile
+        size sees.
+
+        tile: a multiple of 2^depth, depth = the number of stride-2 levels (num_downs: 128 at 7, 256 at 8), at most
+        6144.  0 <= overlap < tile, batch >= 1.  Returns SceneImage(image, values): image is uint8 [H, W, output_nc]
+        = uint8(clamp((v * 0.5 + 0.5) * 255, 0, 255)), truncated as the out_u8 output of forward() and torchvision's
+        to_pil_image; values (return_float=True) is v, fp32 [output_nc, H, W].
+
+        Memory: (output_nc + 1) * 4 bytes per scene pixel of accumulators (which become `values`), output_nc bytes
+        for `image`, and the generator's activation buffers sized for `batch` tiles.  Like any call at a new shape,
+        this re-sizes those buffers: the next training step re-allocates them, and Pix2PixTrainer.train_step_graphed
+        re-captures its graph.  Everything runs on the current stream; device inputs need no host synchronisation.
+        The `training` flag is restored afterwards, and no parameter, gradient, BatchNorm buffer or dropout counter
+        changes, so later training draws the dropout masks it would have drawn without this call.  Bad arguments
+        raise ValueError before any work is enqueued."""
+        if self.virtual0:
+            raise ValueError("translate_scene needs a whole generator: a stand-alone inner block has no image output")
+        for name, v in (("tile", tile), ("overlap", overlap), ("batch", batch)):
+            if isinstance(v, bool) or not isinstance(v, int):
+                raise ValueError(f"{name} must be an int, got {v!r}")
+        align = 1 << self.L                          # the input side must divide by 2 at every stride-2 level
+        if tile < align or tile % align:
+            raise ValueError(f"tile must be a positive multiple of 2^{self.L} = {align}, got {tile}")
+        if 2 * tile > ops.SCENE_MAX_WINDOW:
+            raise ValueError(f"tile must be at most {ops.SCENE_MAX_WINDOW // 2}, got {tile}")
+        if not 0 <= overlap < tile:
+            raise ValueError(f"overlap must be in [0, tile = {tile}), got {overlap}")
+        if batch < 1:
+            raise ValueError(f"batch must be >= 1, got {batch}")
+        _, h, w = self._scene_input(img)
+        oc = self.output_nc
+        grid = _scene_grid(h, w, tile, overlap, align)
+        (_, ey, _, ny), (_, ex, _, nx) = grid
+        img = img.to(self.dev).contiguous()
+        acc = torch.empty(oc, h, w, device=self.dev)       # every pixel is written by the batch of its first tile
+        wsum = torch.empty(h, w, device=self.dev)
+        image = torch.empty(h, w, oc, device=self.dev, dtype=torch.uint8)
+        was, calls = self.training, self.dropout_calls
+        self.training = False
+        try:
+            self._alloc(batch, ey, ex)
+            for t0 in range(0, ny * nx, batch):             # the last batch is padded with zero tiles
+                ops.scene_gather_one(img, grid, t0, self.x_nhwc)
+                self.forward(None, x_ready=True)
+                ops.scene_blend_image(self.fake_f32, grid, t0, acc, wsum)
+            ops.scene_finalize_image(acc, wsum, image, return_float)
+        finally:
+            self.training = was
+            self.dropout_calls = calls
+        return SceneImage(image, acc if return_float else None)
 
     def _dropout_layer(self, j: int) -> bool:
         """True if the block whose up-conv output is yu[j] ends in nn.Dropout(0.5) (training mode only)."""

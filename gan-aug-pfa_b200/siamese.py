@@ -27,6 +27,7 @@ import torch
 from . import ops
 from .ops import ACT_NONE, ACT_RELU
 from .pix2pix import BN_EPS, BN_MOMENTUM, _BN, _Net, _on_device
+from .scene import _scene_grid, scene_axis, scene_window  # noqa: F401  (predict_scene's grid and window)
 
 ENC = (("dconv_down1", 64), ("dconv_down2", 128), ("dconv_down3", 256), ("dconv_down4", 512), ("bottleneck", 1024))
 MAX_CLASSES = ops.MAX_CLASSES
@@ -43,36 +44,6 @@ def check_n_classes(n_classes) -> None:
     if isinstance(n_classes, bool) or not isinstance(n_classes, int) or not 1 <= n_classes <= MAX_CLASSES:
         raise NotImplementedError(f"n_classes = {n_classes!r} is not implemented natively: 1 to {MAX_CLASSES} classes "
                                   "are")
-
-
-def scene_axis(length: int, tile: int, overlap: int) -> Tuple[List[int], int]:
-    """The tile origins along one scene axis of `length` pixels and the tile extent E (predict_scene's grid; csrc/scene.cu
-    derives the same origins on the device).  length <= tile: one tile at 0 with E = ceil16(length), whose reads past
-    the scene clamp to its last row / column.  Otherwise E = tile, step S = tile - overlap and
-    n = ceil((length - tile) / S) + 1 tiles at min(i*S, length - tile): the last one is snapped to the edge."""
-    if length <= tile:
-        return [0], -(-length // 16) * 16
-    step = tile - overlap
-    n = -(-(length - tile) // step) + 1
-    return [min(i * step, length - tile) for i in range(n)], tile
-
-
-def scene_window(extent: int) -> torch.Tensor:
-    """The 1-D blending window of a tile axis, fp64 [extent]: g(t) = exp(-(t + 0.5 - E/2)^2 / (2 sigma^2)), sigma = E/8
-    (nnU-Net's choice); a tile's weight is g_y(ty) * g_x(tx).  Its smallest value is about exp(-8), so every covered
-    pixel has a positive weight sum, and with overlap 0 it cancels (plain stitching)."""
-    t = torch.arange(extent, dtype=torch.float64)
-    sigma = extent / 8
-    return torch.exp(-(t + 0.5 - extent / 2) ** 2 / (2 * sigma ** 2))
-
-
-def _scene_grid(h: int, w: int, tile: int, overlap: int):
-    """((len, ext, step, n) of the y axis, same of the x axis): the grid in the form the scene kernels take."""
-    out = []
-    for length in (h, w):
-        origins, ext = scene_axis(length, tile, overlap)
-        out.append((length, ext, tile - overlap if len(origins) > 1 else ext, len(origins)))
-    return tuple(out)
 
 
 class SceneResult(NamedTuple):

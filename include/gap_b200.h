@@ -396,6 +396,21 @@ int gap_scene_blend(const float* logits, int k, int h, int w, int ey, int ex, in
  * counted.  The caller zeroes counts. */
 int gap_scene_finalize(float* acc, const float* wsum, int k, int64_t pixels, uint8_t* pred, int write_probs,
                        const int64_t* labels, int64_t ignore_index, int64_t* counts, void* stream);
+/* The generator's scene kernels (GeneratorEngine.translate_scene), on the same tile grid and window.
+ * gather_one: tiles tile0 .. tile0+batch-1 of one scene -> NHWC bf16 [batch][ey][ex][4 slots] (out, dense, 8-byte
+ *   aligned), with the values, zero slots and zero padding tiles of gap_scene_gather. */
+int gap_scene_gather_one(const void* img, int src_u8, int c, int h, int w, int ey, int ex, int sy, int sx, int ny,
+                         int nx, int tile0, int batch, void* out, void* stream);
+/* blend_image: the generator's fp32 output of tiles tile0 .. , fake [batch][ey][ex][4 slots] (16-byte aligned) ->
+ *   for every scene pixel, over the covering tiles of this batch in ascending index: acc[ch][pixel] += w * v_ch for
+ *   ch < c, wsum[pixel] += w (fp32 [c][h][w] and [h][w]); c = 1..4.  Same start-from-zero rule as gap_scene_blend, no
+ *   floating-point atomics.  ey + ex <= 12288 (the window table lives in shared memory). */
+int gap_scene_blend_image(const float* fake, int c, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx,
+                          int tile0, int batch, float* acc, float* wsum, void* stream);
+/* finalize_image: v = acc / wsum over `pixels`; image (uint8 [pixels][c]) = uint8(clamp((v*0.5 + 0.5)*255, 0, 255)),
+ *   truncated; write_float: acc is overwritten with v.  c = 1..4. */
+int gap_scene_finalize_image(float* acc, const float* wsum, int c, int64_t pixels, uint8_t* image, int write_float,
+                             void* stream);
 
 /* evaluate.py:34-64 calculate_metrics, device side: per-sample counts[n][4] += [TP, FP, FN, TN] of
  * (sigmoid(logits) > 0.5) against {0,1} labels (int64 when labels_are_i64, else fp32); logits are [n][hw] fp32.
