@@ -20,6 +20,7 @@
 #include <algorithm>
 
 #include "common.h"
+#include "confusion.cuh"
 #include "ptx.cuh"
 
 namespace gap {
@@ -226,7 +227,7 @@ __global__ void __launch_bounds__(256) scene_finalize_kernel(float* __restrict__
   constexpr int KM = KT > 0 ? KT : kSceneMaxClasses;
   const int K = KT > 0 ? KT : k;
   const int bins = K == 1 ? 4 : K * K;
-  __shared__ unsigned int hist[kSceneMaxClasses * kSceneMaxClasses];
+  __shared__ unsigned int hist[kConfusionMaxBins];
   if (labels) {
     for (int i = threadIdx.x; i < bins; i += blockDim.x) hist[i] = 0u;
     __syncthreads();
@@ -256,21 +257,13 @@ __global__ void __launch_bounds__(256) scene_finalize_kernel(float* __restrict__
           }
       }
       pred[i] = static_cast<uint8_t>(best);
-      if (labels) {
-        const long long y = labels[i];
-        if (y != ignore && y >= 0 && y < (K == 1 ? 2 : K))
-          bin = K == 1 ? (y == 1 ? (best ? 0 : 2) : (best ? 1 : 3)) : static_cast<int>(y) * K + best;
-      }
+      if (labels) bin = confusion_bin(labels[i], best, K, ignore);
     }
-    if (labels) {
-      const unsigned int peers = __match_any_sync(0xffffffffu, bin);
-      if (bin >= 0 && (threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(&hist[bin], __popc(peers));
-    }
+    if (labels) hist_add_warp(hist, bin);
   }
   if (labels) {
     __syncthreads();
-    for (int i = threadIdx.x; i < bins; i += blockDim.x)
-      if (hist[i]) atomicAdd(counts + i, static_cast<unsigned long long>(hist[i]));
+    hist_flush(hist, bins, counts);
   }
 }
 

@@ -91,3 +91,18 @@ def multiclass_metrics(counts, smooth: float = 1e-6) -> Dict[str, object]:
     accuracy = (tp.sum() + smooth) / (total + smooth)
     return {"precision": precision.tolist(), "recall": recall.tolist(), "f1": f1.tolist(), "iou": iou.tolist(),
             "mean_iou": float(iou.mean()), "accuracy": float(accuracy)}
+
+
+OBJECT_KEYS = ("precision", "recall", "f1")
+
+
+def object_metrics(object_counts, smooth: float = 1e-6) -> Dict[str, List[float]]:
+    """Object-level precision (matched / predicted objects), recall (detected / reference objects) and F1 per change
+    class 1..K-1 (lists, index 0 = class 1) from the int64 [max(K, 2), 4] object_counts of objects.change_objects,
+    with the formulas and ``smooth`` placement of ``metrics_from_counts``."""
+    c = torch.as_tensor(object_counts).detach().cpu().to(torch.int64)[1:].to(torch.float32)
+    ref, det, prd, mat = c.unbind(1)
+    precision = (mat + smooth) / (prd + smooth)
+    recall = (det + smooth) / (ref + smooth)
+    f1 = (2 * precision * recall + smooth) / (precision + recall + smooth)
+    return {"precision": precision.tolist(), "recall": recall.tolist(), "f1": f1.tolist()}

@@ -1168,3 +1168,83 @@ def scene_finalize_image(acc: torch.Tensor, wsum: torch.Tensor, image: torch.Ten
     _cuda(what, acc, wsum, image)
     _lib.check(_lib.lib().gap_scene_finalize_image(_ptr(acc), _ptr(wsum), c, h * w, _ptr(image),
                                                    int(bool(write_float)), _stream()), "gap_scene_finalize_image")
+
+
+# ------------------------------------------------------------------------------------------------
+# Change objects (gap_b200.h "Change objects"): connected components of a class map [n, h, w], flat int32 buffers of
+# n*h*w pixels
+# ------------------------------------------------------------------------------------------------
+OBJECTS_CHUNK = 4096            # pixels per entry of gap_objects_number's chunk scratch
+
+
+def _flat(t: Optional[torch.Tensor], numel: int, dtype, what: str, name: str) -> None:
+    if t is not None and (t.dtype != dtype or t.numel() != numel or not t.is_contiguous()):
+        raise ValueError(f"{what}: {name} must be a contiguous {dtype} tensor of {numel} elements, got {t.dtype} "
+                         f"{tuple(t.shape)}")
+
+
+def objects_label(src: torch.Tensor, n: int, h: int, w: int, k: int, connectivity: int, parent: torch.Tensor,
+                  area: torch.Tensor, classes: Optional[torch.Tensor] = None, info: Optional[torch.Tensor] = None,
+                  ignore_index: int = -100) -> None:
+    """Components of a uint8 pred (info: int32 [2], info[1] counts values >= max(k, 2)) or of int64 labels (classes:
+    uint8, the label class or 255 for ignore_index / out-of-range labels): parent <- each pixel's root, area <- the
+    pixel count at each root (int32, n*h*w each)."""
+    what = "objects_label"
+    _check_k(k, what)
+    px = n * h * w
+    i64 = src.dtype == torch.int64
+    _flat(src, px, torch.int64 if i64 else torch.uint8, what, "src")
+    for name, t, dt in (("parent", parent, torch.int32), ("area", area, torch.int32), ("classes", classes, torch.uint8),
+                        ("info", info, torch.int32)):
+        _flat(t, 2 if name == "info" else px, dt, what, name)
+    if i64 != (classes is not None) or (not i64 and info is None):
+        raise ValueError(f"{what}: int64 labels need classes, a uint8 pred needs info")
+    _cuda(what, src, parent, area, classes, info)
+    _lib.check(_lib.lib().gap_objects_label(_ptr(src), int(i64), n, h, w, k, int(ignore_index), int(connectivity),
+                                            _ptr(classes), _ptr(parent), _ptr(area), _ptr(info), _stream()),
+               "gap_objects_label")
+
+
+def objects_number(pred: torch.Tensor, parent: torch.Tensor, area_ids: torch.Tensor, min_area: int,
+                   chunk: torch.Tensor, info: torch.Tensor) -> None:
+    """Roots of non-zero class with area >= min_area get ids 1..count in raster order (area_ids[root], 0 for the
+    others); info[0] <- count.  chunk: int32 scratch of ceil(pixels / OBJECTS_CHUNK)."""
+    what = "objects_number"
+    px = pred.numel()
+    _flat(pred, px, torch.uint8, what, "pred")
+    _flat(parent, px, torch.int32, what, "parent")
+    _flat(area_ids, px, torch.int32, what, "area_ids")
+    _flat(chunk, -(-px // OBJECTS_CHUNK), torch.int32, what, "chunk")
+    _flat(info, 2, torch.int32, what, "info")
+    _cuda(what, pred, parent, area_ids, chunk, info)
+    _lib.check(_lib.lib().gap_objects_number(_ptr(pred), _ptr(parent), _ptr(area_ids), px, int(min_area), _ptr(chunk),
+                                             _ptr(info), _stream()), "gap_objects_number")
+
+
+def objects_finish(pred: torch.Tensor, parent: torch.Tensor, ids: torch.Tensor, n: int, h: int, w: int, k: int,
+                   count: int, pred_out: torch.Tensor, objects: torch.Tensor, overlap: Optional[torch.Tensor] = None,
+                   lparent: Optional[torch.Tensor] = None, larea: Optional[torch.Tensor] = None,
+                   loverlap: Optional[torch.Tensor] = None, min_overlap: float = 0.0,
+                   confusion: Optional[torch.Tensor] = None, object_counts: Optional[torch.Tensor] = None) -> None:
+    """ids of every pixel, pred_out (pred with dropped objects zeroed) and objects (int64 [count, 7]); with the label
+    map's lparent / larea (and its classes in pred_out on entry): confusion and object_counts (see gap_b200.h)."""
+    what = "objects_finish"
+    _check_k(k, what)
+    px = n * h * w
+    kk = max(k, 2)
+    for name, t, numel, dt in (("pred", pred, px, torch.uint8), ("parent", parent, px, torch.int32),
+                               ("ids", ids, px, torch.int32), ("pred_out", pred_out, px, torch.uint8),
+                               ("objects", objects, count * 7, torch.int64), ("overlap", overlap, count, torch.int32),
+                               ("lparent", lparent, px, torch.int32), ("larea", larea, px, torch.int32),
+                               ("loverlap", loverlap, px, torch.int32),
+                               ("confusion", confusion, 4 if k == 1 else k * k, torch.int64),
+                               ("object_counts", object_counts, kk * 4, torch.int64)):
+        _flat(t, numel, dt, what, name)
+    labelled = (lparent, larea, loverlap, confusion, object_counts, overlap)
+    if any(t is None for t in labelled) and any(t is not None for t in labelled):
+        raise ValueError(f"{what}: lparent, larea, loverlap, overlap, confusion and object_counts go together")
+    _cuda(what, pred, parent, ids, pred_out, objects, *labelled)
+    _lib.check(_lib.lib().gap_objects_finish(_ptr(pred), _ptr(parent), _ptr(ids), n, h, w, k, int(count),
+                                             _ptr(pred_out), _ptr(overlap), _ptr(objects), _ptr(lparent), _ptr(larea),
+                                             _ptr(loverlap), float(min_overlap), _ptr(confusion),
+                                             _ptr(object_counts), _stream()), "gap_objects_finish")

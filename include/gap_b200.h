@@ -412,6 +412,32 @@ int gap_scene_blend_image(const float* fake, int c, int h, int w, int ey, int ex
 int gap_scene_finalize_image(float* acc, const float* wsum, int c, int64_t pixels, uint8_t* image, int write_float,
                              void* stream);
 
+/* Change objects (objects.cu, objects.change_objects): connected components of one non-zero class within one sample of
+ * a class map [n][h][w] (4- or 8-connected), numbered 1..count in raster order of their first pixel over (n, y, x).
+ * k = 1..16 classes (k = 1 is the 0/1 map: two classes); kk = max(k, 2); n*h*w < 2^31.  Deterministic: every union
+ * links the larger root under the smaller, so each root is its component's first pixel.
+ * label: src_i64 = 0: src is the uint8 pred; classes must be null; info (int32[2]) is zeroed and info[1] counts
+ *   values >= kk.  src_i64 = 1: src is int64 labels; classes (uint8 [n*h*w]) receives the label class, 0xFF for
+ *   ignore_index and values outside [0, kk).  parent (int32 [n*h*w]) <- each object pixel's root (its own index for
+ *   class 0); area (int32 [n*h*w], zeroed here) <- the pixel count at each root. */
+int gap_objects_label(const void* src, int src_i64, int n, int h, int w, int k, int64_t ignore_index, int connectivity,
+                      uint8_t* classes, int32_t* parent, int32_t* area, int32_t* info, void* stream);
+/* number: a root of non-zero class is kept when its area >= min_area; area_ids[root] <- its id (1 + kept roots before
+ *   it) or 0; info[0] <- the number of kept roots.  chunk: int32 scratch of ceil(pixels / 4096). */
+int gap_objects_number(const uint8_t* pred, const int32_t* parent, int32_t* area_ids, int64_t pixels, int64_t min_area,
+                       int32_t* chunk, int32_t* info, void* stream);
+/* finish, once count (= info[0]) is known: ids (area_ids of number) <- the id of every pixel (0: background or dropped);
+ *   pred_out (uint8) <- pred with dropped objects set to 0; objects (int64 [count][7]) <- (sample, class, area, y0, x0,
+ *   y1, x1), inclusive box.  With labels (lparent / larea of gap_objects_label on the label map, their classes in
+ *   pred_out on entry; lparent is consumed): confusion (k > 1: [k][k], rows = label; k = 1: [TP, FP, FN, TN]) of
+ *   pred_out; object_counts [kk][4] <- per class (reference objects, detected ones, predicted objects, matched ones),
+ *   where an object matches when at least max(1, ceil(min_overlap * area)) of its pixels have the other map's class;
+ *   overlap (int32 [count]) and loverlap (int32 [n*h*w]) are scratch.  confusion and object_counts are zeroed here. */
+int gap_objects_finish(const uint8_t* pred, const int32_t* parent, int32_t* ids, int n, int h, int w, int k,
+                       int64_t count, uint8_t* pred_out, int32_t* overlap, int64_t* objects, int32_t* lparent,
+                       const int32_t* larea, int32_t* loverlap, double min_overlap, int64_t* confusion,
+                       int64_t* object_counts, void* stream);
+
 /* evaluate.py:34-64 calculate_metrics, device side: per-sample counts[n][4] += [TP, FP, FN, TN] of
  * (sigmoid(logits) > 0.5) against {0,1} labels (int64 when labels_are_i64, else fp32); logits are [n][hw] fp32.
  * The caller zeroes counts once and may accumulate several batches; the ratios are formed on the host. */
