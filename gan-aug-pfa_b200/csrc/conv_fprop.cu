@@ -619,7 +619,9 @@ conv_fprop_kernel(const __grid_constant__ FpropParams p) {
                 my_stats[256 + c * 16 + stat_col + 8] += static_cast<double>(cs[3]);
               }
             }
-            if (valid && !(p.skip & 1)) st_global_32B(p.out + pix * p.out_ld + col0, pk, true);
+            // n_tiles * block_n can exceed n_out (272 = 2 x 144, 640 = 3 x 224): the chunks past the last channel are
+            // whole (n_out - c0 and c0 are multiples of 16) and are not stored
+            if (valid && col0 < p.n_out && !(p.skip & 1)) st_global_32B(p.out + pix * p.out_ld + col0, pk, true);
             continue;
           }
           if (p.scale != nullptr) {
