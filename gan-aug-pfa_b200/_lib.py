@@ -137,6 +137,8 @@ _SIGNATURES = {
     "gap_seg_confusion_ck": (C.c_int, [_P, _P, _I, _I, _L, _L, _P, _P]),
     "gap_scene_gather": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "gap_scene_blend": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "gap_scene_gather_tta": (C.c_int, [_P, _P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
+    "gap_scene_blend_tta": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),
     "gap_scene_finalize": (C.c_int, [_P, _P, _I, _L, _P, _I, _P, _L, _P, _P]),
     "gap_scene_gather_one": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P]),
     "gap_scene_blend_image": (C.c_int, [_P, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _I, _P, _P, _P]),

@@ -14,6 +14,8 @@
 // gap_scene_gather   scene pixels (uint8 HWC or fp32 CHW) -> the engine's two 4-slot NHWC bf16 input batches
 // gap_scene_blend    logits of one batch -> acc[K][H][W] += w p, wsum[H][W] += w (gather form, no float atomics)
 // gap_scene_finalize acc / wsum -> uint8 pred (argmax or > 0.5), optional in-place probabilities, confusion counts
+// gap_scene_gather_tta / gap_scene_blend_tta  the same gather and blend for a dihedral transform d of every tile, and
+//                    a blend that keeps adding over several passes (test-time augmentation, checkpoint ensembles)
 // gap_scene_gather_one      one scene -> the generator's 4-slot NHWC bf16 input batch
 // gap_scene_blend_image     generator output of one batch (fp32 [batch][ey][ex][4]) -> acc[C][H][W] += w v, wsum += w
 // gap_scene_finalize_image  acc / wsum -> uint8 image [H][W][C] (the Tanh output's 8-bit rule), optional in-place values
@@ -94,116 +96,241 @@ __device__ __forceinline__ bool visit_batch_tiles(const SceneAxis& ay, const Sce
 }
 
 // ------------------------------------------------------------------------------------------------
-// Gather: one thread per pixel of the batch, NIMG = 1 or 2 scenes.  Tile index tile0 + b >= ny*nx is a padding tile
-// (zeros).  The values are those of gap_u8_hwc_to_nhwc_bf16_c (x * 2/255 - 1) / gap_nchw_f32_to_nhwc_bf16 (round to
-// nearest) on the same crop; slots >= C are zero.
+// Dihedral tile transforms (test-time augmentation).  d = 4 s + 2 v + u: f_d transposes the tile's two axes if s, then
+// flips its rows if v, then its columns if u, so the network sees [ex][ey] when s = 1.  Pixel (ty, tx) of a tile sits
+// at (i, j) of f_d(tile) with (i, j) = (s ? tx : ty, s ? ty : tx), i -> OY-1-i if v, j -> OX-1-j if u, where
+// [OY][OX] is the transformed extent; the logits of f_d(tile) are read back at the same (i, j) (the map f_d^-1).
 // ------------------------------------------------------------------------------------------------
-template <int C, bool U8, int NIMG>
+__device__ __forceinline__ long long tta_offset(int d, int ty, int tx, int ey, int ex) {
+  const bool s = d & 4;
+  const int oy = s ? ex : ey, ox = s ? ey : ex;
+  int i = s ? tx : ty, j = s ? ty : tx;
+  if (d & 2) i = oy - 1 - i;
+  if (d & 1) j = ox - 1 - j;
+  return static_cast<long long>(i) * ox + j;
+}
+
+// The 4-slot values of scene pixel p: gap_u8_hwc_to_nhwc_bf16_c (x * 2/255 - 1) or gap_nchw_f32_to_nhwc_bf16 (round to
+// nearest) of the same pixel, slots >= C zero, packed as one 8-byte NHWC bf16 pixel.
+template <int C, bool U8>
+__device__ __forceinline__ uint2 scene_pixel(const void* img, long long p, long long hw) {
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  if (U8) {
+    const uint8_t* s = static_cast<const uint8_t*>(img) + p * C;
+#pragma unroll
+    for (int j = 0; j < C; ++j) v[j] = s[j] * (2.f / 255.f) - 1.f;
+  } else {
+    const float* s = static_cast<const float*>(img) + p;
+#pragma unroll
+    for (int j = 0; j < C; ++j) v[j] = __ldg(s + j * hw);
+  }
+  return make_uint2(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]));
+}
+
+// ------------------------------------------------------------------------------------------------
+// Gather, NIMG = 1 or 2 scenes, of f_d of every tile (d < 4 when S = false, d >= 4 when S = true).  Tile index
+// tile0 + b >= ny*nx is a padding tile (zeros).
+// S = false: one thread per output pixel; consecutive threads read consecutive (or, flipped, reversed) scene columns.
+// S = true (transposed tiles): one CTA of 256 threads per 16 x 16 square of an output tile.  The threads first read
+// the square's source pixels along scene rows into shared memory, then write the output square row by row from there,
+// so both the scene reads and the output writes stay coalesced.  Extents are multiples of 16: squares are whole.
+// ------------------------------------------------------------------------------------------------
+template <int C, bool U8, int NIMG, bool S>
 __global__ void __launch_bounds__(256) scene_gather_kernel(const void* __restrict__ img1, const void* __restrict__ img2,
-                                                           SceneAxis ay, SceneAxis ax, int tile0, int batch,
+                                                           SceneAxis ay, SceneAxis ax, int tile0, int batch, int d,
                                                            bf16* __restrict__ out1, bf16* __restrict__ out2) {
   const long long per_tile = static_cast<long long>(ay.ext) * ax.ext;
-  const long long total = per_tile * batch;
   const long long hw = static_cast<long long>(ay.len) * ax.len;
   const int n_tiles = ay.n * ax.n;
   const void* img[2] = {img1, img2};
   bf16* out[2] = {out1, out2};
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int b = static_cast<int>(i / per_tile);
-    const int r = static_cast<int>(i - b * per_tile);
-    const int t = tile0 + b;
-    float v[NIMG][4];
+  const int oy = S ? ax.ext : ay.ext, ox = S ? ay.ext : ax.ext;       // the transformed extent [oy][ox]
+  if constexpr (!S) {
+    const long long total = per_tile * batch;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+      const int b = static_cast<int>(i / per_tile);
+      const int r = static_cast<int>(i - b * per_tile);
+      const int t = tile0 + b;
+      uint2 v[NIMG];
 #pragma unroll
-    for (int m = 0; m < NIMG; ++m) v[m][0] = v[m][1] = v[m][2] = v[m][3] = 0.f;
-    if (t < n_tiles) {
-      const int ty = t / ax.n, tx = t - ty * ax.n;
-      const int y = min(axis_origin(ay, ty) + r / ax.ext, ay.len - 1);
-      const int x = min(axis_origin(ax, tx) + r % ax.ext, ax.len - 1);
-      const long long p = static_cast<long long>(y) * ax.len + x;
+      for (int m = 0; m < NIMG; ++m) v[m] = make_uint2(0u, 0u);
+      if (t < n_tiles) {
+        const int ty = t / ax.n, tx = t - ty * ax.n;
+        const int ri = r / ox, rj = r % ox;
+        const int y = min(axis_origin(ay, ty) + ((d & 2) ? oy - 1 - ri : ri), ay.len - 1);
+        const int x = min(axis_origin(ax, tx) + ((d & 1) ? ox - 1 - rj : rj), ax.len - 1);
+        const long long p = static_cast<long long>(y) * ax.len + x;
 #pragma unroll
-      for (int m = 0; m < NIMG; ++m) {
-        if (U8) {
-          const uint8_t* s = static_cast<const uint8_t*>(img[m]) + p * C;
-#pragma unroll
-          for (int j = 0; j < C; ++j) v[m][j] = s[j] * (2.f / 255.f) - 1.f;
-        } else {
-          const float* s = static_cast<const float*>(img[m]) + p;
-#pragma unroll
-          for (int j = 0; j < C; ++j) v[m][j] = __ldg(s + j * hw);
-        }
+        for (int m = 0; m < NIMG; ++m) v[m] = scene_pixel<C, U8>(img[m], p, hw);
       }
-    }
 #pragma unroll
-    for (int m = 0; m < NIMG; ++m)
-      *reinterpret_cast<uint2*>(out[m] + i * 4) =
-          make_uint2(pack_bf16x2(v[m][0], v[m][1]), pack_bf16x2(v[m][2], v[m][3]));
+      for (int m = 0; m < NIMG; ++m) *reinterpret_cast<uint2*>(out[m] + i * 4) = v[m];
+    }
+  } else {
+    __shared__ uint2 sq[NIMG][16][17];                  // [source row][source column] of one square, padded
+    const int sqx = ox / 16, per_tile_sq = (oy / 16) * sqx;
+    const int lo = threadIdx.x & 15, hi = threadIdx.x >> 4;
+    for (int q = blockIdx.x; q < batch * per_tile_sq; q += gridDim.x) {   // uniform per CTA
+      const int b = q / per_tile_sq, qs = q - b * per_tile_sq;
+      const int r0 = (qs / sqx) * 16, c0 = (qs % sqx) * 16;        // the output square [r0, r0+16) x [c0, c0+16)
+      const int t = tile0 + b;
+      // its source: tile rows ty = c0.. (or, flipped, ox-16-c0..), tile columns tx = r0.. (or oy-16-r0..)
+      const int sy0 = (d & 1) ? ox - 16 - c0 : c0, sx0 = (d & 2) ? oy - 16 - r0 : r0;
+      const bool real = t < n_tiles;
+      __syncthreads();                                 // the previous square's reads of sq are done
+      if (real) {
+        const int ty = t / ax.n, tx = t - ty * ax.n;
+        const int y = min(axis_origin(ay, ty) + sy0 + hi, ay.len - 1);
+        const int x = min(axis_origin(ax, tx) + sx0 + lo, ax.len - 1);
+        const long long p = static_cast<long long>(y) * ax.len + x;
+#pragma unroll
+        for (int m = 0; m < NIMG; ++m) sq[m][hi][lo] = scene_pixel<C, U8>(img[m], p, hw);
+      }
+      __syncthreads();
+      // output pixel (r0 + hi, c0 + lo) is tile pixel (ty, tx) = (c', r') with c' = c0 + lo or ox-1-(c0 + lo) and
+      // r' = r0 + hi or oy-1-(r0 + hi); relative to the source square that is (lo or 15 - lo, hi or 15 - hi)
+      const int a = (d & 1) ? 15 - lo : lo, bb = (d & 2) ? 15 - hi : hi;
+      const long long o = (static_cast<long long>(b) * per_tile + static_cast<long long>(r0 + hi) * ox + c0 + lo) * 4;
+#pragma unroll
+      for (int m = 0; m < NIMG; ++m)
+        *reinterpret_cast<uint2*>(out[m] + o) = real ? sq[m][a][bb] : make_uint2(0u, 0u);
+    }
   }
 }
 
 // ------------------------------------------------------------------------------------------------
-// Blend, gather form: one thread per scene pixel of the box [y0, y0+bh) x [x0, x0+bw) that the batch's tiles
-// [t0, t1) cover.  The thread visits the tiles of the batch that cover its pixel in ascending index and adds w*p and w
-// onto the running sums, one fused multiply-add per tile, so each pixel sees the same sequence of operations whatever
-// the batch size.  When the first tile of the whole grid that covers the pixel is in this batch the sums start from
-// zero (the accumulators need no clearing), otherwise from what the earlier batches stored.  KT: the class count when
-// fixed at compile time (1 = sigmoid), 0 = runtime k <= 16.
+// Blend, gather form, over the scene pixels of the box [y0, y0+bh) x [x0, x0+bw) that the batch's tiles [t0, t1)
+// cover.  Each pixel visits the tiles of the batch that cover it in ascending index and adds w*p and w onto its
+// running sums, one fused multiply-add per tile, so each pixel sees the same sequence of operations whatever the batch
+// size.  When the first tile of the whole grid that covers the pixel is in this batch and this is the first pass the
+// sums start from zero (the accumulators need no clearing), otherwise from what the earlier batches and passes stored.
+// The logits are those of f_d(tile) (tta_offset).  KT: the class count when fixed at compile time (1 = sigmoid),
+// 0 = runtime k <= 16.
+// S = false (d < 4): one thread per pixel, consecutive threads on consecutive (flipped: reversed) tile columns.
+// S = true (d >= 4, logits [ex][ey] per class plane): one CTA per 16 x 16 box of pixels.  For each batch tile that
+// covers part of the box, in ascending index, the threads first copy the box's logits into shared memory with
+// consecutive threads on consecutive scene rows (consecutive addresses of the transposed plane), then every thread
+// reads its pixel's K values from there; the per-pixel arithmetic is that of S = false.
 // ------------------------------------------------------------------------------------------------
-template <int KT>
-__global__ void __launch_bounds__(256) scene_blend_kernel(const float* __restrict__ logits, int k, SceneAxis ay,
-                                                          SceneAxis ax, int t0, int t1, int y0, int x0, int bh, int bw,
-                                                          float* __restrict__ acc, float* __restrict__ wsum) {
+template <int KT, class LD>
+__device__ __forceinline__ void blend_tile(LD ld, int K, float w, float* a) {
   constexpr int KM = KT > 0 ? KT : kSceneMaxClasses;
-  const int K = KT > 0 ? KT : k;
-  const long long total = static_cast<long long>(bh) * bw;
-  const long long hw = static_cast<long long>(ay.len) * ax.len;
-  const long long tile_px = static_cast<long long>(ay.ext) * ax.ext;
-  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
-       i += static_cast<long long>(gridDim.x) * blockDim.x) {
-    const int Y = y0 + static_cast<int>(i / bw), X = x0 + static_cast<int>(i % bw);
-    PixelCover cv;
-    if (!batch_cover(ay, ax, Y, X, t0, t1, cv)) continue;
-    const long long p = static_cast<long long>(Y) * ax.len + X;
-    float a[KM];
-    float ws = 0.f;
-#pragma unroll
-    for (int c = 0; c < KM; ++c) a[c] = (c < K && !cv.fresh) ? acc[c * hw + p] : 0.f;
-    if (!cv.fresh) ws = wsum[p];
-    const bool any = visit_batch_tiles(
-        ay, ax, Y, X, t0, t1, cv, [&](int d) { return window(d, ay.ext); }, [&](int d) { return window(d, ax.ext); },
-        [&](int b, int ty, int tx, float w) {
-          const float* lg = logits + b * K * tile_px + static_cast<long long>(ty) * ax.ext + tx;
-          if (KT == 1) {
-            const float pr = 1.f / (1.f + expf(-__ldg(lg)));
-            a[0] = fmaf(w, pr, a[0]);
-          } else {
-            float v[KM];
-            float m = -INFINITY;
-#pragma unroll
-            for (int c = 0; c < KM; ++c)
-              if (c < K) {
-                v[c] = __ldg(lg + c * tile_px);
-                m = fmaxf(m, v[c]);
-              }
-            float se = 0.f;
-#pragma unroll
-            for (int c = 0; c < KM; ++c)
-              if (c < K) {
-                v[c] = expf(v[c] - m);
-                se += v[c];
-              }
-            const float inv = 1.f / se;
-#pragma unroll
-            for (int c = 0; c < KM; ++c)
-              if (c < K) a[c] = fmaf(w, v[c] * inv, a[c]);
-          }
-          ws += w;
-        });
-    if (!any) continue;
+  if (KT == 1) {
+    const float pr = 1.f / (1.f + expf(-ld(0)));
+    a[0] = fmaf(w, pr, a[0]);
+  } else {
+    float v[KM];
+    float m = -INFINITY;
 #pragma unroll
     for (int c = 0; c < KM; ++c)
-      if (c < K) acc[c * hw + p] = a[c];
-    wsum[p] = ws;
+      if (c < K) {
+        v[c] = ld(c);
+        m = fmaxf(m, v[c]);
+      }
+    float se = 0.f;
+#pragma unroll
+    for (int c = 0; c < KM; ++c)
+      if (c < K) {
+        v[c] = expf(v[c] - m);
+        se += v[c];
+      }
+    const float inv = 1.f / se;
+#pragma unroll
+    for (int c = 0; c < KM; ++c)
+      if (c < K) a[c] = fmaf(w, v[c] * inv, a[c]);
+  }
+}
+
+template <int KT, bool S>
+__global__ void __launch_bounds__(256) scene_blend_kernel(const float* __restrict__ logits, int k, SceneAxis ay,
+                                                          SceneAxis ax, int t0, int t1, int y0, int x0, int bh, int bw,
+                                                          int d, int first_pass, float* __restrict__ acc,
+                                                          float* __restrict__ wsum) {
+  constexpr int KM = KT > 0 ? KT : kSceneMaxClasses;
+  const int K = KT > 0 ? KT : k;
+  const long long hw = static_cast<long long>(ay.len) * ax.len;
+  const long long tile_px = static_cast<long long>(ay.ext) * ax.ext;
+  auto gy = [&](int t) { return window(t, ay.ext); };
+  auto gx = [&](int t) { return window(t, ax.ext); };
+  if constexpr (!S) {
+    const long long total = static_cast<long long>(bh) * bw;
+    for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+         i += static_cast<long long>(gridDim.x) * blockDim.x) {
+      const int Y = y0 + static_cast<int>(i / bw), X = x0 + static_cast<int>(i % bw);
+      PixelCover cv;
+      if (!batch_cover(ay, ax, Y, X, t0, t1, cv)) continue;
+      const bool fresh = cv.fresh && first_pass;
+      const long long p = static_cast<long long>(Y) * ax.len + X;
+      float a[KM];
+      float ws = 0.f;
+#pragma unroll
+      for (int c = 0; c < KM; ++c) a[c] = (c < K && !fresh) ? acc[c * hw + p] : 0.f;
+      if (!fresh) ws = wsum[p];
+      const bool any = visit_batch_tiles(ay, ax, Y, X, t0, t1, cv, gy, gx, [&](int b, int ty, int tx, float w) {
+        const float* lg = logits + b * K * tile_px + tta_offset(d, ty, tx, ay.ext, ax.ext);
+        blend_tile<KT>([&](int c) { return __ldg(lg + c * tile_px); }, K, w, a);
+        ws += w;
+      });
+      if (!any) continue;
+#pragma unroll
+      for (int c = 0; c < KM; ++c)
+        if (c < K) acc[c * hw + p] = a[c];
+      wsum[p] = ws;
+    }
+  } else {
+    __shared__ float sz[KM][16][17];                   // [class][box row][box column] of one tile's logits
+    const int lo = threadIdx.x & 15, hi = threadIdx.x >> 4;
+    const int bxn = (bw + 15) / 16, n_box = ((bh + 15) / 16) * bxn;
+    for (int q = blockIdx.x; q < n_box; q += gridDim.x) {             // uniform per CTA
+      const int by0 = y0 + (q / bxn) * 16, bx0 = x0 + (q % bxn) * 16;
+      const int Y = by0 + hi, X = bx0 + lo;                            // this thread's pixel
+      PixelCover cv;
+      const bool mine = Y < y0 + bh && X < x0 + bw && batch_cover(ay, ax, Y, X, t0, t1, cv);
+      const bool fresh = mine && cv.fresh && first_pass;
+      const long long p = static_cast<long long>(Y) * ax.len + X;
+      float a[KM];
+      float ws = 0.f;
+#pragma unroll
+      for (int c = 0; c < KM; ++c) a[c] = (mine && c < K && !fresh) ? acc[c * hw + p] : 0.f;
+      if (mine && !fresh) ws = wsum[p];
+      bool any = false;
+      // the tiles that cover some pixel of the box: contiguous ranges per axis
+      int tya, tyb, txa, txb, dummy;
+      axis_cover(ay, by0, tya, dummy);
+      axis_cover(ay, min(by0 + 15, ay.len - 1), dummy, tyb);
+      axis_cover(ax, bx0, txa, dummy);
+      axis_cover(ax, min(bx0 + 15, ax.len - 1), dummy, txb);
+      // the copy: consecutive threads on consecutive rows of the box
+      const int LY = by0 + lo, LX = bx0 + hi;
+      for (int ty = tya; ty <= tyb; ++ty) {
+        const int row = ty * ax.n;
+        const int xa = max(txa, t0 - row), xb = min(txb, t1 - 1 - row);
+        for (int tx = xa; tx <= xb; ++tx) {
+          const int b = row + tx - t0;
+          const int oy = axis_origin(ay, ty), ox = axis_origin(ax, tx);
+          __syncthreads();                             // the previous tile's reads of sz are done
+          if (LY < ay.len && LX < ax.len && LY >= oy && LY < oy + ay.ext && LX >= ox && LX < ox + ax.ext) {
+            const float* lg = logits + b * K * tile_px + tta_offset(d, LY - oy, LX - ox, ay.ext, ax.ext);
+#pragma unroll
+            for (int c = 0; c < KM; ++c)
+              if (c < K) sz[c][lo][hi] = __ldg(lg + c * tile_px);
+          }
+          __syncthreads();
+          if (mine && Y >= oy && Y < oy + ay.ext && X >= ox && X < ox + ax.ext) {
+            const float w = gy(Y - oy) * gx(X - ox);
+            blend_tile<KT>([&](int c) { return sz[c][hi][lo]; }, K, w, a);
+            ws += w;
+            any = true;
+          }
+        }
+      }
+      if (!any) continue;
+#pragma unroll
+      for (int c = 0; c < KM; ++c)
+        if (c < K) acc[c * hw + p] = a[c];
+      wsum[p] = ws;
+    }
   }
 }
 
@@ -414,13 +541,16 @@ static inline SceneBox scene_batch_box(const SceneAxis& ay, const SceneAxis& ax,
   return SceneBox{t0, t1, y0, x0, y1 - y0, x1 - x0};
 }
 
-template <int NIMG>
+template <int NIMG, bool S>
 static void scene_gather_launch(const void* img1, const void* img2, int src_u8, int c, const SceneAxis& ay,
-                                const SceneAxis& ax, int tile0, int batch, void* out1, void* out2, cudaStream_t st) {
+                                const SceneAxis& ax, int tile0, int batch, int d, void* out1, void* out2,
+                                cudaStream_t st) {
+  // one thread per output pixel, or (S) one CTA of 256 threads per 16 x 16 square: the same CTA count
   const int grid = scene_grid(static_cast<long long>(ay.ext) * ax.ext * batch, 148 * 8);
   bf16* o1 = static_cast<bf16*>(out1);
   bf16* o2 = static_cast<bf16*>(out2);
-#define GATHER(CC, U) scene_gather_kernel<CC, U, NIMG><<<grid, 256, 0, st>>>(img1, img2, ay, ax, tile0, batch, o1, o2)
+#define GATHER(CC, U) \
+  scene_gather_kernel<CC, U, NIMG, S><<<grid, 256, 0, st>>>(img1, img2, ay, ax, tile0, batch, d, o1, o2)
   if (src_u8) {
     switch (c) {
       case 1: GATHER(1, true); break;
@@ -445,38 +575,68 @@ using namespace gap;
 
 extern "C" {
 
-int gap_scene_gather(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy,
-                     int sx, int ny, int nx, int tile0, int batch, void* out1, void* out2, void* stream) {
+int gap_scene_gather_tta(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy,
+                         int sx, int ny, int nx, int tile0, int batch, int d, void* out1, void* out2, void* stream) {
   GAP_CHECK_ARG(c >= 1 && c <= 4, "gap_scene_gather: c must be 1..4, got %d", c);
+  GAP_CHECK_ARG(d >= 0 && d <= 7, "gap_scene_gather: d must be 0..7, got %d", d);
   const SceneAxis ay{h, ey, sy, ny}, ax{w, ex, sx, nx};
   GAP_CHECK_ARG(img1 && img2 && out1 && out2 && scene_axis_ok(ay) && scene_axis_ok(ax) && batch >= 1 && tile0 >= 0 &&
                     tile0 < ny * nx,
                 "gap_scene_gather: bad arguments");
   GAP_CHECK_ARG((reinterpret_cast<uintptr_t>(out1) & 7) == 0 && (reinterpret_cast<uintptr_t>(out2) & 7) == 0,
                 "gap_scene_gather: out1 / out2 must be 8-byte aligned (one 8-byte store per 4-slot pixel)");
-  scene_gather_launch<2>(img1, img2, src_u8, c, ay, ax, tile0, batch, out1, out2, static_cast<cudaStream_t>(stream));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (d & 4)
+    scene_gather_launch<2, true>(img1, img2, src_u8, c, ay, ax, tile0, batch, d, out1, out2, st);
+  else
+    scene_gather_launch<2, false>(img1, img2, src_u8, c, ay, ax, tile0, batch, d, out1, out2, st);
   GAP_CUDA(cudaGetLastError());
   return 0;
 }
 
-int gap_scene_blend(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx, int tile0,
-                    int batch, float* acc, float* wsum, void* stream) {
+int gap_scene_gather(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy,
+                     int sx, int ny, int nx, int tile0, int batch, void* out1, void* out2, void* stream) {
+  return gap_scene_gather_tta(img1, img2, src_u8, c, h, w, ey, ex, sy, sx, ny, nx, tile0, batch, 0, out1, out2, stream);
+}
+
+int gap_scene_blend_tta(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx,
+                        int tile0, int batch, int d, int first_pass, float* acc, float* wsum, void* stream) {
   GAP_CHECK_ARG(k >= 1 && k <= kSceneMaxClasses, "gap_scene_blend: k must be 1..16, got %d", k);
+  GAP_CHECK_ARG(d >= 0 && d <= 7, "gap_scene_blend: d must be 0..7, got %d", d);
   const SceneAxis ay{h, ey, sy, ny}, ax{w, ex, sx, nx};
   GAP_CHECK_ARG(logits && acc && wsum && scene_axis_ok(ay) && scene_axis_ok(ax) && batch >= 1 && tile0 >= 0 &&
                     tile0 < ny * nx,
                 "gap_scene_blend: bad arguments");
   const SceneBox bx = scene_batch_box(ay, ax, tile0, batch);
   const int t0 = bx.t0, t1 = bx.t1, y0 = bx.y0, x0 = bx.x0, bh = bx.bh, bw = bx.bw;
-  const int grid = scene_grid(static_cast<long long>(bh) * bw, 148 * 8);
+  const int fp = first_pass ? 1 : 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  switch (k) {
-    case 1: scene_blend_kernel<1><<<grid, 256, 0, st>>>(logits, k, ay, ax, t0, t1, y0, x0, bh, bw, acc, wsum); break;
-    case 2: scene_blend_kernel<2><<<grid, 256, 0, st>>>(logits, k, ay, ax, t0, t1, y0, x0, bh, bw, acc, wsum); break;
-    default: scene_blend_kernel<0><<<grid, 256, 0, st>>>(logits, k, ay, ax, t0, t1, y0, x0, bh, bw, acc, wsum); break;
+  if (d & 4) {        // one CTA per 16 x 16 box of pixels
+    const int grid = static_cast<int>(std::min<long long>(static_cast<long long>((bh + 15) / 16) * ((bw + 15) / 16),
+                                                          148 * 8));
+#define BLEND(KK, SS) \
+  scene_blend_kernel<KK, SS><<<grid, 256, 0, st>>>(logits, k, ay, ax, t0, t1, y0, x0, bh, bw, d, fp, acc, wsum)
+    switch (k) {
+      case 1: BLEND(1, true); break;
+      case 2: BLEND(2, true); break;
+      default: BLEND(0, true); break;
+    }
+  } else {
+    const int grid = scene_grid(static_cast<long long>(bh) * bw, 148 * 8);
+    switch (k) {
+      case 1: BLEND(1, false); break;
+      case 2: BLEND(2, false); break;
+      default: BLEND(0, false); break;
+    }
+#undef BLEND
   }
   GAP_CUDA(cudaGetLastError());
   return 0;
+}
+
+int gap_scene_blend(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx, int tile0,
+                    int batch, float* acc, float* wsum, void* stream) {
+  return gap_scene_blend_tta(logits, k, h, w, ey, ex, sy, sx, ny, nx, tile0, batch, 0, 1, acc, wsum, stream);
 }
 
 int gap_scene_finalize(float* acc, const float* wsum, int k, int64_t pixels, uint8_t* pred, int write_probs,
@@ -505,7 +665,8 @@ int gap_scene_gather_one(const void* img, int src_u8, int c, int h, int w, int e
                 "gap_scene_gather_one: bad arguments");
   GAP_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 7) == 0,
                 "gap_scene_gather_one: out must be 8-byte aligned (one 8-byte store per 4-slot pixel)");
-  scene_gather_launch<1>(img, nullptr, src_u8, c, ay, ax, tile0, batch, out, nullptr, static_cast<cudaStream_t>(stream));
+  scene_gather_launch<1, false>(img, nullptr, src_u8, c, ay, ax, tile0, batch, 0, out, nullptr,
+                                static_cast<cudaStream_t>(stream));
   GAP_CUDA(cudaGetLastError());
   return 0;
 }

@@ -564,8 +564,24 @@ class SiameseUNet(_NativeModule):
         return _SiameseFn.apply(self, x1, x2, *self.parameters())
 
     def predict_scene(self, img1, img2, tile=256, overlap=64, batch=8, return_probs=False, labels=None,
-                      ignore_index=-100):
-        """Sliding-window change map of a whole scene at its own resolution (SiameseEngine.predict_scene): always in
-        eval mode, whatever mode the module is in; no autograd.  Returns a siamese.SceneResult(pred, probs, confusion)."""
+                      ignore_index=-100, tta=None):
+        """Sliding-window change map of a whole scene at its own resolution (SiameseEngine.predict_scene; tta: None,
+        "flips" or "d4" test-time augmentation): always in eval mode, whatever mode the module is in; no autograd.
+        Returns a siamese.SceneResult(pred, probs, confusion)."""
         return self._engine().predict_scene(img1, img2, tile=tile, overlap=overlap, batch=batch,
-                                            return_probs=return_probs, labels=labels, ignore_index=ignore_index)
+                                            return_probs=return_probs, labels=labels, ignore_index=ignore_index,
+                                            tta=tta)
+
+
+def predict_scene_ensemble(modules, img1, img2, tile=256, overlap=64, batch=8, tta=None, return_probs=False,
+                           labels=None, ignore_index=-100):
+    """Sliding-window change map of a whole scene averaged over several SiameseUNet modules (a checkpoint ensemble)
+    and, with tta = "flips" / "d4", over flipped / rotated tiles (siamese.predict_scene_ensemble): always in eval mode,
+    whatever mode each module is in; no autograd.  Returns a siamese.SceneResult(pred, probs, confusion)."""
+    from .siamese import predict_scene_ensemble as ensemble
+    if isinstance(modules, nn.Module) or not isinstance(modules, (list, tuple)) or not modules:
+        raise ValueError(f"modules must be a non-empty list of SiameseUNet, got {modules!r}")
+    if not all(isinstance(m, SiameseUNet) for m in modules):
+        raise ValueError(f"modules must all be SiameseUNet, got {[type(m).__name__ for m in modules]}")
+    return ensemble([m._engine() for m in modules], img1, img2, tile=tile, overlap=overlap, batch=batch, tta=tta,
+                    return_probs=return_probs, labels=labels, ignore_index=ignore_index)

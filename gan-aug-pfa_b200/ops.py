@@ -8,7 +8,7 @@ from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Optional, Sequence
+from typing import Optional, Sequence, Tuple
 
 import torch
 
@@ -1021,11 +1021,22 @@ def _scene_input(x: torch.Tensor, c: int, h: int, w: int, what: str, name: str) 
                      f"{x.dtype} {tuple(x.shape)}")
 
 
-def scene_gather(img1: torch.Tensor, img2: torch.Tensor, grid, tile0: int, out1: torch.Tensor, out2: torch.Tensor) -> None:
+def _tta_extent(d, ey: int, ex: int, what: str) -> Tuple[int, int]:
+    """The extent of the dihedral transform d (0..7, d = 4 s + 2 v + u) of an [ey, ex] tile: [ex, ey] when s = 1."""
+    if isinstance(d, bool) or not isinstance(d, int) or not 0 <= d <= 7:
+        raise ValueError(f"{what}: d must be an int in 0..7, got {d!r}")
+    return (ex, ey) if d & 4 else (ey, ex)
+
+
+def scene_gather(img1: torch.Tensor, img2: torch.Tensor, grid, tile0: int, out1: torch.Tensor, out2: torch.Tensor,
+                 d: int = 0) -> None:
     """Tiles tile0 .. tile0 + batch - 1 of both scenes (uint8 [H, W, C] normalised as dataset.py does, or fp32 [C, H, W]
-    rounded to bf16) -> out1 / out2, dense NHWC bf16 [batch, E_y, E_x, 4]; slots >= C and tiles past the grid are zero."""
+    rounded to bf16) -> out1 / out2, dense NHWC bf16 [batch, E_y, E_x, 4]; slots >= C and tiles past the grid are zero.
+    d (0..7): each tile is replaced by its dihedral transform d = 4 s + 2 v + u (transposed if s, then rows flipped if
+    v, then columns flipped if u), so out1 / out2 are [batch, E_x, E_y, 4] when s = 1."""
     what = "scene_gather"
     h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    oy, ox = _tta_extent(d, ey, ex, what)
     c = img1.shape[-1] if img1.dtype == torch.uint8 else img1.shape[0]
     if not 1 <= c <= 4:
         raise ValueError(f"{what}: scenes of 1 to 4 channels are supported, got {c}")
@@ -1034,28 +1045,34 @@ def scene_gather(img1: torch.Tensor, img2: torch.Tensor, grid, tile0: int, out1:
         raise ValueError(f"{what}: img1 and img2 must have the same dtype")
     batch = out1.shape[0]
     for name, o in (("out1", out1), ("out2", out2)):
-        if o.dtype != torch.bfloat16 or tuple(o.shape) != (batch, ey, ex, 4) or not o.is_contiguous():
-            raise ValueError(f"{what}: {name} must be a contiguous bf16 [batch, {ey}, {ex}, 4] tensor, got "
+        if o.dtype != torch.bfloat16 or tuple(o.shape) != (batch, oy, ox, 4) or not o.is_contiguous():
+            raise ValueError(f"{what}: {name} must be a contiguous bf16 [batch, {oy}, {ox}, 4] tensor, got "
                              f"{o.dtype} {tuple(o.shape)}")
         if o.data_ptr() % 8:
             raise ValueError(f"{what}: {name} must be 8-byte aligned (each 4-slot pixel is one 8-byte store)")
     if not 0 <= tile0 < ny * nx:
         raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
     _cuda(what, img1, img2, out1, out2)
-    _lib.check(_lib.lib().gap_scene_gather(_ptr(img1), _ptr(img2), int(u8), c, h, w, ey, ex, sy, sx, ny, nx, int(tile0),
-                                           batch, _ptr(out1), _ptr(out2), _stream()), "gap_scene_gather")
+    _lib.check(_lib.lib().gap_scene_gather_tta(_ptr(img1), _ptr(img2), int(u8), c, h, w, ey, ex, sy, sx, ny, nx,
+                                               int(tile0), batch, d, _ptr(out1), _ptr(out2), _stream()),
+               "gap_scene_gather_tta")
 
 
-def scene_blend(logits: torch.Tensor, grid, tile0: int, acc: torch.Tensor, wsum: torch.Tensor) -> None:
+def scene_blend(logits: torch.Tensor, grid, tile0: int, acc: torch.Tensor, wsum: torch.Tensor, d: int = 0,
+                first_pass: bool = True) -> None:
     """Window-weighted probabilities of one batch of tile logits (fp32 [batch, E_y, E_x] for K = 1, [batch, K, E_y, E_x]
-    for K > 1) -> acc [K, H, W] += w * p, wsum [H, W] += w (fp32) at every scene pixel the batch covers."""
+    for K > 1) -> acc [K, H, W] += w * p, wsum [H, W] += w (fp32) at every scene pixel the batch covers.
+    d (0..7): the logits are those of scene_gather(..., d)'s transformed tiles ([.., E_x, E_y] when d >= 4) and are
+    mapped back by the inverse transform.  first_pass: a pixel's sums may start from zero at its first covering tile
+    (the accumulators need no clearing); False for every later pass over the grid, which adds onto acc / wsum."""
     what = "scene_blend"
     h, w, ey, ex, sy, sx, ny, nx = _scene_grid_args(grid, what)
+    oy, ox = _tta_extent(d, ey, ex, what)
     k = 1 if logits.dim() == 3 else (logits.shape[1] if logits.dim() == 4 else -1)
     _check_k(k, what)
     batch = logits.shape[0]
-    if logits.dtype != torch.float32 or not logits.is_contiguous() or tuple(logits.shape[-2:]) != (ey, ex):
-        raise ValueError(f"{what}: logits must be contiguous fp32 [batch, (K,) {ey}, {ex}], got {logits.dtype} "
+    if logits.dtype != torch.float32 or not logits.is_contiguous() or tuple(logits.shape[-2:]) != (oy, ox):
+        raise ValueError(f"{what}: logits must be contiguous fp32 [batch, (K,) {oy}, {ox}], got {logits.dtype} "
                          f"{tuple(logits.shape)}")
     if acc.dtype != torch.float32 or tuple(acc.shape) != (k, h, w) or not acc.is_contiguous():
         raise ValueError(f"{what}: acc must be a contiguous fp32 [{k}, {h}, {w}] tensor")
@@ -1064,8 +1081,9 @@ def scene_blend(logits: torch.Tensor, grid, tile0: int, acc: torch.Tensor, wsum:
     if not 0 <= tile0 < ny * nx:
         raise ValueError(f"{what}: tile0 = {tile0} outside the {ny * nx} tiles of the grid")
     _cuda(what, logits, acc, wsum)
-    _lib.check(_lib.lib().gap_scene_blend(_ptr(logits), k, h, w, ey, ex, sy, sx, ny, nx, int(tile0), batch, _ptr(acc),
-                                          _ptr(wsum), _stream()), "gap_scene_blend")
+    _lib.check(_lib.lib().gap_scene_blend_tta(_ptr(logits), k, h, w, ey, ex, sy, sx, ny, nx, int(tile0), batch, d,
+                                              int(bool(first_pass)), _ptr(acc), _ptr(wsum), _stream()),
+               "gap_scene_blend_tta")
 
 
 def scene_finalize(acc: torch.Tensor, wsum: torch.Tensor, pred: torch.Tensor, write_probs: bool,

@@ -492,7 +492,7 @@ class SiameseEngine(_Net):
     @_on_device
     def predict_scene(self, img1: torch.Tensor, img2: torch.Tensor, tile: int = 256, overlap: int = 64, batch: int = 8,
                       return_probs: bool = False, labels: Optional[torch.Tensor] = None,
-                      ignore_index: int = -100) -> SceneResult:
+                      ignore_index: int = -100, tta: Optional[str] = None) -> SceneResult:
         """A change map of a whole scene of any size at its own resolution, by sliding-window inference.
 
         img1, img2: the two images of the scene, either uint8 [H, W, C] as PIL / numpy give them (host or device;
@@ -507,57 +507,22 @@ class SiameseEngine(_Net):
         p = sum_tiles w * p_tile / sum_tiles w, summed in ascending tile index, so the result does not depend on
         `batch`.  pred is the argmax of p (ties to the lowest class) or, for K = 1, p > 0.5.
 
+        tta: test-time augmentation, None, "flips" or "d4" (predict_scene_ensemble): every tile also runs flipped
+        (and, for "d4", transposed), each output is mapped back, and the probabilities of all passes are averaged.
+
         return_probs: also return p (fp32 [K, H, W]).  labels (int64 [H, W]): also return the confusion counts of pred
         against them at full resolution: [K, K] (rows = label; metrics.multiclass_metrics takes it) or, for K = 1,
         [TP, FP, FN, TN] (metrics.metrics_from_counts); pixels labelled ignore_index or outside [0, K) ({0, 1} for
         K = 1) are not counted.
 
         Memory: (K + 1) * 4 bytes per scene pixel of accumulators (which become probs), and the engine's activation
-        buffers sized for `batch` tiles; like any call at a new shape this may re-allocate them.  Everything runs on
+        buffers sized for `batch` tiles; like any call at a new shape this may re-allocate them.  With tta="d4" on a
+        grid whose tiles are not square (a scene side shorter than the tile), they are re-sized once more, at the first
+        transposed pass (d = 4), to `batch` tiles of the transposed extent [E_x, E_y].  Everything runs on
         the current stream without a host synchronisation.  The `training` flag is restored afterwards and no
         parameter, gradient or BatchNorm buffer changes.  Bad arguments raise ValueError before any work is enqueued."""
-        for name, v in (("tile", tile), ("overlap", overlap), ("batch", batch)):
-            if isinstance(v, bool) or not isinstance(v, int):
-                raise ValueError(f"{name} must be an int, got {v!r}")
-        if tile < 16 or tile % 16:
-            raise ValueError(f"tile must be a multiple of 16 and at least 16, got {tile}")
-        if not 0 <= overlap < tile:
-            raise ValueError(f"overlap must be in [0, tile = {tile}), got {overlap}")
-        if batch < 1:
-            raise ValueError(f"batch must be >= 1, got {batch}")
-        u8, h, w = self._scene_input(img1, "img1")
-        if self._scene_input(img2, "img2")[0] != u8 or img2.shape != img1.shape:
-            raise ValueError(f"img1 and img2 must have the same dtype and shape, got {img1.dtype} "
-                             f"{tuple(img1.shape)} and {img2.dtype} {tuple(img2.shape)}")
-        if labels is not None and (not isinstance(labels, torch.Tensor) or labels.dtype != torch.int64
-                                   or tuple(labels.shape) != (h, w)):
-            raise ValueError(f"labels must be an int64 [{h}, {w}] tensor, got "
-                             f"{getattr(labels, 'dtype', type(labels))} {tuple(getattr(labels, 'shape', ()))}")
-        k = self.n_classes
-        grid = _scene_grid(h, w, tile, overlap)
-        (_, ey, _, ny), (_, ex, _, nx) = grid
-        img1, img2 = img1.to(self.dev).contiguous(), img2.to(self.dev).contiguous()
-        if labels is not None:
-            labels = labels.to(self.dev).contiguous()
-        acc = torch.empty(k, h, w, device=self.dev)              # every pixel is written by the batch of its first tile
-        wsum = torch.empty(h, w, device=self.dev)
-        pred = torch.empty(h, w, device=self.dev, dtype=torch.uint8)
-        conf = None
-        if labels is not None:
-            conf = torch.zeros((4,) if k == 1 else (k, k), device=self.dev, dtype=torch.int64)
-        was = self.training
-        self.training = False
-        try:
-            self._alloc(batch, ey, ex)
-            for t0 in range(0, ny * nx, batch):                 # the last batch is padded with zero tiles
-                ops.scene_gather(img1, img2, grid, t0, self.x_in[0], self.x_in[1])
-                self._forward_from((None, None))
-                ops.scene_blend(self.logits, grid, t0, acc, wsum)
-            ops.scene_finalize(acc, wsum, pred, return_probs, labels, ignore_index, conf)
-        finally:
-            self.training = was
-            self._tape = []
-        return SceneResult(pred, acc if return_probs else None, conf)
+        return predict_scene_ensemble([self], img1, img2, tile=tile, overlap=overlap, batch=batch, tta=tta,
+                                      return_probs=return_probs, labels=labels, ignore_index=ignore_index)
 
     # -- backward --------------------------------------------------------------------------------------
     @_on_device
@@ -733,3 +698,104 @@ class GateEngine(SiameseEngine):
         for fn in reversed(self._tape):
             fn()
         self._tape = []
+
+
+TTA_TRANSFORMS = {None: (0,), "flips": (0, 1, 2, 3), "d4": tuple(range(8))}
+
+
+def predict_scene_ensemble(engines, img1: torch.Tensor, img2: torch.Tensor, tile: int = 256, overlap: int = 64,
+                           batch: int = 8, tta: Optional[str] = None, return_probs: bool = False,
+                           labels: Optional[torch.Tensor] = None, ignore_index: int = -100) -> SceneResult:
+    """SiameseEngine.predict_scene averaged over test-time augmentation and over several networks (a checkpoint
+    ensemble): the same inputs, tile grid, window and SceneResult, with p the mean of the blended probabilities of
+    every pass.
+
+    engines: one or more SiameseEngines on the same device with the same n_channels and n_classes, equally weighted.
+    tta: None (each tile as it is), "flips" (also flipped along rows, columns and both) or "d4" (the eight symmetries
+    of the square: the flips, and the tile transposed, then flipped).  Transform d = 4 s + 2 v + u transposes the tile
+    if s, then flips its rows if v, then its columns if u; the network's logits are mapped back by the inverse, and
+    probabilities (softmax, K = 1: sigmoid), not logits, are averaged.
+
+    A pass is one (network, transform) pair; the passes run network by network in list order and, within a network,
+    in ascending d, each over all tiles in ascending index.  Per pixel acc = sum_passes sum_tiles w * p_tile and
+    wsum = sum_passes sum_tiles w are summed in that order in fp32 and p = acc / wsum: deterministic and independent of
+    `batch`.  One network without tta is exactly predict_scene.
+
+    Memory: as predict_scene; a host scene is copied to the device once for all passes.  For tta="d4" on a grid whose
+    tiles are not square (a scene side shorter than the tile), each network's activation buffers are re-sized once, at
+    the first transposed pass, to `batch` tiles of the transposed extent.  No host synchronisation; every network's
+    `training` flag is restored and no parameter, gradient or BatchNorm buffer changes.  Bad arguments raise
+    ValueError before any work is enqueued."""
+    if isinstance(engines, SiameseEngine) or not isinstance(engines, (list, tuple)) or not engines:
+        raise ValueError(f"engines must be a non-empty list of SiameseEngine, got {engines!r}")
+    if not all(isinstance(e, SiameseEngine) for e in engines):
+        raise ValueError("engines must all be SiameseEngine instances, got "
+                         f"{[type(e).__name__ for e in engines]}")
+    lead = engines[0]
+    for e in engines[1:]:
+        if (e.dev, e.n_channels, e.n_classes) != (lead.dev, lead.n_channels, lead.n_classes):
+            raise ValueError("ensemble members must share device, n_channels and n_classes, got "
+                             f"{(lead.dev, lead.n_channels, lead.n_classes)} and {(e.dev, e.n_channels, e.n_classes)}")
+    if not isinstance(tta, (str, type(None))) or tta not in TTA_TRANSFORMS:
+        raise ValueError(f"tta must be None, 'flips' or 'd4', got {tta!r}")
+    for name, v in (("tile", tile), ("overlap", overlap), ("batch", batch)):
+        if isinstance(v, bool) or not isinstance(v, int):
+            raise ValueError(f"{name} must be an int, got {v!r}")
+    if tile < 16 or tile % 16:
+        raise ValueError(f"tile must be a multiple of 16 and at least 16, got {tile}")
+    if not 0 <= overlap < tile:
+        raise ValueError(f"overlap must be in [0, tile = {tile}), got {overlap}")
+    if batch < 1:
+        raise ValueError(f"batch must be >= 1, got {batch}")
+    u8, h, w = lead._scene_input(img1, "img1")
+    if lead._scene_input(img2, "img2")[0] != u8 or img2.shape != img1.shape:
+        raise ValueError(f"img1 and img2 must have the same dtype and shape, got {img1.dtype} "
+                         f"{tuple(img1.shape)} and {img2.dtype} {tuple(img2.shape)}")
+    if labels is not None and (not isinstance(labels, torch.Tensor) or labels.dtype != torch.int64
+                               or tuple(labels.shape) != (h, w)):
+        raise ValueError(f"labels must be an int64 [{h}, {w}] tensor, got "
+                         f"{getattr(labels, 'dtype', type(labels))} {tuple(getattr(labels, 'shape', ()))}")
+    idx = lead.dev.index
+    if idx is None or torch.cuda.current_device() == idx:
+        return _predict_scene_passes(engines, img1, img2, tile, overlap, batch, TTA_TRANSFORMS[tta], return_probs,
+                                     labels, ignore_index)
+    with torch.cuda.device(idx):
+        return _predict_scene_passes(engines, img1, img2, tile, overlap, batch, TTA_TRANSFORMS[tta], return_probs,
+                                     labels, ignore_index)
+
+
+def _predict_scene_passes(engines, img1, img2, tile, overlap, batch, transforms, return_probs, labels,
+                          ignore_index) -> SceneResult:
+    """predict_scene_ensemble after its argument checks, with the members' device current."""
+    lead = engines[0]
+    dev, k = lead.dev, lead.n_classes
+    h, w = (img1.shape[:2] if img1.dtype == torch.uint8 else img1.shape[1:])
+    grid = _scene_grid(h, w, tile, overlap)
+    (_, ey, _, ny), (_, ex, _, nx) = grid
+    img1, img2 = img1.to(dev).contiguous(), img2.to(dev).contiguous()
+    if labels is not None:
+        labels = labels.to(dev).contiguous()
+    acc = torch.empty(k, h, w, device=dev)                   # every pixel is written by the batch of its first tile
+    wsum = torch.empty(h, w, device=dev)
+    pred = torch.empty(h, w, device=dev, dtype=torch.uint8)
+    conf = None
+    if labels is not None:
+        conf = torch.zeros((4,) if k == 1 else (k, k), device=dev, dtype=torch.int64)
+    was = [e.training for e in engines]
+    first = True
+    try:
+        for eng in engines:
+            eng.training = False
+            for d in transforms:
+                eng._alloc(batch, *((ex, ey) if d & 4 else (ey, ex)))
+                for t0 in range(0, ny * nx, batch):             # the last batch is padded with zero tiles
+                    ops.scene_gather(img1, img2, grid, t0, eng.x_in[0], eng.x_in[1], d)
+                    eng._forward_from((None, None))
+                    ops.scene_blend(eng.logits, grid, t0, acc, wsum, d, first)
+                first = False
+        ops.scene_finalize(acc, wsum, pred, return_probs, labels, ignore_index, conf)
+    finally:
+        for eng, t in zip(engines, was):
+            eng.training = t
+            eng._tape = []
+    return SceneResult(pred, acc if return_probs else None, conf)

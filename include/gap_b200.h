@@ -384,12 +384,22 @@ int gap_seg_confusion_ck(const float* logits, const int64_t* labels, int k, int 
  *   out1 / out2 must be 8-byte aligned: each 4-slot pixel is one 8-byte store. */
 int gap_scene_gather(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy, int sx,
                      int ny, int nx, int tile0, int batch, void* out1, void* out2, void* stream);
+/* gather_tta: the same for the dihedral transform d = 4s + 2v + u (0..7) of every tile: transposed if s, then rows
+ *   flipped if v, then columns flipped if u.  out1 / out2 are [batch][ex][ey][4 slots] when s = 1.  d = 0 is
+ *   gap_scene_gather. */
+int gap_scene_gather_tta(const void* img1, const void* img2, int src_u8, int c, int h, int w, int ey, int ex, int sy,
+                         int sx, int ny, int nx, int tile0, int batch, int d, void* out1, void* out2, void* stream);
 /* blend: logits fp32 [batch][k][ey][ex] (k = 1: sigmoid, else softmax over the k planes) of tiles tile0 .. -> for every
  * scene pixel, over the covering tiles of this batch in ascending index: acc[c][pixel] += w * p_c, wsum[pixel] += w
  * (fp32 [k][h][w] and [h][w]).  A pixel whose first covering tile of the grid is in this batch starts from zero, so the
  * accumulators need no clearing when the batches run in order.  No floating-point atomics: deterministic. */
 int gap_scene_blend(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx, int tile0,
                     int batch, float* acc, float* wsum, void* stream);
+/* blend_tta: the same for logits of the transformed tiles of gap_scene_gather_tta (d = 0..7; [batch][k][ex][ey] when
+ *   s = 1), each mapped back by the inverse transform.  Only when first_pass != 0 may a pixel start from zero; later
+ *   passes (other transforms, other networks) always add onto acc / wsum.  d = 0, first_pass = 1 is gap_scene_blend. */
+int gap_scene_blend_tta(const float* logits, int k, int h, int w, int ey, int ex, int sy, int sx, int ny, int nx,
+                        int tile0, int batch, int d, int first_pass, float* acc, float* wsum, void* stream);
 /* finalize: p = acc / wsum over `pixels`; pred (uint8) = argmax_c p (ties to the lowest class) or, k = 1, p > 0.5;
  * write_probs: acc is overwritten with p.  labels (int64, optional, with counts): counts += k > 1 ? [label][pred] (k*k)
  * : [TP, FP, FN, TN] (label 1 positive, 0 negative); ignore_index and labels outside [0, k) ({0, 1} for k = 1) are not

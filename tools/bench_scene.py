@@ -10,7 +10,14 @@
    the other benches use;
 4. the device name and enforced power limit, read from NVML in the same run.
 
-    python tools/bench_scene.py [--calls 5] [--out FILE]
+With --tta flips / d4 or --members N > 1 it measures test-time augmentation and checkpoint ensembles
+(siamese.predict_scene_ensemble) instead, on the same pair, K = 2, tile 512 / batch 4 and tile 256 / batch 16, overlap
+64, with N differently seeded members: the whole call (median of --calls after a warm-up), its ratio to passes x the
+tta=None one-member call measured in the same run, and one instrumented call with the gather and blend times, bytes
+and GB/s split into the passes with untransposed (s = 0) and transposed (s = 1) tiles.  A later pass reads the
+accumulators wherever its batch covers them (no pixel starts from zero again).
+
+    python tools/bench_scene.py [--calls 5] [--tta none|flips|d4] [--members N] [--out FILE]
 """
 from __future__ import annotations
 
@@ -27,11 +34,13 @@ ROOT = Path(__file__).resolve().parents[1]
 sys.path.insert(0, str(ROOT))
 
 from gan_aug_pfa_b200 import ops, spec  # noqa: E402
-from gan_aug_pfa_b200.siamese import SiameseEngine, _scene_grid, scene_axis  # noqa: E402
+from gan_aug_pfa_b200.siamese import (TTA_TRANSFORMS, SiameseEngine, _scene_grid, predict_scene_ensemble,  # noqa: E402
+                                      scene_axis)
 
 ROOF_GBS = 6527.0
 SIZE = 8192
 CONFIGS = ((512, 4, 0), (512, 4, 64), (256, 16, 0), (256, 16, 64))       # (tile, batch, overlap)
+TTA_CONFIGS = ((512, 4, 64), (256, 16, 64))
 
 
 def device_info() -> dict:
@@ -49,9 +58,10 @@ def _cells(origins, ext, length):
     return np.diff(b), [(b.index(o), b.index(min(o + ext, length))) for o in origins]
 
 
-def blend_bytes(h: int, w: int, tile: int, overlap: int, batch: int, k: int) -> int:
-    """Bytes the blend must move over a whole call: logits of every real tile, plus per batch the accumulators
-    ((K + 1) * 4 B per pixel) written where the batch covers and read where an earlier batch started them."""
+def blend_bytes(h: int, w: int, tile: int, overlap: int, batch: int, k: int, first_pass: bool = True) -> int:
+    """Bytes the blend must move over a whole pass: logits of every real tile, plus per batch the accumulators
+    ((K + 1) * 4 B per pixel) written where the batch covers and read where an earlier batch started them (in a later
+    pass: wherever the batch covers)."""
     oy, ey = scene_axis(h, tile, overlap)
     ox, ex = scene_axis(w, tile, overlap)
     dy, ry = _cells(oy, ey, h)
@@ -68,7 +78,7 @@ def blend_bytes(h: int, w: int, tile: int, overlap: int, batch: int, k: int) -> 
         for (y0, y1), (x0, x1) in tiles[t0:t0 + batch]:
             touched[y0:y1, x0:x1] = True
         total += int(area[touched].sum()) * (k + 1) * 4
-        total += int(area[touched & (first < t0)].sum()) * (k + 1) * 4
+        total += int(area[touched & (first < t0) if first_pass else touched].sum()) * (k + 1) * 4
     return total
 
 
@@ -163,14 +173,119 @@ def run(calls: int) -> list:
     return rows
 
 
+def timed_passes(engines, img1, img2, tile, overlap, batch, transforms) -> dict:
+    """predict_scene_ensemble's passes with CUDA events around each gather and blend, summed per kind of pass."""
+    h, w = img1.shape[:2]
+    k = engines[0].n_classes
+    grid = _scene_grid(h, w, tile, overlap)
+    (_, ey, _, ny), (_, ex, _, nx) = grid
+    acc = torch.empty(k, h, w, device=img1.device)
+    wsum = torch.empty(h, w, device=img1.device)
+    pred = torch.empty(h, w, device=img1.device, dtype=torch.uint8)
+    ev = {"gather_s0": [], "gather_s1": [], "blend_s0": [], "blend_s1": [], "finalize": []}
+
+    def rec(name, fn):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fn()
+        e1.record()
+        ev[name].append((e0, e1))
+
+    first = True
+    for eng in engines:
+        eng.training = False
+        for d in transforms:
+            s = "s1" if d & 4 else "s0"
+            eng._alloc(batch, *((ex, ey) if d & 4 else (ey, ex)))
+            for t0 in range(0, ny * nx, batch):
+                rec("gather_" + s, lambda: ops.scene_gather(img1, img2, grid, t0, eng.x_in[0], eng.x_in[1], d))
+                eng._forward_from((None, None))
+                rec("blend_" + s, lambda: ops.scene_blend(eng.logits, grid, t0, acc, wsum, d, first))
+            first = False
+        eng._tape = []
+    rec("finalize", lambda: ops.scene_finalize(acc, wsum, pred, False))
+    torch.cuda.synchronize()
+    return {name: sum(a.elapsed_time(b) for a, b in pairs) for name, pairs in ev.items()}
+
+
+def median_call(fn, calls: int) -> tuple:
+    fn()                                                                           # warm-up
+    torch.cuda.synchronize()
+    times = []
+    for _ in range(calls):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        fn()
+        e1.record()
+        torch.cuda.synchronize()
+        times.append(e0.elapsed_time(e1))
+    return statistics.median(times), times
+
+
+def run_tta(calls: int, tta: str, members: int) -> list:
+    dev = torch.device("cuda:0")
+    g = torch.Generator(device=dev).manual_seed(0)
+    img1 = torch.randint(0, 256, (SIZE, SIZE, 3), device=dev, generator=g, dtype=torch.uint8)
+    img2 = torch.randint(0, 256, (SIZE, SIZE, 3), device=dev, generator=g, dtype=torch.uint8)
+    k = 2
+    engines = []
+    for m in range(members):
+        torch.manual_seed(m)
+        eng = SiameseEngine(dev, 3, k)
+        eng.load_state_dict(spec.SiameseSpec(3, k).default_state_dict())
+        engines.append(eng)
+    transforms = TTA_TRANSFORMS[None if tta == "none" else tta]
+    rows = []
+    for tile, batch, overlap in TTA_CONFIGS:
+        grid = _scene_grid(SIZE, SIZE, tile, overlap)
+        (_, ey, _, ny), (_, ex, _, nx) = grid
+        n_tiles = ny * nx
+        n_batches = -(-n_tiles // batch)
+        kw = dict(tile=tile, overlap=overlap, batch=batch)
+        base_ms, _ = median_call(lambda: engines[0].predict_scene(img1, img2, **kw), calls)
+        call_ms, times = median_call(
+            lambda: predict_scene_ensemble(engines, img1, img2, tta=None if tta == "none" else tta, **kw), calls)
+        parts = timed_passes(engines, img1, img2, tile, overlap, batch, transforms)
+        n_pass = {"s0": members * sum(1 for d in transforms if d < 4), "s1": members * sum(1 for d in transforms if d >= 4)}
+        gather_pass = n_batches * batch * ey * ex * 4 * 2 * 2 + n_tiles * ey * ex * 3 * 2
+        blend_first = blend_bytes(SIZE, SIZE, tile, overlap, batch, k)
+        blend_later = blend_bytes(SIZE, SIZE, tile, overlap, batch, k, first_pass=False)
+        nbytes = {"gather_s0": n_pass["s0"] * gather_pass, "gather_s1": n_pass["s1"] * gather_pass,
+                  "blend_s0": blend_first + (n_pass["s0"] - 1) * blend_later,     # the first pass is an s = 0 one
+                  "blend_s1": n_pass["s1"] * blend_later, "finalize": SIZE * SIZE * ((k + 1) * 4 + 1)}
+        n_passes = members * len(transforms)
+        row = {"k": k, "tile": tile, "batch": batch, "overlap": overlap, "tta": tta, "members": members,
+               "passes": n_passes, "tiles": n_tiles, "call_ms_median": round(call_ms, 2),
+               "call_ms": [round(t, 2) for t in times], "tta_none_call_ms": round(base_ms, 2),
+               "call_over_passes_x_none": round(call_ms / (n_passes * base_ms), 4)}
+        for name, ms in parts.items():
+            if not nbytes[name]:
+                continue
+            passes = n_pass[name[-2:]] if name != "finalize" else 1
+            gbs = nbytes[name] / (ms * 1e-3) / 1e9
+            row[name] = {"ms": round(ms, 3), "ms_per_pass": round(ms / passes, 3), "MB": round(nbytes[name] / 1e6, 1),
+                         "GB/s": round(gbs, 1), "frac_roof": round(gbs / ROOF_GBS, 3)}
+        rows.append(row)
+        print(json.dumps(row), flush=True)
+    return rows
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--calls", type=int, default=5)
+    ap.add_argument("--tta", choices=("none", "flips", "d4"), default="none")
+    ap.add_argument("--members", type=int, default=1)
     ap.add_argument("--out", default=None)
     a = ap.parse_args()
+    if a.members < 1:
+        raise SystemExit("--members must be >= 1")
     if not torch.cuda.is_available():
         raise SystemExit("bench_scene needs a CUDA device")
-    res = {"info": device_info(), "roof_GBs": ROOF_GBS, "scene": [SIZE, SIZE, 3], "rows": run(a.calls)}
+    if a.tta == "none" and a.members == 1:
+        rows = run(a.calls)
+    else:
+        rows = run_tta(a.calls, a.tta, a.members)
+    res = {"info": device_info(), "roof_GBs": ROOF_GBS, "scene": [SIZE, SIZE, 3], "rows": rows}
     print(json.dumps(res["info"]))
     if a.out:
         Path(a.out).parent.mkdir(parents=True, exist_ok=True)
